@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - train iterations/sec of the dynamic-splatting hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c4_iphone] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c4_iphone] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one camera-time view per GPU:
 deformation + preprocess + binning + blend forward + (L1 + D-SSIM + Pearson depth + alpha
@@ -21,6 +21,8 @@ is not part of BASELINE.json's metric ("raster fwd+bwd+loss"); `--adam` adds the
 `cpu_baseline` / `--impl reference`: the PyTorch-CPU oracle (oracle/) on a bounded sample of the workload - a 256x256
            window at the workload's Gaussian density per tile - extrapolated to the full workload by algorithmic bytes
            (`"extrapolated": true`; `steps` / `warmup` are the frames actually run).
+`--dump-outputs DIR`: after the timed steps, rank 0 writes what the last timed step returned to its caller as DIR/<name>.npy
+           (see dump_outputs), so that two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -246,6 +248,45 @@ def workload_name(cfg, sh_degree=3):
 
 
 # ------------------------------------------------------------------------------------ GPU arm
+DUMP_ROWS = 16384          # Gaussians per model in the seeded sample of the per-Gaussian outputs
+DUMP_LIMIT = 64 << 20      # bytes written by --dump-outputs
+
+
+def dump_outputs(step, out_dir: str, forward_only: bool, with_sh: bool) -> None:
+    """What the last SplatTrainStep.forward_backward left for its caller, as float32 / float64 .npy files in out_dir.
+    In full: the colour / depth / alpha maps and (training step) the loss parts, dL/dV, dL/dtable and dL/dB(t).  The full
+    per-Gaussian gradients of the flagship workload are ~0.5 GB, so radii, dL/dmeans2D and every per-Gaussian parameter
+    gradient are written at a fixed, seeded sample of DUMP_ROWS Gaussians per model (indices in index_<model>.npy).
+    with_sh=False: dL/dSH was left in its factored form by the data-parallel exchange and is not written."""
+    import numpy as np
+    from rodygs_b200.trainer import PARAM_ORDER
+    color, depth, alpha, radii = step.last_outputs
+    out = {"color": color, "depth": depth, "alpha": alpha}
+    if not forward_only:
+        out.update(loss_parts=step.loss_parts, grad_viewmatrix=step.view_grad, grad_table=step.g("table"),
+                   grad_basis_t=step.g("basis_t"))
+    for tag, n, first in (("static", step.ns, 0), ("dynamic", step.nd, step.ns)):
+        if n == 0:
+            continue
+        idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+        out[f"index_{tag}"] = idx.double()
+        rows = idx.to(radii.device)
+        out[f"radii_{tag}"] = radii[first + rows]
+        if forward_only:
+            continue
+        out[f"grad_means2D_{tag}"] = step.means2D_grad[first + rows]
+        names = [k for k in PARAM_ORDER if with_sh or not k.startswith("features")]
+        for k in names + (["motion_coeff"] if tag == "dynamic" else []):
+            out[f"grad_{tag}_{k}"] = step.g(k if k == "motion_coeff" else f"{tag}.{k}")[rows]
+    arrays = {k: v.detach().cpu().numpy().astype(np.float64 if v.dtype == torch.float64 else np.float32) for k, v in out.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total / 2**20:.1f} MB (limit {DUMP_LIMIT >> 20} MB)")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args, rank, world, local_rank):
     import torch.distributed as dist
     from rodygs_b200 import _lib, engine, synthetic
@@ -253,6 +294,9 @@ def run_ours(args, rank, world, local_rank):
 
     dev = torch.device("cuda", local_rank)
     torch.cuda.set_device(dev)
+    # the step draws its local-Pearson boxes on the device; torch seeds CUDA generators differently in every process, so
+    # seed it to give every run with the same arguments the same inputs
+    torch.cuda.manual_seed(rank)
     lib = _lib.load()
     engine.config.sync_free = False   # target generation below sizes the duplicate buffers exactly
     N, H, W, T, _ = synthetic.CONFIGS[args.config]
@@ -438,6 +482,8 @@ def run_ours(args, rank, world, local_rank):
     events = step.stage_events
     step.stage_events = None
     clocks = sampler.stop(t_region0, t_region1) if sampler else None
+    if args.dump_outputs and rank == 0:    # before the other legs overwrite the step's buffers
+        dump_outputs(step, args.dump_outputs, args.forward_only, with_sh=not defer_sh)
 
     # e2e leg (host buffers -> H2D -> step -> D2H loss).  One GPU: the step is replayed as a CUDA graph (one per staging
     # slot), so the GPU does not wait for Python to enqueue ~25 launches after every loss read.
@@ -724,6 +770,8 @@ def main():
     ap.add_argument("--sm-reserve", type=int, default=16,
                     help="N>1: SMs the persistent backward kernels leave to NCCL while the bucketed all-reduce runs beside them")
     ap.add_argument("--timeline", default="", help="write the kernel timeline of one step (rank 0, torch.profiler) to this file")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write the last step's outputs as DIR/<name>.npy (at most 64 MB; see dump_outputs)")
     ap.add_argument("--no-sm-partition", action="store_true",
                     help="N>1: size the persistent backward grids for 148 - sm_reserve SMs instead of the SM-partitioned chunk queue (A/B)")
     ap.add_argument("--bwd-parts", type=int, default=-1,
@@ -739,6 +787,8 @@ def main():
     ap.add_argument("--plain-allreduce", action="store_true",
                     help="N>1: all-reduce the whole flat gradient buffer instead of the factored SH exchange (A/B)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -40,6 +40,47 @@ def test_reference_arm_caps_the_frames_it_runs():
     assert b.sample_shape("c4_iphone")[:3] == (62745, 256, 256)
 
 
+def test_dump_outputs_writes_the_last_step_within_64_mb(tmp_path):
+    """--dump-outputs at the flagship's image size (1080p) with more Gaussians per model than the sample takes (so the same
+    bytes as 2M Gaussians): float32 / float64 arrays only, at most 64 MB, the sampled rows are the ones the indices name,
+    and the sample is the same from run to run."""
+    import importlib.util
+    import types
+
+    import numpy as np
+    import torch
+    spec =importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    b = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(b)
+    from rodygs_b200 import trainer
+    ns, nd, K, T, H, W = 20000, 20001, 16, 100, 1080, 1920
+    layout, total = trainer.flat_layout(ns, nd, K, T)
+    grads = torch.randn(total, generator=torch.Generator().manual_seed(1))
+    step = types.SimpleNamespace(ns=ns, nd=nd, loss_parts=torch.rand(8), view_grad=torch.randn(4, 4),
+                                 means2D_grad=torch.randn(ns + nd, 3),
+                                 last_outputs=(torch.rand(3, H, W), torch.rand(1, H, W), torch.rand(1, H, W),
+                                               torch.randint(0, 50, (ns + nd,), dtype=torch.int32)))
+    step.g = lambda name: trainer.SplatTrainStep._slice(step, grads, name)
+    step.layout = layout
+    for run in ("a", "b"):
+        b.dump_outputs(step, str(tmp_path / run), forward_only=False, with_sh=True)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == sorted(os.listdir(tmp_path / "b"))
+    arrays = {f[:-4]: np.load(tmp_path / "a" / f) for f in files}
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64 << 20
+    for f in files:
+        assert np.array_equal(arrays[f[:-4]], np.load(tmp_path / "b" / f)), f
+    idx = torch.from_numpy(arrays["index_dynamic"]).long()
+    assert len(idx) == b.DUMP_ROWS and len(arrays["index_static"]) == b.DUMP_ROWS
+    for k in trainer.PARAM_ORDER + ("motion_coeff",):
+        ref = step.g(k if k == "motion_coeff" else f"dynamic.{k}")[idx]
+        assert np.array_equal(arrays[f"grad_dynamic_{k}"], ref.numpy()), k
+    assert np.array_equal(arrays["radii_dynamic"], step.last_outputs[3][ns + idx].float().numpy())
+    assert np.array_equal(arrays["grad_means2D_dynamic"], step.means2D_grad[ns + idx].numpy())
+    assert arrays["color"].shape == (3, H, W) and arrays["grad_table"].shape == (T, K, 7)
+
+
 def test_cpu_sample_matches_the_workload_density():
     """The bounded sample keeps the workload's Gaussians per tile: N' = N * 256 / tiles on a 256x256 window."""
     sys.path.insert(0, ROOT)
