@@ -101,9 +101,11 @@ __global__ void __launch_bounds__(RDG_BLOCK, 2) sh_grad_views_kernel(const ShGra
             campos_s[threadIdx.x][j] = -(vm[j * 4 + 0] * vm[12 + 0] + vm[j * 4 + 1] * vm[12 + 1] + vm[j * 4 + 2] * vm[12 + 2]);
     }
     if (deform) {
-        for (int e = threadIdx.x; e < nv * sc.num_basis * 3; e += RDG_BLOCK) {
-            const int v = e / (sc.num_basis * 3), r = e - v * sc.num_basis * 3, k = r / 3, j = r - k * 3;
-            bt3_s[v][k][j] = p.basis_ts[((int64_t)v * sc.num_basis + k) * 7 + j];
+        // all RDG_NUM_BASIS_MAX rows: the per-view sum below runs over every row (c[k] = 0 beyond num_basis), and 0 times a
+        // stale NaN / Inf left in shared memory by an earlier kernel is NaN
+        for (int e = threadIdx.x; e < nv * RDG_NUM_BASIS_MAX * 3; e += RDG_BLOCK) {
+            const int v = e / (RDG_NUM_BASIS_MAX * 3), r = e - v * RDG_NUM_BASIS_MAX * 3, k = r / 3, j = r - k * 3;
+            bt3_s[v][k][j] = k < sc.num_basis ? p.basis_ts[((int64_t)v * sc.num_basis + k) * 7 + j] : 0.f;
         }
         // every dynamic Gaussian needs the translation part of its birth-frame row: 48 scattered floats of a 448-byte row per
         // thread from global memory (the L1TEX-bound gather the preprocess kernels got rid of in round 1) - or 19 KB staged once

@@ -28,17 +28,7 @@ IMG_TOL, GRAD_TOL = 1e-4, 1e-3
 
 
 elementwise_ok = helpers.elementwise_ok
-
-
-def elementwise_vs_truth(got, ref32, ref64, rtol=1e-3, floor=1e-5):
-    """Element-wise bar against the float64 oracle: |a - b64| <= rtol |b64| + floor max|b64| - or, where float32 arithmetic
-    cannot resolve that (sums with cancellation: the float32 ORACLE misses its own float64 twin by more), 1.5 x the float32
-    oracle's error.  Returns (ok, ratio of the CUDA result, ratio of the float32 oracle)."""
-    got, ref32, ref64 = got.double().cpu(), ref32.double().cpu(), ref64.double().cpu()
-    bound = (rtol * ref64.abs() + floor * ref64.abs().max()).clamp_min(1e-300)
-    r_cu = ((got - ref64).abs() / bound).max().item()
-    r_32 = ((ref32 - ref64).abs() / bound).max().item()
-    return r_cu <= max(1.0, 1.5 * r_32), r_cu, r_32
+elementwise_vs_truth = helpers.elementwise_vs_truth
 
 
 def normwise_vs_truth(got, ref32, ref64, tol=GRAD_TOL):
