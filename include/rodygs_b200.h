@@ -440,6 +440,20 @@ int64_t rdg_knn_workspace_bytes(int64_t n);
 int rdg_knn(int64_t n, const float* points, int32_t K, int32_t* idx, float* dist2, void* workspace,
             int64_t workspace_bytes, void* stream);
 
+/* simple-knn's distCUDA2 (src/model/rodygs_static.py:130-133, initial scales): out[i] = ((b0 + b1) + b2) / 3 in
+ * float32, b ascending, the squared distances from point i to its 3 nearest OTHER points.  The point itself is skipped
+ * by index, not by distance: an exact duplicate counts as a neighbour at distance 0.  Same distance contract and
+ * exactness as rdg_knn.  n >= 4 (RDG_E_ARG below); out [n]; workspace as rdg_knn (rdg_knn_workspace_bytes(n)). */
+int rdg_knn3_mean_dist2(int64_t n, const float* points, float* out, void* workspace, int64_t workspace_bytes,
+                        void* stream);
+
+/* Backward of dist2[i, k] = |p_i - p_idx[i,k]|^2 (rdg_knn's output) for upstream gradient d_dist2 [n, K]:
+ *   d_query[i] = sum_k 2 g_ik (p_i - p_j)   overwritten, row-local, no atomics;
+ *   d_ref[j]  -= 2 g_ik (p_i - p_j)          float atomics, ADDED to what d_ref holds (the caller zeroes it).
+ * Either output may be NULL (the side that needs no gradient).  idx [n, K] int32. */
+int rdg_knn_dist2_bwd(int64_t n, int32_t K, const float* points, const int32_t* idx, const float* d_dist2, float* d_query,
+                      float* d_ref, void* stream);
+
 /* RigidityLoss.forward, modes "surface" and "distance_preserving" (src/trainer/losses.py:216-361), value and
  * gradient.  The n rows are the reference's random sample (`indice`, :228-232) gathered by the caller:
  *   points = (xyz + pred_translation)[indice], canon = xyz[indice], coeff = _motion_coeff[indice],

@@ -152,6 +152,8 @@ SYMBOLS = {
                                        c_ptr, c_ptr]),
     "rdg_knn_workspace_bytes": (C.c_int64, [C.c_int64]),
     "rdg_knn": (C.c_int, [C.c_int64, c_ptr, C.c_int32, c_ptr, c_ptr, c_ptr, C.c_int64, c_ptr]),
+    "rdg_knn3_mean_dist2": (C.c_int, [C.c_int64, c_ptr, c_ptr, c_ptr, C.c_int64, c_ptr]),
+    "rdg_knn_dist2_bwd": (C.c_int, [C.c_int64, C.c_int32, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
     "rdg_rigidity_workspace_bytes": (C.c_int64, [C.c_int64, C.c_int32, C.c_int32]),
     "rdg_rigidity": (C.c_int, [C.POINTER(RdgRigidity), c_ptr, C.c_int64, c_ptr]),
     "rdg_rigidity_sample": (C.c_int, [C.c_int64, C.c_int32, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, C.c_float, c_ptr, c_ptr,

@@ -14,6 +14,8 @@
 //   float32 rounding per operation (explicit _rn intrinsics, no FMA contraction), K smallest ascending, the query
 //   itself included, exact ties towards the lower index.  Indices are therefore bit-exact against the oracle.
 // Bound: L2 / LSU latency (gathered 16-byte records), ~27 cells x 2 records per query; HBM traffic is 16 B x n x 3.
+// The same grid build and walk also give simple-knn's distCUDA2 (rdg_knn3_mean_dist2) and the gradient of the distances
+// for the pytorch3d.ops.knn_points drop-in (rdg_knn_dist2_bwd).
 #include <float.h>
 #include <math.h>
 #include "common.cuh"
@@ -166,7 +168,9 @@ __global__ void __launch_bounds__(RDG_BLOCK) knn_fill_kernel(int64_t n, const fl
 
 __device__ __forceinline__ bool pair_less(float da, int ia, float db, int ib) { return da < db || (da == db && ia < ib); }
 
-template <int KMAX>
+// MEAN3 is simple-knn's distCUDA2: K = 3, the query itself is skipped BY INDEX (an exact duplicate is another point at
+// distance 0 and may sort ahead of it), and the output is one float per point, ((b0 + b1) + b2) / 3 with b ascending.
+template <int KMAX, bool MEAN3>
 __global__ void __launch_bounds__(128) knn_query_kernel(int64_t n, int K, const float4* __restrict__ sorted,
                                                         const uint32_t* __restrict__ start, const KnnGrid* __restrict__ grid,
                                                         int32_t* __restrict__ out_idx, float* __restrict__ out_d) {
@@ -174,6 +178,7 @@ __global__ void __launch_bounds__(128) knn_query_kernel(int64_t n, int K, const 
     if (s >= n) return;
     const KnnGrid g = *grid;
     const float4 q = sorted[s];
+    const int qi = __float_as_int(q.w);
     int cx, cy, cz;
     cell_of(g, q.x, q.y, q.z, cx, cy, cz);
     float bd[KMAX];
@@ -204,6 +209,7 @@ __global__ void __launch_bounds__(128) knn_query_kernel(int64_t n, int K, const 
                         const float dx = __fsub_rn(q.x, c.x), dy = __fsub_rn(q.y, c.y), dz = __fsub_rn(q.z, c.z);
                         const float d = __fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz));
                         const int ci = __float_as_int(c.w);
+                        if (MEAN3 && ci == qi) continue;
                         bool worse = true;   // candidate vs the current K-th best
 #pragma unroll
                         for (int j = 0; j < KMAX; ++j)
@@ -233,7 +239,10 @@ __global__ void __launch_bounds__(128) knn_query_kernel(int64_t n, int K, const 
         const float bound = fmaxf((float)r - 0.01f, 0.f) * g.cell;   // 1 % slack for the rounding of the cell index
         if (kth < bound * bound) break;
     }
-    const int qi = __float_as_int(q.w);
+    if (MEAN3) {
+        out_d[qi] = __fdiv_rn(__fadd_rn(__fadd_rn(bd[0], bd[1]), bd[2]), 3.0f);
+        return;
+    }
 #pragma unroll
     for (int j = 0; j < KMAX; ++j)
         if (j < K) {
@@ -262,17 +271,8 @@ static KnnLayout knn_layout(int64_t n) {
 
 extern "C" int64_t rdg_knn_workspace_bytes(int64_t n) { return n > 0 ? knn_layout(n).total : 0; }
 
-extern "C" int rdg_knn(int64_t n, const float* points, int32_t K, int32_t* idx, float* dist2, void* workspace,
-                       int64_t workspace_bytes, void* stream) {
-    RDG_CHECK_ARG(points && idx && dist2 && workspace, "null argument");
-    RDG_CHECK_ARG(K >= 1 && K <= 16, "K must be in 1..16");
-    RDG_CHECK_ARG(n >= K, "fewer points than neighbours requested");
-    RDG_CHECK_ARG(n < ((int64_t)1 << 31), "too many points");
-    const KnnLayout L = knn_layout(n);
-    RDG_CHECK_ARG(workspace_bytes >= L.total, "workspace too small (rdg_knn_workspace_bytes)");
-    RDG_CHECK_ARG(((uintptr_t)workspace & 255) == 0, "workspace must be 256-byte aligned");
-    cudaStream_t st = (cudaStream_t)stream;
-    char* ws = (char*)workspace;
+// bounding box -> cell size -> per-cell counts -> exclusive scan -> counting sort; 6 launches, no host round trip
+static int knn_build_grid(int64_t n, const float* points, const KnnLayout& L, char* ws, cudaStream_t st) {
     uint32_t* bbox = (uint32_t*)(ws + L.bbox);
     KnnGrid* grid = (KnnGrid*)(ws + L.grid);
     uint32_t* count = (uint32_t*)(ws + L.count);
@@ -288,10 +288,89 @@ extern "C" int rdg_knn(int64_t n, const float* points, int32_t K, int32_t* idx, 
     knn_count_kernel<<<pgrid, RDG_BLOCK, 0, st>>>(n, points, grid, count, cell_id);
     knn_scan_kernel<<<1, KNN_SCAN_THREADS, 0, st>>>(count, L.cell_cap, start);
     knn_fill_kernel<<<pgrid, RDG_BLOCK, 0, st>>>(n, points, cell_id, start, count, sorted);
+    return RDG_OK;
+}
+
+extern "C" int rdg_knn(int64_t n, const float* points, int32_t K, int32_t* idx, float* dist2, void* workspace,
+                       int64_t workspace_bytes, void* stream) {
+    RDG_CHECK_ARG(points && idx && dist2 && workspace, "null argument");
+    RDG_CHECK_ARG(K >= 1 && K <= 16, "K must be in 1..16");
+    RDG_CHECK_ARG(n >= K, "fewer points than neighbours requested");
+    RDG_CHECK_ARG(n < ((int64_t)1 << 31), "too many points");
+    const KnnLayout L = knn_layout(n);
+    RDG_CHECK_ARG(workspace_bytes >= L.total, "workspace too small (rdg_knn_workspace_bytes)");
+    RDG_CHECK_ARG(((uintptr_t)workspace & 255) == 0, "workspace must be 256-byte aligned");
+    cudaStream_t st = (cudaStream_t)stream;
+    char* ws = (char*)workspace;
+    const int rc = knn_build_grid(n, points, L, ws, st);
+    if (rc != RDG_OK) return rc;
+    const float4* sorted = (const float4*)(ws + L.sorted);
+    const uint32_t* start = (const uint32_t*)(ws + L.start);
+    const KnnGrid* grid = (const KnnGrid*)(ws + L.grid);
     const int qgrid = rdg_div_up(n, 128);
-    if (K <= 8) knn_query_kernel<8><<<qgrid, 128, 0, st>>>(n, K, sorted, start, grid, idx, dist2);
-    else knn_query_kernel<16><<<qgrid, 128, 0, st>>>(n, K, sorted, start, grid, idx, dist2);
+    if (K <= 8) knn_query_kernel<8, false><<<qgrid, 128, 0, st>>>(n, K, sorted, start, grid, idx, dist2);
+    else knn_query_kernel<16, false><<<qgrid, 128, 0, st>>>(n, K, sorted, start, grid, idx, dist2);
     RDG_CHECK_LAUNCH();
     rdg_count_launches(7);
+    return RDG_OK;
+}
+
+extern "C" int rdg_knn3_mean_dist2(int64_t n, const float* points, float* out, void* workspace, int64_t workspace_bytes,
+                                   void* stream) {
+    RDG_CHECK_ARG(points && out && workspace, "null argument");
+    RDG_CHECK_ARG(n >= 4, "distCUDA2 needs at least 4 points (3 neighbours besides the point itself)");
+    RDG_CHECK_ARG(n < ((int64_t)1 << 31), "too many points");
+    const KnnLayout L = knn_layout(n);
+    RDG_CHECK_ARG(workspace_bytes >= L.total, "workspace too small (rdg_knn_workspace_bytes)");
+    RDG_CHECK_ARG(((uintptr_t)workspace & 255) == 0, "workspace must be 256-byte aligned");
+    cudaStream_t st = (cudaStream_t)stream;
+    char* ws = (char*)workspace;
+    const int rc = knn_build_grid(n, points, L, ws, st);
+    if (rc != RDG_OK) return rc;
+    knn_query_kernel<3, true><<<rdg_div_up(n, 128), 128, 0, st>>>(
+        n, 3, (const float4*)(ws + L.sorted), (const uint32_t*)(ws + L.start), (const KnnGrid*)(ws + L.grid), nullptr, out);
+    RDG_CHECK_LAUNCH();
+    rdg_count_launches(7);
+    return RDG_OK;
+}
+
+// dist2[i, k] = |p_i - p_j|^2 with j = idx[i, k]: d/dp_i = 2 g (p_i - p_j) summed over k in registers (every row is one
+// thread's), d/dp_j = -2 g (p_i - p_j) scattered with float atomics (a point is the neighbour of many rows).
+__global__ void __launch_bounds__(RDG_BLOCK) knn_dist2_bwd_kernel(int64_t n, int K, const float* __restrict__ pts,
+                                                                  const int32_t* __restrict__ idx,
+                                                                  const float* __restrict__ g,
+                                                                  float* __restrict__ d_query, float* __restrict__ d_ref) {
+    const int64_t i = (int64_t)blockIdx.x * RDG_BLOCK + threadIdx.x;
+    if (i >= n) return;
+    const float px = pts[i * 3], py = pts[i * 3 + 1], pz = pts[i * 3 + 2];
+    float ax = 0.f, ay = 0.f, az = 0.f;
+    for (int k = 0; k < K; ++k) {
+        const int64_t j = idx[i * K + k];
+        const float g2 = 2.0f * g[i * K + k];
+        const float cx = g2 * (px - pts[j * 3]), cy = g2 * (py - pts[j * 3 + 1]), cz = g2 * (pz - pts[j * 3 + 2]);
+        ax += cx; ay += cy; az += cz;
+        if (d_ref) {
+            atomicAdd(d_ref + j * 3, -cx);
+            atomicAdd(d_ref + j * 3 + 1, -cy);
+            atomicAdd(d_ref + j * 3 + 2, -cz);
+        }
+    }
+    if (d_query) {
+        d_query[i * 3] = ax;
+        d_query[i * 3 + 1] = ay;
+        d_query[i * 3 + 2] = az;
+    }
+}
+
+extern "C" int rdg_knn_dist2_bwd(int64_t n, int32_t K, const float* points, const int32_t* idx, const float* d_dist2,
+                                 float* d_query, float* d_ref, void* stream) {
+    RDG_CHECK_ARG(points && idx && d_dist2, "null argument");
+    RDG_CHECK_ARG(K >= 1 && K <= 16, "K must be in 1..16");
+    RDG_CHECK_ARG(n >= K && n < ((int64_t)1 << 31), "n out of range");
+    if (!d_query && !d_ref) return RDG_OK;
+    knn_dist2_bwd_kernel<<<rdg_div_up(n, RDG_BLOCK), RDG_BLOCK, 0, (cudaStream_t)stream>>>(n, K, points, idx, d_dist2,
+                                                                                          d_query, d_ref);
+    RDG_CHECK_LAUNCH();
+    rdg_count_launches(1);
     return RDG_OK;
 }
