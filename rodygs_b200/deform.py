@@ -167,6 +167,9 @@ class BasisMLP:
         self._lib = _lib
         _lib.load()                                   # raises if the CUDA library is not built: no fallback
         self.width, self.num_basis, self.out_dim = netwidth, num_basis, out_dim
+        # everything but the device: what a checkpoint needs to build the same network again (SplatTrainStep.state_dict)
+        self.init_args = {"netwidth": int(netwidth), "num_basis": int(num_basis), "t_emb_multires": int(t_emb_multires),
+                          "t_log_sampling": bool(t_log_sampling), "activation": str(activation), "out_dim": int(out_dim)}
         self.emb_dim = 2 * t_emb_multires + 1
         self.activation = 1 if activation.lower() == "relu" else 0
         self.device = torch.device(device)

@@ -25,6 +25,9 @@ from ._lib import check, ptr
 from .engine import SceneArgs, SceneGrads, SetArgs, SetGrads, ViewArgs
 
 PARAM_ORDER = ("xyz", "scaling", "rotation", "opacity", "features_dc", "features_rest")
+# SplatTrainStep.state_dict(): the tag and version a loader checks before it reads anything else
+CHECKPOINT_FORMAT, CHECKPOINT_VERSION = "rodygs_b200.SplatTrainStep", 1
+STATS_FIELDS = ("grad_accum", "denom", "max_radii2D")
 
 
 def flat_layout(n_static: int, n_dynamic: int, num_basis: int, num_times: int) -> Tuple[Dict[str, Tuple[int, Tuple[int, ...]]], int]:
@@ -101,7 +104,8 @@ def allgather_rows(local: torch.Tensor, out: torch.Tensor, group=None) -> torch.
 class CapturedStep:
     """A captured SplatTrainStep.forward_backward (CUDA graph).  replay() runs it on the current stream; the duplicate count of
     the PREVIOUS replay (copied to pinned host memory by the graph) is checked against the captured buffers' capacity first -
-    the graph cannot re-bin, so an overflow raises and the step has to be captured again."""
+    the graph cannot re-bin, so an overflow raises and the step has to be captured again.  The graph holds the step's buffers
+    of the moment: capture again after densify_and_prune and after load_state_dict, which both replace them."""
 
     def __init__(self, graph, host_count, d_cap, state, outputs):
         self.graph, self._host, self.d_cap = graph, host_count, int(d_cap)
@@ -146,13 +150,7 @@ class SplatTrainStep:
         self.bg = torch.zeros(3, dtype=torch.float32, device=self.dev)          # rodygs.py:267
         self.view_grad = torch.zeros(4, 4, **f32)
         self.loss_parts = torch.zeros(8, **f32)   # [0:3] photometric (loss, l1, ssim), [3] pearson, [4] alpha term, [5] local pearson
-        if self.n_local > 0:
-            # boxes (row0, col0, rows, cols): the origins are redrawn on the device every step like the reference does
-            # (torch.randint(0, max_h) / (0, max_w), losses.py:149-150): one randint launch + one remainder launch
-            self._boxes = torch.zeros(self.n_local, 4, dtype=torch.int32, device=self.dev)
-            self._boxes[:, 2:] = self.box_p
-            self._box_limits = torch.tensor([self.H - self.box_p, self.W - self.box_p], dtype=torch.int32, device=self.dev)
-            self._box_rand = torch.empty(self.n_local, 2, dtype=torch.int32, device=self.dev)
+        self._alloc_boxes()
         self.local_box_origins = None             # tests: fixed [n, 2] (row0, col0) instead of the random draw
         self.dL_dcolor = torch.empty(3, self.H, self.W, **f32)
         self.dL_ddepth = torch.zeros(1, self.H, self.W, **f32)
@@ -164,6 +162,15 @@ class SplatTrainStep:
         self.last_state: Optional[engine.FwdState] = None
         self._deferred = None      # exchange_grads(defer_sh=True): the factors the next optimizer_step consumes
         self.stage_events = None   # set by enable_stage_timing()
+
+    def _alloc_boxes(self):
+        if self.n_local > 0:
+            # boxes (row0, col0, rows, cols): the origins are redrawn on the device every step like the reference does
+            # (torch.randint(0, max_h) / (0, max_w), losses.py:149-150): one randint launch + one remainder launch
+            self._boxes = torch.zeros(self.n_local, 4, dtype=torch.int32, device=self.dev)
+            self._boxes[:, 2:] = self.box_p
+            self._box_limits = torch.tensor([self.H - self.box_p, self.W - self.box_p], dtype=torch.int32, device=self.dev)
+            self._box_rand = torch.empty(self.n_local, 2, dtype=torch.int32, device=self.dev)
 
     def _load_scene(self, scene: Dict):
         """(Re)build everything whose size depends on the Gaussian counts: the flat parameter / gradient buffers, the
@@ -181,6 +188,8 @@ class SplatTrainStep:
                 self.p(f"{tag}.{k}").copy_(scene[tag][k])
         self.p("motion_coeff").copy_(scene["motion_coeff"])
         self.p("table").copy_(scene["table"])
+        if "basis_t" in scene:                  # optional: B(t) of the last query time (checkpoints); zero otherwise
+            self.p("basis_t").copy_(scene["basis_t"])
         self.time_ind = scene["time_ind"].to(self.dev, torch.int32).contiguous()
         self.spatial_lr_scale = float(scene["spatial_lr_scale"])
         self.frame_order, self.frame_offsets = engine.frame_csr(self.time_ind, self.T) if nd > 0 else (None, None)
@@ -954,3 +963,237 @@ class SplatTrainStep:
         """photometric + w_p * pearson + w_local * local pearson + alpha term (device scalar)."""
         lp = self.loss_parts
         return lp[0] + self.w[2] * lp[3] + lp[4] + (self.w_local * lp[5] if self.n_local > 0 else 0.0)
+
+    # -- checkpoints -------------------------------------------------------------------------------------------
+    def _check_saveable(self):
+        d = getattr(self, "_deferred", None)
+        if d is not None and d["pending"]:
+            raise RuntimeError("SplatTrainStep.state_dict: exchange_grads(defer_sh=True) left the SH gradient factors of "
+                               f"{sorted(d['pending'])} pending; call optimizer_step for them first")
+
+    def _dp_rank_world(self) -> Tuple[int, int]:
+        import torch.distributed as dist
+        if dist.is_available() and dist.is_initialized() and dist.get_world_size(self.pg) > 1:
+            return dist.get_rank(self.pg), dist.get_world_size(self.pg)
+        return 0, 1
+
+    def _rank_state(self) -> Dict:
+        """The part of the state that differs between data-parallel ranks: the densification statistics (each rank adds
+        its own views' radii and means2D gradients; they are only reduced inside densify_and_prune) and the CUDA
+        generator (seeded per rank)."""
+        return {"stats": {tag: {f: getattr(st, f).detach().to("cpu", copy=True) for f in STATS_FIELDS}
+                          for tag, st in self.stats.items()},
+                "cuda_rng_state": torch.cuda.get_rng_state(self.dev)}
+
+    def state_dict(self) -> Dict:
+        """Everything a resumed run needs to train on exactly as this one would, as CPU tensors, numbers, strings, lists
+        and dicts (so torch.load(weights_only=True) reads it back).  Parameters and moments are stored by name, never as
+        the flat buffer: the flat layout changes with every densification.  Gradients are not state (every step
+        rewrites them): save between iterations, after optimizer_step.  "ranks" holds one entry per data-parallel rank
+        (statistics, CUDA generator; see _rank_state); state_dict() fills in the calling process only, save() all ranks."""
+        self._check_saveable()
+        from .optim import GROUP_OF
+        from dataclasses import asdict
+
+        def cpu(t):
+            return t.detach().to("cpu", copy=True)
+
+        w_l1, w_dssim, w_pearson, w_alpha = self.w
+        sd = {"format": CHECKPOINT_FORMAT, "version": CHECKPOINT_VERSION,
+              "ns": self.ns, "nd": self.nd, "num_basis": self.num_basis, "T": self.T, "H": self.H, "W": self.W,
+              "sh_degree": self.sh_degree, "w_l1": w_l1, "w_dssim": w_dssim, "w_pearson": w_pearson, "w_alpha": w_alpha,
+              "w_local": self.w_local, "box_p": self.box_p, "n_local": self.n_local,
+              "params": {name: cpu(self.p(name)) for name in self.layout},
+              "time_ind": cpu(self.time_ind), "spatial_lr_scale": self.spatial_lr_scale,
+              "optim": {}, "skip_step": sorted(self._skip_step), "ranks": [self._rank_state()]}
+        field_of = {g: f for f, g in GROUP_OF.items()}
+        for tag, opt in self.optim.items():
+            shapes = {g: self.layout["motion_coeff" if g == "motion_coeff" else f"{tag}.{field_of[g]}"][1] for g in opt.ranges}
+            moments = {g: opt.moments(g) for g in opt.ranges}
+            sd["optim"][tag] = {"lrs": {k: v for k, v in asdict(opt.lrs).items() if v is not None},
+                                "betas": [float(b) for b in opt.betas], "eps": float(opt.eps), "steps": int(opt.steps),
+                                "exp_avg": {g: cpu(m.view(shapes[g])) for g, (m, _) in moments.items()},
+                                "exp_avg_sq": {g: cpu(v.view(shapes[g])) for g, (_, v) in moments.items()}}
+        mlp = getattr(self, "mlp", None)
+        if mlp is not None:
+            sd["mlp"] = {"args": dict(mlp.init_args), "state_dict": {k: cpu(v) for k, v in mlp.state_dict().items()},
+                         "lr": self._mlp_lr, "steps": int(self._mlp_steps), "train_times": cpu(self._mlp_times[1:])}
+            if self._mlp_moments is not None:
+                sd["mlp"]["exp_avg"], sd["mlp"]["exp_avg_sq"] = (cpu(t) for t in self._mlp_moments)
+        return sd
+
+    def _rank_entry(self, ranks: List[Dict]) -> Tuple[Dict, torch.Tensor]:
+        """(statistics, generator state) this process resumes from.  Same number of ranks as saved: its own entry.
+        Otherwise the statistics are combined (sum, sum, max) into rank 0 and the other ranks start their sums at zero, so
+        the all-reduce inside the next densify_and_prune still sees every saved contribution once; rank r takes the
+        generator of saved rank r mod the saved count."""
+        rank, world = self._dp_rank_world()
+        if len(ranks) == world:
+            return ranks[rank]["stats"], ranks[rank]["cuda_rng_state"]
+        stats = {}
+        for tag in ranks[0]["stats"]:
+            per = [r["stats"][tag] for r in ranks]
+            s = {"grad_accum": sum(p["grad_accum"] for p in per), "denom": sum(p["denom"] for p in per),
+                 "max_radii2D": torch.stack([p["max_radii2D"] for p in per]).amax(0)}
+            if rank > 0:
+                s["grad_accum"], s["denom"] = torch.zeros_like(s["grad_accum"]), torch.zeros_like(s["denom"])
+            stats[tag] = s
+        return stats, ranks[rank % len(ranks)]["cuda_rng_state"]
+
+    def _parse_state(self, sd: Dict):
+        """Every check of load_state_dict, before anything of this step changes."""
+        from .optim import GROUP_OF, GaussianLRs
+        pre = "SplatTrainStep.load_state_dict"
+        for field, have in (("H", self.H), ("W", self.W)):
+            if int(sd[field]) != have:
+                raise ValueError(f"{pre}: {field} is {sd[field]} in the state dict but {have} here "
+                                 "(the image buffers are sized by it); build the step with from_state_dict instead")
+        ns, nd, K, T = (int(sd[k]) for k in ("ns", "nd", "num_basis", "T"))
+        mlp = getattr(self, "mlp", None)
+        if mlp is not None:
+            for field, have in (("num_basis", mlp.num_basis), ("T", self._mlp_times.numel() - 1)):
+                if int(sd[field]) != have:
+                    raise ValueError(f"{pre}: {field} is {sd[field]} in the state dict but the attached basis MLP has {have}")
+            if "mlp" not in sd:
+                raise ValueError(f"{pre}: the state dict has no basis MLP but one is attached to this step (its next "
+                                 "basis_forward would overwrite the saved table); load it with from_state_dict")
+            for k, v in sd["mlp"]["args"].items():
+                if mlp.init_args[k] != v:
+                    raise ValueError(f"{pre}: the attached basis MLP has {k}={mlp.init_args[k]!r}, the state dict {v!r}")
+        layout, _ = flat_layout(ns, nd, K, T)
+        P = sd["params"]
+        for name, (_, shp) in layout.items():
+            if tuple(P[name].shape) != shp:
+                raise ValueError(f"{pre}: params[{name!r}] has shape {tuple(P[name].shape)}, the saved counts give {shp}")
+        if tuple(sd["time_ind"].shape) != (nd,):
+            raise ValueError(f"{pre}: time_ind has shape {tuple(sd['time_ind'].shape)}, expected ({nd},)")
+        scene = {tag: {k: P[f"{tag}.{k}"] for k in PARAM_ORDER} for tag in ("static", "dynamic")}
+        scene.update(motion_coeff=P["motion_coeff"], table=P["table"], basis_t=P["basis_t"], time_ind=sd["time_ind"],
+                     spatial_lr_scale=float(sd["spatial_lr_scale"]))
+        optims = {}
+        for tag, o in sd["optim"].items():
+            if tag not in ("static", "dynamic"):
+                raise ValueError(f"{pre}: optimiser of unknown model {tag!r}")
+            groups = {g: layout[f"{tag}.{f}"][1] for f, g in GROUP_OF.items()}
+            if tag == "dynamic":
+                groups["motion_coeff"] = layout["motion_coeff"][1]
+            for kind in ("exp_avg", "exp_avg_sq"):
+                for g, shp in groups.items():
+                    if o[kind][g].numel() != math.prod(shp):
+                        raise ValueError(f"{pre}: optim[{tag!r}][{kind!r}][{g!r}] has {o[kind][g].numel()} elements, "
+                                         f"expected {math.prod(shp)}")
+            optims[tag] = (GaussianLRs(**o["lrs"]), tuple(float(b) for b in o["betas"]), float(o["eps"]), int(o["steps"]), o)
+        stats, rng = self._rank_entry(sd["ranks"])
+        for tag, s in stats.items():
+            n = {"static": ns, "dynamic": nd}[tag]
+            for f in STATS_FIELDS:
+                if tuple(s[f].shape) != (n,):
+                    raise ValueError(f"{pre}: statistics {tag}.{f} have shape {tuple(s[f].shape)}, expected ({n},)")
+        if "mlp" in sd:
+            m = sd["mlp"]
+            if m["train_times"].numel() != T:
+                raise ValueError(f"{pre}: the basis MLP has {m['train_times'].numel()} training times, the table {T} rows")
+            missing = [k for k in ("args", "state_dict", "lr", "steps") if k not in m]
+            if missing:
+                raise ValueError(f"{pre}: the basis MLP entry has no {missing}")
+        return scene, optims, stats, rng
+
+    def load_state_dict(self, sd: Dict):
+        """Restore a state_dict(): the flat buffers are rebuilt at the saved Gaussian counts (this step may have been built
+        for any other N), then the loss configuration, the optimisers, the pending post-densification skips, the
+        densification statistics, the basis MLP (built from the saved arguments when none is attached) and the CUDA
+        generator that draws the local Pearson boxes.  Every check runs before anything changes; it refuses what it cannot
+        repair, naming the field: another image size, a num_basis / T / network that differs from the MLP attached to this
+        step, or a state without an MLP while one is attached.  Like densify_and_prune this replaces every buffer: a
+        CapturedStep taken before must be captured again, and an enabled factored exchange is set up again."""
+        pre = "SplatTrainStep.load_state_dict"
+        if not isinstance(sd, dict) or sd.get("format") != CHECKPOINT_FORMAT or sd.get("version") != CHECKPOINT_VERSION:
+            got = (sd.get("format"), sd.get("version")) if isinstance(sd, dict) else type(sd).__name__
+            raise ValueError(f"{pre}: not a {CHECKPOINT_FORMAT} v{CHECKPOINT_VERSION} state dict ({got!r})")
+        try:
+            scene, optims, stats, rng = self._parse_state(sd)
+        except (KeyError, TypeError, AttributeError) as e:
+            raise ValueError(f"{pre}: malformed state dict ({type(e).__name__}: {e})") from None
+        from .densify import DensifyStats
+        from .optim import GaussianAdam
+        self._load_scene(scene)
+        self.sh_degree = int(sd["sh_degree"])
+        self.w = tuple(float(sd[k]) for k in ("w_l1", "w_dssim", "w_pearson", "w_alpha"))
+        self.w_local, self.box_p, self.n_local = float(sd["w_local"]), int(sd["box_p"]), int(sd["n_local"])
+        self._alloc_boxes()
+        self.optim = {}
+        for tag, (lrs, betas, eps, steps, o) in optims.items():
+            opt = GaussianAdam(self._group_ranges(tag), self.params.numel(), lrs, self.spatial_lr_scale, self.dev, betas, eps)
+            opt.steps = steps
+            for g in opt.ranges:
+                m, v = opt.moments(g)
+                m.copy_(o["exp_avg"][g].reshape(-1))
+                v.copy_(o["exp_avg_sq"][g].reshape(-1))
+            self.optim[tag] = opt
+        self._skip_step = set(sd["skip_step"])
+        self.stats = {}
+        for tag, s in stats.items():
+            st = DensifyStats(s["denom"].shape[0], self.dev)
+            for f in STATS_FIELDS:
+                getattr(st, f).copy_(s[f])
+            self.stats[tag] = st
+        if "mlp" in sd:
+            m = sd["mlp"]
+            mlp = getattr(self, "mlp", None)
+            if mlp is None:
+                from .deform import BasisMLP
+                mlp = BasisMLP(**m["args"], device=self.dev)
+            mlp.load_state_dict(m["state_dict"])
+            self.attach_basis_mlp(mlp, m["train_times"], lr=float(m["lr"]))
+            self._mlp_steps = int(m["steps"])
+            if "exp_avg" in m:
+                self._mlp_moments = (m["exp_avg"].to(self.dev), m["exp_avg_sq"].to(self.dev))
+        torch.cuda.set_rng_state(rng, self.dev)
+        if getattr(self, "_fx_args", None) is not None:          # the exchange buffers are sized by the Gaussian count
+            self.enable_factored_exchange(*self._fx_args)
+        return self
+
+    @classmethod
+    def from_state_dict(cls, sd: Dict, device="cuda", process_group=None) -> "SplatTrainStep":
+        """A step built from a state_dict() alone (no scene dict): image size, loss weights and counts come from it."""
+        f32 = dict(dtype=torch.float32)
+        K, T = int(sd["num_basis"]), int(sd["T"])
+        empty = {k: torch.zeros((0,) + s, **f32) for k, s in (("xyz", (3,)), ("scaling", (3,)), ("rotation", (4,)),
+                                                             ("opacity", (1,)), ("features_dc", (1, 3)), ("features_rest", (15, 3)))}
+        scene = {"static": empty, "dynamic": empty, "motion_coeff": torch.zeros(0, 1, K, **f32),
+                 "table": torch.zeros(T, K, 7, **f32), "time_ind": torch.zeros(0, dtype=torch.int32), "spatial_lr_scale": 1.0}
+        step = cls(scene, int(sd["H"]), int(sd["W"]), sh_degree=int(sd["sh_degree"]), device=device, process_group=process_group,
+                   w_local=float(sd["w_local"]), box_p=int(sd["box_p"]))
+        return step.load_state_dict(sd)
+
+    def save(self, path):
+        """torch.save(state_dict(), path).  Under data parallelism every rank calls it: the per-rank part of the state
+        (_rank_state) is gathered from all ranks, rank 0 writes the file, and every rank returns once it is complete - or
+        raises, on every rank, when the state cannot be saved or rank 0 could not write it."""
+        import torch.distributed as dist
+        self._check_saveable()                 # on every rank before any collective (the ranks hold the same pending set)
+        rank, world = self._dp_rank_world()
+        if world == 1:
+            torch.save(self.state_dict(), path)
+            return
+        ranks = [None] * world
+        dist.all_gather_object(ranks, self._rank_state(), group=self.pg)
+        err = None
+        if rank == 0:
+            try:
+                sd = self.state_dict()
+                sd["ranks"] = ranks
+                torch.save(sd, path)
+            except Exception as e:   # noqa: BLE001 - reported on every rank below
+                err = e
+        flag = torch.tensor([0 if err is None else 1], dtype=torch.int32, device=self.dev)
+        dist.broadcast(flag, 0 if self.pg is None else dist.get_global_rank(self.pg, 0), group=self.pg)
+        if err is not None:
+            raise err
+        if int(flag.item()):
+            raise RuntimeError(f"SplatTrainStep.save: rank 0 could not write {path} (see its error)")
+
+    def load(self, path):
+        """load_state_dict(torch.load(path, weights_only=True)); every rank of a data-parallel run reads the same file and
+        takes its own statistics and generator from it."""
+        return self.load_state_dict(torch.load(path, map_location="cpu", weights_only=True))
