@@ -35,7 +35,8 @@ __constant__ float c_taps[11] = {1.028380124e-03f, 7.598758209e-03f, 3.600077331
 // Header of the loss workspace (256 bytes reserved): running sums and the Pearson gradient coefficients.
 struct LossHdr {
     double sums[8];   // 0 ssim, 1 |x-y|, 2..6 depth: sum p, g, pp, gg, pg, 7 sum(1 - alpha)
-    float coef[8];    // 0 mean g, 1 mean p, 2 d/d(g - mg), 3 d/d(p - mp)  (dL/ddepth = c2 (g-mg) + c3 (p-mp)), 4 dL/dalpha
+    float coef[8];    // 0 mean g, 1 mean p, 2 d/d(g - mg), 3 d/d(p - mp), 5 rounding correction of the two float means
+                      // (dL/ddepth = c2 (g-mg) + c3 (p-mp) + c5), 4 dL/dalpha
     double local_sum; // sum over the boxes of (1 - Pearson_b)
 };
 #define LOCAL_BOXES_MAX 256
@@ -43,9 +44,18 @@ struct LossHdr {
 struct __align__(16) LocalBox {
     float coef[4];    // mean g, mean p, d/d(g - mg), d/d(p - mp), weight included (read as one float4)
     double st[5];     // sum p, g, pp, gg, pg over the box
-    int pad[2];
+    float c0;         // rounding correction of the two float means (see pearson_coef_correction)
+    int pad;
 };
 static_assert(sizeof(LocalBox) == 64, "LocalBox layout");
+
+// The gradient of a Pearson term is applied per pixel as c_g (g - mean g) + c_p (p - mean p) with both means rounded to
+// float.  Their rounding error is a constant offset over the box that the exact gradient does not have (it sums to zero
+// over the box), and c_p grows as 1 / std(p): in a nearly flat box it swamped the per-pixel values.  This constant,
+// formed in double, cancels the offset.
+__device__ __forceinline__ float pearson_coef_correction(double cg, double mg, double cp, double mp) {
+    return (float)(-(cg * (mg - (double)(float)mg) + cp * (mp - (double)(float)mp)));
+}
 
 // The local Pearson boxes that overlap the 32x32 tile at (tx0, ty0), in box order, into near[] (call from warp 0; ballot
 // compaction, so that per-pixel sums over the list keep one order).  A 128x128 box overlaps ~1 % of the tiles: every thread
@@ -302,8 +312,8 @@ __global__ void __launch_bounds__(LTHREADS) ssim_bwd_kernel(const float* __restr
         __syncthreads();
     }
     const int n_near = (do_depth && n_boxes > 0) ? n_near_s : 0;
-    float mg = 0.f, mp = 0.f, cg = 0.f, cp = 0.f, ca = 0.f;
-    if (do_depth) { mg = hdr->coef[0]; mp = hdr->coef[1]; cg = hdr->coef[2]; cp = hdr->coef[3]; }
+    float mg = 0.f, mp = 0.f, cg = 0.f, cp = 0.f, c0g = 0.f, ca = 0.f;
+    if (do_depth) { mg = hdr->coef[0]; mp = hdr->coef[1]; cg = hdr->coef[2]; cp = hdr->coef[3]; c0g = hdr->coef[5]; }
     if (do_alpha) ca = hdr->coef[4];
 #pragma unroll
     for (int i = 0; i < VSEG; ++i) {
@@ -317,13 +327,13 @@ __global__ void __launch_bounds__(LTHREADS) ssim_bwd_kernel(const float* __restr
             dL_dpred[pix] = k_ssim * dssim + k_l1 * sgn;
             if (do_depth) {
                 const float g = gt_depth[hwpix], pv = depth[hwpix];
-                float acc = cg * (g - mg) + cp * (pv - mp);
+                float acc = cg * (g - mg) + cp * (pv - mp) + c0g;
                 for (int k = 0; k < n_near; ++k) {                // every local box that covers this pixel adds its term
                     const int b = near_box[k];
                     const int4 bx = boxes[b];
                     if (y >= bx.x && y < bx.x + bx.z && x >= bx.y && x < bx.y + bx.w) {
                         const float4 c4 = *reinterpret_cast<const float4*>(lbox[b].coef);
-                        acc += c4.z * (g - c4.x) + c4.w * (pv - c4.y);
+                        acc += c4.z * (g - c4.x) + c4.w * (pv - c4.y) + lbox[b].c0;
                     }
                 }
                 dL_ddepth[hwpix] = acc;
@@ -357,6 +367,7 @@ __global__ void loss_finalize_kernel(LossHdr* __restrict__ hdr, double n, double
         hdr->coef[1] = (float)mp;
         hdr->coef[2] = (float)(-(double)w_pearson * k1);
         hdr->coef[3] = (float)((double)w_pearson * k2);
+        hdr->coef[5] = pearson_coef_correction(-(double)w_pearson * k1, mg, (double)w_pearson * k2, mp);
     }
     if (use_alpha) {
         out[4] = (float)((double)w_alpha * sums[7] / npix);
@@ -387,6 +398,7 @@ __global__ void local_pearson_finalize_kernel(LossHdr* __restrict__ hdr, const i
         lbox[b].coef[1] = (float)mp;
         lbox[b].coef[2] = (float)(-wgt * k1);
         lbox[b].coef[3] = (float)(wgt * k2);
+        lbox[b].c0 = pearson_coef_correction(-wgt * k1, mg, wgt * k2, mp);
     }
     part[threadIdx.x] = loss_b;
     __syncthreads();
@@ -397,9 +409,13 @@ __global__ void local_pearson_finalize_kernel(LossHdr* __restrict__ hdr, const i
     }
 }
 
+// Workspace: LossHdr (256 B), the three derivative maps, then the LocalBox array.  The maps are rounded up to 256 B so that
+// the boxes stay 16-byte aligned (pass 2 reads their coefficients as one float4) when C * H * W is not a multiple of 4.
+static int64_t loss_boxes_offset(int64_t plane) { return 256 + rdg_align_up(3 * plane * (int64_t)sizeof(float), 256); }
+
 extern "C" int64_t rdg_l1_dssim_workspace_bytes(int32_t channels, int32_t height, int32_t width) {
     if (channels <= 0 || height <= 0 || width <= 0) return RDG_E_ARG;
-    return 256 + (int64_t)3 * channels * height * width * (int64_t)sizeof(float) + (int64_t)LOCAL_BOXES_MAX * (int64_t)sizeof(LocalBox);
+    return loss_boxes_offset((int64_t)channels * height * width) + (int64_t)LOCAL_BOXES_MAX * (int64_t)sizeof(LocalBox);
 }
 
 extern "C" int rdg_losses(const float* pred, const float* gt, int32_t channels, int32_t height, int32_t width,
@@ -417,12 +433,13 @@ extern "C" int rdg_losses(const float* pred, const float* gt, int32_t channels, 
                            extra->w_local != 0.0f;
     RDG_CHECK_ARG(!use_local || extra->n_local_boxes <= LOCAL_BOXES_MAX, "at most 256 local Pearson boxes");
     RDG_CHECK_ARG(!(use_local && dL_dpred) || extra->dL_ddepth, "the local Pearson term needs dL_ddepth");
+    RDG_CHECK_ARG(((uintptr_t)workspace & 15) == 0, "workspace must be 16-byte aligned");
     const bool any_depth = use_depth || use_local;
     cudaStream_t s = (cudaStream_t)stream;
     LossHdr* hdr = (LossHdr*)workspace;
     const size_t plane = (size_t)channels * height * width;
     float* maps = (float*)((char*)workspace + 256);
-    LocalBox* lbox = (LocalBox*)((char*)workspace + 256 + 3 * plane * sizeof(float));
+    LocalBox* lbox = (LocalBox*)((char*)workspace + loss_boxes_offset((int64_t)plane));
     const int4* boxes = use_local ? (const int4*)extra->local_boxes : nullptr;
     const int n_boxes = use_local ? extra->n_local_boxes : 0;
     RDG_CUDA(cudaMemsetAsync(hdr, 0, sizeof(LossHdr), s));

@@ -201,6 +201,9 @@ __global__ void __launch_bounds__(RG_BLOCK) rg_space_kernel(int64_t n, int K, co
     double lsum = 0.0;
     if (i < n) {
         const float px = pts[i * 3], py = pts[i * 3 + 1], pz = pts[i * 3 + 2];
+        // p_i - mean_k p_j as the mean of the differences.  Each difference is rounded once at the scale of the difference
+        // (and is exact when the two coordinates are within a factor of 2 of each other), where p_i minus the float mean
+        // of the coordinates kept the sum's rounding (~ulp of the coordinates) on a value ~1e-2 of them
         float mx = 0.f, my = 0.f, mz = 0.f;
         float ax = 0.f, ay = 0.f, az = 0.f;          // gradient on the point itself
         int js[RG_KMAX];
@@ -209,13 +212,13 @@ __global__ void __launch_bounds__(RG_BLOCK) rg_space_kernel(int64_t n, int K, co
             if (k < K) {
                 const int j = nn[i * K + k];
                 js[k] = j;
-                mx += pts[(int64_t)j * 3]; my += pts[(int64_t)j * 3 + 1]; mz += pts[(int64_t)j * 3 + 2];
+                mx += px - pts[(int64_t)j * 3]; my += py - pts[(int64_t)j * 3 + 1]; mz += pz - pts[(int64_t)j * 3 + 2];
             }
         float sx = 0.f, sy = 0.f, sz = 0.f;          // -(surface gradient) / K, shared by all neighbours
         if (surface) {
             const float invK = 1.0f / (float)K;
             // F.pairwise_distance(x1, x2) = || x1 - x2 + eps ||_2, eps 1e-6 (losses.py:254)
-            const float dx = px - mx * invK + pd_eps, dy = py - my * invK + pd_eps, dz = pz - mz * invK + pd_eps;
+            const float dx = mx * invK + pd_eps, dy = my * invK + pd_eps, dz = mz * invK + pd_eps;
             const float s = sqrtf(dx * dx + dy * dy + dz * dz);
             lsum = (double)s;
             if (s > 0.f) {
