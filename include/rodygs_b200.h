@@ -347,6 +347,20 @@ int rdg_pearson(const float* pred, const float* gt, int32_t height, int32_t widt
  * the reference itself has no alpha consumer (SURVEY.md §8 a12). */
 int rdg_alpha_reg(const float* alpha, int64_t n, float weight, float* out_loss, float* dL_dalpha, void* stream);
 
+/* ---- evaluation image metrics ------------------------------------------------------------------------------------ */
+
+/* MSE, PSNR, SSIM and MS-SSIM of `batch` image pairs, piqa's definitions (what the reference's evaluators report;
+ * INTEGRATION.md "Scoring held-out views"): 11-tap Gaussian window, sigma 1.5, VALID region only, averaged per channel;
+ * MS-SSIM over 5 scales joined by avg_pool2d(2, ceil_mode=True).  Not the training SSIM of rdg_losses (zero padding).
+ * pred, gt: contiguous [batch, channels, height, width]; out (device): [batch, 4] float32 = (mse, psnr, ssim, ms_ssim),
+ * psnr = 10 log10(value_range^2 / (mse + 1e-8)).  height, width >= 11; ms_ssim is NaN unless ceil(height / 16) and
+ * ceil(width / 16) are >= 11.  At most 6 launches, no float atomics: bit-identical from run to run, and row b does not
+ * depend on the other images.  workspace: 16-byte aligned, rdg_image_metrics_workspace_bytes() bytes (RDG_E_ARG with a
+ * message for a bad size).  Every argument error returns RDG_E_ARG before anything reaches the device. */
+int64_t rdg_image_metrics_workspace_bytes(int32_t batch, int32_t channels, int32_t height, int32_t width);
+int rdg_image_metrics(const float* pred, const float* gt, int32_t batch, int32_t channels, int32_t height, int32_t width,
+                      float value_range, float* out, void* workspace, int64_t workspace_bytes, void* stream);
+
 /* ---- optimiser (next row, SURVEY.md §8 f1) ------------------------------------ */
 
 /* In-place Adam over a flat fp32 parameter range (rodygs_static.py:106-149 uses

@@ -133,6 +133,9 @@ SYMBOLS = {
                                c_ptr, C.c_int64, c_ptr]),
     "rdg_losses": (C.c_int, [c_ptr, c_ptr, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_float, C.POINTER(RdgLossTerms),
                              c_ptr, c_ptr, c_ptr, C.c_int64, c_ptr]),
+    "rdg_image_metrics_workspace_bytes": (C.c_int64, [C.c_int32, C.c_int32, C.c_int32, C.c_int32]),
+    "rdg_image_metrics": (C.c_int, [c_ptr, c_ptr, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_float, c_ptr, c_ptr,
+                                    C.c_int64, c_ptr]),
     "rdg_pearson": (C.c_int, [c_ptr, c_ptr, C.c_int32, C.c_int32, c_ptr, c_ptr, C.c_int32, C.c_float, c_ptr, c_ptr,
                               c_ptr, c_ptr]),
     "rdg_adam": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, C.c_int64, C.c_float, C.c_float, C.c_float, C.c_float,

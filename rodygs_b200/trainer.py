@@ -263,6 +263,17 @@ class SplatTrainStep:
             raise ValueError(f"SplatTrainStep: {name} must be a contiguous float32 tensor of shape {tuple(shape)} on {self.params.device}, got {got}")
 
     # -- one view --------------------------------------------------------------------------------
+    def _scene_view(self, viewmatrix, projmatrix, tanfovx, tanfovy, basis_t) -> Tuple[SceneArgs, ViewArgs]:
+        deform = self.nd > 0
+        scene = SceneArgs(st=self._set("static"), dy=self._set("dynamic"), raw=True, use_deform=deform,
+                          motion_coeff=self.p("motion_coeff").view(self.nd, self.num_basis) if deform else None,
+                          time_ind=self.time_ind if deform else None, basis_t=basis_t if deform else None,
+                          table=self.p("table") if deform else None, spatial_lr_scale=self.spatial_lr_scale,
+                          frame_order=self.frame_order, frame_offsets=self.frame_offsets)
+        view = ViewArgs(height=self.H, width=self.W, tanfovx=tanfovx, tanfovy=tanfovy, scale_modifier=1.0,
+                        sh_degree=self.sh_degree, viewmatrix=viewmatrix, projmatrix=projmatrix, bg=self.bg)
+        return scene, view
+
     def forward_backward(self, viewmatrix: torch.Tensor, projmatrix: torch.Tensor, tanfovx: float, tanfovy: float,
                          basis_t: torch.Tensor, gt_image: torch.Tensor, gt_depth: Optional[torch.Tensor],
                          accumulate: bool = False, forward_only: bool = False, dcolor_slot: Optional[int] = None):
@@ -283,13 +294,7 @@ class SplatTrainStep:
             self._check_input("gt_image", gt_image, (3, self.H, self.W))
             if gt_depth is not None:
                 self._check_input("gt_depth", gt_depth, (1, self.H, self.W))
-        scene = SceneArgs(st=self._set("static"), dy=self._set("dynamic"), raw=True, use_deform=deform,
-                          motion_coeff=self.p("motion_coeff").view(self.nd, self.num_basis) if deform else None,
-                          time_ind=self.time_ind if deform else None, basis_t=basis_t if deform else None,
-                          table=self.p("table") if deform else None, spatial_lr_scale=self.spatial_lr_scale,
-                          frame_order=self.frame_order, frame_offsets=self.frame_offsets)
-        view = ViewArgs(height=self.H, width=self.W, tanfovx=tanfovx, tanfovy=tanfovy, scale_modifier=1.0,
-                        sh_degree=self.sh_degree, viewmatrix=viewmatrix, projmatrix=projmatrix, bg=self.bg)
+        scene, view = self._scene_view(viewmatrix, projmatrix, tanfovx, tanfovy, basis_t)
         self._mark("start")
         color, depth, alpha, radii, state = engine.render_forward(scene, view, stage_hook=self._mark)
         self.last_state = state
@@ -963,6 +968,54 @@ class SplatTrainStep:
         """photometric + w_p * pearson + w_local * local pearson + alpha term (device scalar)."""
         lp = self.loss_parts
         return lp[0] + self.w[2] * lp[3] + lp[4] + (self.w_local * lp[5] if self.n_local > 0 else 0.0)
+
+    # -- held-out views -------------------------------------------------------------------------------------------
+    def evaluate(self, viewmats: torch.Tensor, projmats: torch.Tensor, tanfovx, tanfovy, basis_ts: Optional[torch.Tensor],
+                 gts: torch.Tensor, value_range: float = 1.0) -> torch.Tensor:
+        """Score V views against their ground truth: [V, 4] float32 on the device, row v = (mse, psnr, ssim, ms_ssim) of view v
+        (rodygs_b200.metrics.image_metrics: the evaluation metrics, not the training SSIM of loss_parts[2]).
+
+        viewmats / projmats [V, 4, 4] in glm storage; tanfovx / tanfovy a float or a length-V sequence; basis_ts [V, K, 7]
+        the B(t) of each view (from BasisMLP.query_and_table or the table: no MLP runs here; None without dynamic
+        Gaussians); gts [V, 3, H, W].  Each view is rendered forward only and its colour clamped to [0, 1] before scoring.
+
+        Data parallel: every rank renders its shard_views() share and one sum all-reduce over the step's group gives every
+        rank the whole table; all ranks call this with the same views.  No training state changes: parameters, gradients,
+        moments, densification statistics, loss_parts, last_state / last_outputs, means2D_grad, the CUDA generator and
+        pending exchange_grads(defer_sh=True) factors stay as they were.  The views are binned with a host read of their
+        duplicate count even under config.sync_free, so that a view which overflows the buffers is re-binned here instead
+        of leaving an overflow for the next training step to raise."""
+        V = viewmats.shape[0] if torch.is_tensor(viewmats) else 0
+        if V < 1:
+            raise ValueError("SplatTrainStep.evaluate: viewmats must be a [V, 4, 4] tensor with V >= 1")
+        self._check_input("viewmats", viewmats, (V, 4, 4))
+        self._check_input("projmats", projmats, (V, 4, 4))
+        self._check_input("gts", gts, (V, 3, self.H, self.W))
+        if self.nd > 0:
+            self._check_input("basis_ts", basis_ts, (V, self.num_basis, 7))
+
+        def per_view(name, v):
+            vals = [float(t) for t in v] if hasattr(v, "__len__") else [float(v)] * V
+            if len(vals) != V:
+                raise ValueError(f"SplatTrainStep.evaluate: {name} must be a float or {V} values, got {len(vals)}")
+            return vals
+
+        fovx, fovy = per_view("tanfovx", tanfovx), per_view("tanfovy", tanfovy)
+        from .metrics import image_metrics
+        rank, world = self._dp_rank_world()
+        table = torch.zeros(V, 4, dtype=torch.float32, device=self.dev)
+        cap = engine._cap_state(self.params.device, self.ns + self.nd)
+        saved = engine.config.sync_free, cap["pending"]          # a training step's unread duplicate count stays for it
+        engine.config.sync_free, cap["pending"] = False, None
+        try:
+            for v in shard_views(V, world, rank):
+                scene, view = self._scene_view(viewmats[v], projmats[v], fovx[v], fovy[v], basis_ts[v] if self.nd > 0 else None)
+                color = engine.render_forward(scene, view)[0]
+                table[v] = image_metrics(color.clamp_(0.0, 1.0), gts[v], value_range)[0]
+        finally:
+            engine.config.sync_free, cap["pending"] = saved
+        allreduce_flat(table, None, self.pg)
+        return table
 
     # -- checkpoints -------------------------------------------------------------------------------------------
     def _check_saveable(self):
