@@ -361,6 +361,41 @@ int64_t rdg_image_metrics_workspace_bytes(int32_t batch, int32_t channels, int32
 int rdg_image_metrics(const float* pred, const float* gt, int32_t batch, int32_t channels, int32_t height, int32_t width,
                       float value_range, float* out, void* workspace, int64_t workspace_bytes, void* stream);
 
+/* ---- test-time pose refinement of a held-out camera (INTEGRATION.md "Refining held-out camera poses") ------------------ */
+
+/* Pose of one camera: param = (q_r, q_x, q_y, q_z, T_x, T_y, T_z), q the camera-to-world rotation (any norm: it is
+ * normalised), T the camera-to-world translation; V(q, T) = [[R^T, -R^T T], [0, 0, 0, 1]] with R = rot(q / |q|). */
+typedef struct RdgPoseAdam {
+    float* param;                  /* [7] updated in place */
+    float* exp_avg;                /* [7] Adam moments (zero before the first step) */
+    float* exp_avg_sq;             /* [7] */
+    int32_t* step;                 /* [1] device step counter: updates applied so far */
+    float* dL_dV;                  /* [16] glm storage, as rdg_preprocess_bwd accumulated it (RdgSceneGrad.viewmatrix); read and
+                                    * ZEROED, so that the next iteration needs no memset */
+    float* viewmatrix;             /* [16] glm storage: receives V(q, T), what the next rdg_preprocess_fwd reads */
+    float* grad;                   /* optional [7]: receives dL/d(q, T) of this call */
+    const uint32_t* num_rendered;  /* optional [2]: this iteration's RdgBins.num_rendered; [1] != 0 (binning overflow) blocks the update */
+    uint32_t* overflow;            /* [2] latch, required with num_rendered: an overflow writes {1, num_rendered[0]} */
+    double lr, beta1, beta2, eps;  /* double, like torch.optim.Adam's Python hyperparameters: 1 - beta is taken before rounding */
+    int32_t max_steps;             /* no update once *step has reached it */
+    int32_t reserved;
+} RdgPoseAdam;
+
+/* update = 0: write V(q, T) into viewmatrix, nothing else (run it once before the loop, so that every rendered V is V(q, T)).
+ * update = 1: dL/dV -> dL/d(q, T) through the normalised quaternion, then one torch.optim.Adam step (constant lr, no weight
+ * decay; bias correction from *step + 1), *step += 1 and V(q, T) of the new pose into viewmatrix.  When num_rendered[1] is
+ * set or *step >= max_steps the call applies nothing: param, moments, *step and viewmatrix stay, dL/dV is still zeroed.
+ * One warp, one launch, no host synchronisation. */
+int rdg_pose_adam(const RdgPoseAdam* args, int32_t update, void* stream);
+
+/* loss = mean((pred - gt)^2) over channels x height x width; dL_dpred = 2 (pred - gt) / n (overwritten); the loss goes to
+ * history[*step] (device step counter, the slot of the pose the image was rendered at) when 0 <= *step < max_steps.  Per-CTA
+ * float64 partials in fixed workspace slots and a fixed-order finalize, no float atomics: bit-identical from run to run.
+ * Two launches.  workspace: 8-byte aligned, rdg_l2_loss_workspace_bytes() bytes. */
+int64_t rdg_l2_loss_workspace_bytes(int32_t channels, int32_t height, int32_t width);
+int rdg_l2_loss(const float* pred, const float* gt, int32_t channels, int32_t height, int32_t width, const int32_t* step,
+                int32_t max_steps, float* history, float* dL_dpred, void* workspace, int64_t workspace_bytes, void* stream);
+
 /* ---- optimiser (next row, SURVEY.md §8 f1) ------------------------------------ */
 
 /* In-place Adam over a flat fp32 parameter range (rodygs_static.py:106-149 uses

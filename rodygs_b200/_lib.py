@@ -88,6 +88,13 @@ class RdgBasisMlp(C.Structure):
                 ("freqs_pi", c_ptr), ("basis", c_ptr), ("basis_row0", c_ptr), ("saved", c_ptr)]
 
 
+class RdgPoseAdam(C.Structure):
+    _fields_ = [("param", c_ptr), ("exp_avg", c_ptr), ("exp_avg_sq", c_ptr), ("step", c_ptr), ("dL_dV", c_ptr),
+                ("viewmatrix", c_ptr), ("grad", c_ptr), ("num_rendered", c_ptr), ("overflow", c_ptr), ("lr", C.c_double),
+                ("beta1", C.c_double), ("beta2", C.c_double), ("eps", C.c_double), ("max_steps", C.c_int32),
+                ("reserved", C.c_int32)]
+
+
 class RdgRigidity(C.Structure):
     _fields_ = [("n", C.c_int64), ("K", C.c_int32), ("num_basis", C.c_int32), ("n_frames", C.c_int32),
                 ("mode_surface", C.c_int32), ("mode_distance", C.c_int32), ("eps", C.c_float),
@@ -136,6 +143,10 @@ SYMBOLS = {
     "rdg_image_metrics_workspace_bytes": (C.c_int64, [C.c_int32, C.c_int32, C.c_int32, C.c_int32]),
     "rdg_image_metrics": (C.c_int, [c_ptr, c_ptr, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_float, c_ptr, c_ptr,
                                     C.c_int64, c_ptr]),
+    "rdg_pose_adam": (C.c_int, [C.POINTER(RdgPoseAdam), C.c_int32, c_ptr]),
+    "rdg_l2_loss_workspace_bytes": (C.c_int64, [C.c_int32, C.c_int32, C.c_int32]),
+    "rdg_l2_loss": (C.c_int, [c_ptr, c_ptr, C.c_int32, C.c_int32, C.c_int32, c_ptr, C.c_int32, c_ptr, c_ptr, c_ptr, C.c_int64,
+                              c_ptr]),
     "rdg_pearson": (C.c_int, [c_ptr, c_ptr, C.c_int32, C.c_int32, c_ptr, c_ptr, C.c_int32, C.c_float, c_ptr, c_ptr,
                               c_ptr, c_ptr]),
     "rdg_adam": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, C.c_int64, C.c_float, C.c_float, C.c_float, C.c_float,

@@ -41,6 +41,7 @@ SOURCES = {
     "rigidity.cu": [],
     "basis_mlp.cu": [],
     "metrics.cu": [],
+    "pose.cu": [],
 }
 # every header the sources include takes part in the digest, so that editing one rebuilds the library
 HEADERS = sorted(f for f in os.listdir(CSRC) if f.endswith(".cuh")) + [os.path.join("..", "..", "include", "rodygs_b200.h")]

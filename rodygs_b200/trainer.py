@@ -1017,6 +1017,43 @@ class SplatTrainStep:
         allreduce_flat(table, None, self.pg)
         return table
 
+    def refine_poses(self, viewmats: torch.Tensor, projmats: torch.Tensor, tanfovx, tanfovy, gts: torch.Tensor, lr: float,
+                     iters: int = 1000) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Test-time pose refinement of V held-out views (the reference's PoseOptimizer; rodygs_b200.pose.refine_poses) with
+        this step's static model, background and SH degree: returns (viewmats_refined [V, 4, 4] glm storage, losses [V, iters]).
+        Score them afterwards with evaluate(viewmats_refined, ...).
+
+        Arguments as for evaluate (viewmats / projmats [V, 4, 4], tanfovx / tanfovy a float or V values, gts [V, 3, H, W]);
+        lr is the constant Adam learning rate.  Data parallel: every rank refines its shard_views() share and one sum
+        all-reduce of each zero-initialised output gives every rank both tables; all ranks call this with the same views.
+        No training state changes (the same list as evaluate): the loop renders into buffers of its own."""
+        from . import pose
+        V = viewmats.shape[0] if torch.is_tensor(viewmats) else 0
+        if V < 1:
+            raise ValueError("SplatTrainStep.refine_poses: viewmats must be a [V, 4, 4] tensor with V >= 1")
+        self._check_input("viewmats", viewmats, (V, 4, 4))
+        self._check_input("projmats", projmats, (V, 4, 4))
+        self._check_input("gts", gts, (V, 3, self.H, self.W))
+        if int(iters) != iters or iters < 1:
+            raise ValueError(f"SplatTrainStep.refine_poses: iters must be an integer >= 1, got {iters}")
+        if not lr > 0 or lr == float("inf"):
+            raise ValueError(f"SplatTrainStep.refine_poses: lr must be a finite value > 0, got {lr}")
+        fovx, fovy = pose.per_view("tanfovx", tanfovx, V), pose.per_view("tanfovy", tanfovy, V)
+        pose.pose_from_viewmatrix(viewmats)              # every rank refuses a bad view, not only the one that holds it
+        rank, world = self._dp_rank_world()
+        out = torch.zeros(V, 4, 4, dtype=torch.float32, device=self.dev)
+        losses = torch.zeros(V, int(iters), dtype=torch.float32, device=self.dev)
+        mine = shard_views(V, world, rank)
+        if mine:
+            idx = torch.tensor(mine, device=self.dev)
+            static = {k: self.p(f"static.{k}") for k in PARAM_ORDER}
+            out[idx], losses[idx] = pose.refine_poses(static, self.H, self.W, self.sh_degree, self.bg, viewmats[idx].contiguous(),
+                                                      projmats[idx].contiguous(), [fovx[v] for v in mine],
+                                                      [fovy[v] for v in mine], gts[idx].contiguous(), lr, int(iters))
+        allreduce_flat(out, None, self.pg)
+        allreduce_flat(losses, None, self.pg)
+        return out, losses
+
     # -- checkpoints -------------------------------------------------------------------------------------------
     def _check_saveable(self):
         d = getattr(self, "_deferred", None)
