@@ -361,6 +361,23 @@ int64_t rdg_image_metrics_workspace_bytes(int32_t batch, int32_t channels, int32
 int rdg_image_metrics(const float* pred, const float* gt, int32_t batch, int32_t channels, int32_t height, int32_t width,
                       float value_range, float* out, void* workspace, int64_t workspace_bytes, void* stream);
 
+/* Masked PSNR and SSIM over a covisibility mask, DyCheck's mPSNR / mSSIM (the iPhone protocol; INTEGRATION.md "Scoring
+ * held-out views", recalled rather than pinned).  mask (device): contiguous [batch, height, width], shared by the channels
+ * and applied as a weight (binary in DyCheck; not validated).  out (device): [batch, 3] float32 = (mmse, mpsnr, mssim) with
+ * mmse = sum m (x - y)^2 / (channels sum m) and mpsnr = 10 log10(value_range^2 / mmse), no epsilon: an empty mask gives
+ * (NaN, NaN, 1).  mssim averages over all channels x (height - 10) x (width - 10) positions the SSIM map of a two-stage
+ * valid partial convolution of the 11-tap Gaussian (width, then height; each stage renormalised by 11 / the count of
+ * covisible taps), with the variances clipped at 0; a window without a covisible pixel scores exactly 1.  With an all-ones
+ * mask mmse and mssim are rdg_image_metrics' mse and ssim.  Values under m = 0 change no bit of the result, NaN and Inf
+ * included.  pred, gt, height, width, value_range as for rdg_image_metrics.  Two launches, no float atomics: bit-identical
+ * from run to run, and row b does not depend on the other images.  workspace: 16-byte aligned,
+ * rdg_masked_image_metrics_workspace_bytes() bytes.  Every argument error returns RDG_E_ARG before anything reaches the
+ * device. */
+int64_t rdg_masked_image_metrics_workspace_bytes(int32_t batch, int32_t channels, int32_t height, int32_t width);
+int rdg_masked_image_metrics(const float* pred, const float* gt, const float* mask, int32_t batch, int32_t channels,
+                             int32_t height, int32_t width, float value_range, float* out, void* workspace,
+                             int64_t workspace_bytes, void* stream);
+
 /* ---- test-time pose refinement of a held-out camera (INTEGRATION.md "Refining held-out camera poses") ------------------ */
 
 /* Pose of one camera: param = (q_r, q_x, q_y, q_z, T_x, T_y, T_z), q the camera-to-world rotation (any norm: it is

@@ -971,9 +971,12 @@ class SplatTrainStep:
 
     # -- held-out views -------------------------------------------------------------------------------------------
     def evaluate(self, viewmats: torch.Tensor, projmats: torch.Tensor, tanfovx, tanfovy, basis_ts: Optional[torch.Tensor],
-                 gts: torch.Tensor, value_range: float = 1.0) -> torch.Tensor:
+                 gts: torch.Tensor, value_range: float = 1.0, masks: Optional[torch.Tensor] = None) -> torch.Tensor:
         """Score V views against their ground truth: [V, 4] float32 on the device, row v = (mse, psnr, ssim, ms_ssim) of view v
-        (rodygs_b200.metrics.image_metrics: the evaluation metrics, not the training SSIM of loss_parts[2]).
+        (rodygs_b200.metrics.image_metrics: the evaluation metrics, not the training SSIM of loss_parts[2]).  With masks
+        [V, 1, H, W] (the test views' covisibility masks, any dtype masked_image_metrics takes) the table is [V, 7]: columns
+        0-3 as without masks, columns 4-6 = (mmse, mpsnr, mssim) of rodygs_b200.metrics.masked_image_metrics over the mask,
+        DyCheck's iPhone protocol.
 
         viewmats / projmats [V, 4, 4] in glm storage; tanfovx / tanfovy a float or a length-V sequence; basis_ts [V, K, 7]
         the B(t) of each view (from BasisMLP.query_and_table or the table: no MLP runs here; None without dynamic
@@ -993,6 +996,11 @@ class SplatTrainStep:
         self._check_input("gts", gts, (V, 3, self.H, self.W))
         if self.nd > 0:
             self._check_input("basis_ts", basis_ts, (V, self.num_basis, 7))
+        if masks is not None and (not torch.is_tensor(masks) or tuple(masks.shape) != (V, 1, self.H, self.W)
+                                  or masks.device != self.params.device):
+            got = f"{tuple(masks.shape)} {masks.device}" if torch.is_tensor(masks) else type(masks).__name__
+            raise ValueError(f"SplatTrainStep.evaluate: masks must be a {(V, 1, self.H, self.W)} tensor on {self.params.device}, "
+                             f"got {got}")
 
         def per_view(name, v):
             vals = [float(t) for t in v] if hasattr(v, "__len__") else [float(v)] * V
@@ -1001,17 +1009,19 @@ class SplatTrainStep:
             return vals
 
         fovx, fovy = per_view("tanfovx", tanfovx), per_view("tanfovy", tanfovy)
-        from .metrics import image_metrics
+        from .metrics import image_metrics, masked_image_metrics
         rank, world = self._dp_rank_world()
-        table = torch.zeros(V, 4, dtype=torch.float32, device=self.dev)
+        table = torch.zeros(V, 4 if masks is None else 7, dtype=torch.float32, device=self.dev)
         cap = engine._cap_state(self.params.device, self.ns + self.nd)
         saved = engine.config.sync_free, cap["pending"]          # a training step's unread duplicate count stays for it
         engine.config.sync_free, cap["pending"] = False, None
         try:
             for v in shard_views(V, world, rank):
                 scene, view = self._scene_view(viewmats[v], projmats[v], fovx[v], fovy[v], basis_ts[v] if self.nd > 0 else None)
-                color = engine.render_forward(scene, view)[0]
-                table[v] = image_metrics(color.clamp_(0.0, 1.0), gts[v], value_range)[0]
+                color = engine.render_forward(scene, view)[0].clamp_(0.0, 1.0)
+                table[v, :4] = image_metrics(color, gts[v], value_range)[0]
+                if masks is not None:
+                    table[v, 4:] = masked_image_metrics(color, gts[v], masks[v], value_range)[0]
         finally:
             engine.config.sync_free, cap["pending"] = saved
         allreduce_flat(table, None, self.pg)
