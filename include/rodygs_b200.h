@@ -600,6 +600,36 @@ int64_t rdg_basis_mlp_bwd_workspace_bytes(int32_t rows, int32_t emb_dim, int32_t
 int rdg_basis_mlp_bwd(const RdgBasisMlp* args, const float* d_basis, const float* d_basis_row0, float* d_params,
                       int32_t accumulate, void* workspace, int64_t workspace_bytes, void* stream);
 
+/* ---- LPIPS of held-out views (INTEGRATION.md "Scoring held-out views") ------------------------------------------------ */
+
+/* The lpips package's LPIPS v0.1 (lpips=True, spatial=False) with the AlexNet or VGG-16 backbone, from the user's
+ * weight files.  x' = (x / value_range - mu) / sigma per channel (mu = 0.485, 0.456, 0.406; sigma = 0.229, 0.224,
+ * 0.225), five ReLU taps of the backbone, f / (sqrt(sum_c f_c^2) + 1e-10) at every position, and
+ * lpips = sum over taps of the mean over positions of sum_c w_c (f0_c - f1_c)^2.  The convolutions run on tcgen05 tensor
+ * cores with TF32 operands (both rounded with cvt.rna: to nearest, ties away from zero) and FP32 accumulation, the
+ * arithmetic cuDNN uses for the reference's float32 convolutions by default. */
+#define RDG_LPIPS_ALEX 0
+#define RDG_LPIPS_VGG 1
+/* Floats of the packed weights of `net` (RDG_E_ARG for an unknown net). */
+int64_t rdg_lpips_packed_floats(int32_t net);
+/* Rewrite the weights, on the device, into the layout the conv kernel reads (TF32-rounded).  conv_w, conv_b: host arrays
+ * of device pointers, one per conv in network order (alex 5: features.0, 3, 6, 8, 10; vgg 13: features.0, 2, 5, 7, 10, 12,
+ * 14, 17, 19, 21, 24, 26, 28), each weight contiguous fp32 [Cout, Cin, kh, kw] as torch stores it, each bias [Cout];
+ * lin_w: 5 device pointers, lin{l}.model.1.weight [C_l].  packed (device, 16-byte aligned): packed_floats =
+ * rdg_lpips_packed_floats(net) floats.  Stream-ordered, no allocation, no host synchronisation. */
+int rdg_lpips_pack(int32_t net, const float* const* conv_w, const float* const* conv_b, const float* const* lin_w,
+                   float* packed, int64_t packed_floats, void* stream);
+/* Workspace of ONE image pair (pairs are processed in turn): two NHWC activation buffers of the pair and the head's
+ * slots.  height, width >= 31 (alex) or >= 16 (vgg), so that the last tap is not empty; RDG_E_ARG otherwise. */
+int64_t rdg_lpips_workspace_bytes(int32_t net, int32_t height, int32_t width);
+/* out (device) [batch] float32 = LPIPS of (pred[b], gt[b]); pred, gt: contiguous [batch, 3, height, width] in
+ * [0, value_range]; channels must be 3.  workspace: 256-byte aligned, rdg_lpips_workspace_bytes() bytes.  No float atomics:
+ * bit-identical from run to run, and out[b] does not depend on the other pairs.  Every argument error returns RDG_E_ARG
+ * before anything reaches the device; no allocation, no host synchronisation. */
+int rdg_lpips(const float* pred, const float* gt, int32_t batch, int32_t channels, int32_t height, int32_t width,
+              float value_range, int32_t net, const float* packed, int64_t packed_floats, float* out, void* workspace,
+              int64_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

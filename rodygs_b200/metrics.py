@@ -9,6 +9,8 @@ lower number near the borders.  piqa's conventions are recalled, not pinned agai
 """
 from __future__ import annotations
 
+import ctypes
+
 import torch
 
 from . import _lib
@@ -94,4 +96,114 @@ def masked_image_metrics(pred: torch.Tensor, gt: torch.Tensor, mask: torch.Tenso
         out = torch.empty(B, 3, dtype=torch.float32, device=x.device)
         check(lib.rdg_masked_image_metrics(ptr(x), ptr(y), ptr(m), B, C, H, W, value_range, ptr(out), ptr(ws), nbytes,
                                            _lib.stream_ptr()))
+    return out
+
+
+# ---- LPIPS ---------------------------------------------------------------------------------------------------------------
+
+# features.{i} of each torchvision backbone that is a conv, in network order, with (Cout, Cin, k); the taps' channels
+LPIPS_CONVS = {
+    "alex": [(0, 64, 3, 11), (3, 192, 64, 5), (6, 384, 192, 3), (8, 256, 384, 3), (10, 256, 256, 3)],
+    "vgg": [(0, 64, 3, 3), (2, 64, 64, 3), (5, 128, 64, 3), (7, 128, 128, 3), (10, 256, 128, 3), (12, 256, 256, 3),
+            (14, 256, 256, 3), (17, 512, 256, 3), (19, 512, 512, 3), (21, 512, 512, 3), (24, 512, 512, 3),
+            (26, 512, 512, 3), (28, 512, 512, 3)],
+}
+LPIPS_TAPS = {"alex": (64, 192, 384, 256, 256), "vgg": (64, 128, 256, 512, 512)}
+_LPIPS_NET = {"alex": 0, "vgg": 1}                 # RDG_LPIPS_ALEX, RDG_LPIPS_VGG
+_LPIPS_MIN_EDGE = {"alex": 31, "vgg": 16}         # the last tap is not empty
+
+
+class LpipsWeights:
+    """One backbone's weights packed on the device for rodygs_b200.metrics.lpips (built by load_lpips)."""
+
+    def __init__(self, net: str, packed: torch.Tensor):
+        self.net = net
+        self.packed = packed
+
+    def __repr__(self):
+        return f"LpipsWeights(net={self.net!r}, device={self.packed.device})"
+
+
+def _state_dict(fn: str, what: str, src):
+    if isinstance(src, dict):
+        return src
+    sd = torch.load(src, map_location="cpu", weights_only=True)
+    if not isinstance(sd, dict):
+        raise ValueError(f"{fn}: {what} {src!r} does not hold a state dict")
+    return sd
+
+
+def _tensor(fn: str, sd: dict, key: str, shape) -> torch.Tensor:
+    if key not in sd:
+        raise ValueError(f"{fn}: missing key {key!r}")
+    t = sd[key]
+    if not torch.is_tensor(t) or tuple(t.shape) != tuple(shape):
+        got = tuple(t.shape) if torch.is_tensor(t) else type(t).__name__
+        raise ValueError(f"{fn}: {key!r} must have shape {tuple(shape)}, got {got}")
+    return t
+
+
+def load_lpips(net: str, backbone, linear, device="cuda") -> LpipsWeights:
+    """LPIPS weights of `net` ("alex" or "vgg") from the files a run of the reference already has; nothing is downloaded.
+
+    backbone: the torchvision state dict of the backbone (e.g. alexnet-owt-7be5be79.pth, vgg16-397923af.pth) or its path;
+    the keys read are features.{i}.weight / .bias of the convs (LPIPS_CONVS), classifier.* is ignored.  linear: the lpips
+    package's heads (weights/v0.1/alex.pth, vgg.pth) or its path, keys lin{0..4}.model.1.weight [1, C_l, 1, 1].  Paths are
+    read with torch.load(map_location="cpu", weights_only=True).  A missing key or a wrong shape raises ValueError naming
+    the key.  Returns the weights packed for the conv kernels on `device` (one rdg_lpips_pack call)."""
+    fn = "load_lpips"
+    if net not in LPIPS_CONVS:
+        raise ValueError(f"{fn}: net must be 'alex' or 'vgg', got {net!r}")
+    bb, lin = _state_dict(fn, "backbone", backbone), _state_dict(fn, "linear", linear)
+    ws, bs = [], []
+    for i, cout, cin, k in LPIPS_CONVS[net]:
+        ws.append(_tensor(fn, bb, f"features.{i}.weight", (cout, cin, k, k)))
+        bs.append(_tensor(fn, bb, f"features.{i}.bias", (cout,)))
+    ls = [_tensor(fn, lin, f"lin{l}.model.1.weight", (1, c, 1, 1)) for l, c in enumerate(LPIPS_TAPS[net])]
+    dev = torch.device(device)
+    if dev.type != "cuda":
+        raise RuntimeError(f"{fn}: device is {dev}; rodygs_b200 runs on CUDA tensors only (no CPU fallback)")
+    ws, bs, ls = ([t.detach().to(device=dev, dtype=torch.float32).contiguous() for t in ts] for ts in (ws, bs, ls))
+    lib = _lib.load()
+    code = _LPIPS_NET[net]
+    n = int(lib.rdg_lpips_packed_floats(code))
+    arr = lambda ts: (ctypes.c_void_p * len(ts))(*[t.data_ptr() for t in ts])   # noqa: E731
+    with torch.cuda.device(dev):
+        packed = torch.empty(n, dtype=torch.float32, device=dev)
+        check(lib.rdg_lpips_pack(code, arr(ws), arr(bs), arr(ls), ptr(packed), n, _lib.stream_ptr()))
+    return LpipsWeights(net, packed)
+
+
+def lpips(pred: torch.Tensor, gt: torch.Tensor, weights: LpipsWeights, value_range: float = 1.0) -> torch.Tensor:
+    """LPIPS (the lpips package v0.1, lpips=True, spatial=False) of every image pair as a [B] float32 tensor on the inputs'
+    device, without a host read.
+
+    pred, gt: [3, H, W] or [B, 3, H, W] CUDA tensors of the same shape in [0, value_range]; other dtypes are converted to
+    float32.  H, W >= 31 for alex and >= 16 for vgg.  weights: from load_lpips, on the inputs' device.  The convolutions
+    run on tensor cores in TF32 (the reference's arithmetic under cuDNN's default).  Not differentiable.  The result of a
+    pair does not depend on the other pairs, and repeated calls give identical bits."""
+    if not isinstance(weights, LpipsWeights):
+        raise TypeError(f"lpips: weights must be an LpipsWeights from load_lpips, got {type(weights).__name__}")
+    for name, t in (("pred", pred), ("gt", gt)):      # shape checks first: they need no device
+        if torch.is_tensor(t) and t.dim() in (3, 4):
+            if t.shape[-3] != 3:
+                raise ValueError(f"lpips: {name} must have 3 channels, got shape {tuple(t.shape)}")
+            edge = _LPIPS_MIN_EDGE[weights.net]
+            if min(t.shape[-2:]) < edge:
+                raise ValueError(f"lpips: {name} is {t.shape[-2]}x{t.shape[-1]}; the {weights.net} backbone needs H and W "
+                                 f">= {edge}")
+    x, y, value_range = _pair("lpips", pred, gt, value_range)
+    B, Cc, H, W = x.shape
+    if weights.packed.device != x.device:
+        raise ValueError(f"lpips: weights are on {weights.packed.device} but pred on {x.device}")
+    lib = _lib.load()
+    code = _LPIPS_NET[weights.net]
+    nbytes = int(lib.rdg_lpips_workspace_bytes(code, H, W))
+    if nbytes < 0:
+        check(nbytes)
+    with torch.cuda.device(x.device):
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
+        out = torch.empty(B, dtype=torch.float32, device=x.device)
+        check(lib.rdg_lpips(ptr(x), ptr(y), B, Cc, H, W, value_range, code, ptr(weights.packed), weights.packed.numel(),
+                            ptr(out), ptr(ws), nbytes, _lib.stream_ptr()))
     return out

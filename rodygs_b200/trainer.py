@@ -971,12 +971,14 @@ class SplatTrainStep:
 
     # -- held-out views -------------------------------------------------------------------------------------------
     def evaluate(self, viewmats: torch.Tensor, projmats: torch.Tensor, tanfovx, tanfovy, basis_ts: Optional[torch.Tensor],
-                 gts: torch.Tensor, value_range: float = 1.0, masks: Optional[torch.Tensor] = None) -> torch.Tensor:
+                 gts: torch.Tensor, value_range: float = 1.0, masks: Optional[torch.Tensor] = None, lpips=None) -> torch.Tensor:
         """Score V views against their ground truth: [V, 4] float32 on the device, row v = (mse, psnr, ssim, ms_ssim) of view v
         (rodygs_b200.metrics.image_metrics: the evaluation metrics, not the training SSIM of loss_parts[2]).  With masks
         [V, 1, H, W] (the test views' covisibility masks, any dtype masked_image_metrics takes) the table is [V, 7]: columns
         0-3 as without masks, columns 4-6 = (mmse, mpsnr, mssim) of rodygs_b200.metrics.masked_image_metrics over the mask,
-        DyCheck's iPhone protocol.
+        DyCheck's iPhone protocol.  lpips: None, or one rodygs_b200.metrics.LpipsWeights or a sequence of them (the
+        reference reports alex and vgg); each adds one column after the others, in the given order, holding
+        rodygs_b200.metrics.lpips of the same clamped render: [V, 4 + L], or [V, 7 + L] with masks.
 
         viewmats / projmats [V, 4, 4] in glm storage; tanfovx / tanfovy a float or a length-V sequence; basis_ts [V, K, 7]
         the B(t) of each view (from BasisMLP.query_and_table or the table: no MLP runs here; None without dynamic
@@ -1009,9 +1011,14 @@ class SplatTrainStep:
             return vals
 
         fovx, fovy = per_view("tanfovx", tanfovx), per_view("tanfovy", tanfovy)
-        from .metrics import image_metrics, masked_image_metrics
+        from .metrics import LpipsWeights, image_metrics, lpips as lpips_metric, masked_image_metrics
+        nets = [] if lpips is None else [lpips] if isinstance(lpips, LpipsWeights) else list(lpips)
+        if not all(isinstance(w, LpipsWeights) for w in nets):
+            raise ValueError("SplatTrainStep.evaluate: lpips must be an LpipsWeights (rodygs_b200.metrics.load_lpips) or a "
+                             "sequence of them")
         rank, world = self._dp_rank_world()
-        table = torch.zeros(V, 4 if masks is None else 7, dtype=torch.float32, device=self.dev)
+        cols = 4 if masks is None else 7
+        table = torch.zeros(V, cols + len(nets), dtype=torch.float32, device=self.dev)
         cap = engine._cap_state(self.params.device, self.ns + self.nd)
         saved = engine.config.sync_free, cap["pending"]          # a training step's unread duplicate count stays for it
         engine.config.sync_free, cap["pending"] = False, None
@@ -1021,7 +1028,9 @@ class SplatTrainStep:
                 color = engine.render_forward(scene, view)[0].clamp_(0.0, 1.0)
                 table[v, :4] = image_metrics(color, gts[v], value_range)[0]
                 if masks is not None:
-                    table[v, 4:] = masked_image_metrics(color, gts[v], masks[v], value_range)[0]
+                    table[v, 4:7] = masked_image_metrics(color, gts[v], masks[v], value_range)[0]
+                for j, w in enumerate(nets):
+                    table[v, cols + j] = lpips_metric(color, gts[v], w, value_range)[0]
         finally:
             engine.config.sync_free, cap["pending"] = saved
         allreduce_flat(table, None, self.pg)
