@@ -630,6 +630,24 @@ int rdg_lpips(const float* pred, const float* gt, int32_t batch, int32_t channel
               float value_range, int32_t net, const float* packed, int64_t packed_floats, float* out, void* workspace,
               int64_t workspace_bytes, void* stream);
 
+/* Masked LPIPS over a covisibility mask, DyCheck's mLPIPS (lpips.LPIPS(spatial=True) on masked inputs, then the masked
+ * mean of the map; INTEGRATION.md "Scoring held-out views", recalled rather than pinned).  mask (device): contiguous fp32
+ * [batch, height, width], shared by the channels and applied as a weight (binary in DyCheck; not validated).  Per pair, the
+ * inputs are x_m = m != 0 ? m x : 0 (likewise y), the backbone, taps, normalisation and heads are rdg_lpips', each tap's
+ * per-position head value d_l [h_l, w_l] is upsampled to [height, width] bilinearly with align_corners = false (the scale
+ * in / out divided in float32) and the five are summed: out[b] = sum_p m_p map_p / sum_p m_p.  An empty mask gives NaN;
+ * values under m = 0 change no bit of the result, NaN and Inf included.  With an all-ones mask this is rdg_lpips only when
+ * every tap size divides the image size (vgg at 64 x 64, never alex).  Workspace of ONE pair: the activation buffers of
+ * rdg_lpips, the five tap maps and the spatial pass's slots; height, width as for rdg_lpips_workspace_bytes. */
+int64_t rdg_masked_lpips_workspace_bytes(int32_t net, int32_t height, int32_t width);
+/* out (device) [batch] float32 = masked LPIPS of (pred[b], gt[b]) under mask[b]; the other arguments as for rdg_lpips.
+ * workspace: 256-byte aligned, rdg_masked_lpips_workspace_bytes() bytes.  No float atomics: bit-identical from run to run,
+ * and out[b] does not depend on the other pairs.  Every argument error returns RDG_E_ARG before anything reaches the
+ * device; no allocation, no host synchronisation. */
+int rdg_masked_lpips(const float* pred, const float* gt, const float* mask, int32_t batch, int32_t channels, int32_t height,
+                     int32_t width, float value_range, int32_t net, const float* packed, int64_t packed_floats, float* out,
+                     void* workspace, int64_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -151,6 +151,9 @@ SYMBOLS = {
     "rdg_lpips_workspace_bytes": (C.c_int64, [C.c_int32, C.c_int32, C.c_int32]),
     "rdg_lpips": (C.c_int, [c_ptr, c_ptr, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_int32, c_ptr, C.c_int64,
                             c_ptr, c_ptr, C.c_int64, c_ptr]),
+    "rdg_masked_lpips_workspace_bytes": (C.c_int64, [C.c_int32, C.c_int32, C.c_int32]),
+    "rdg_masked_lpips": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_int32, c_ptr,
+                                   C.c_int64, c_ptr, c_ptr, C.c_int64, c_ptr]),
     "rdg_pose_adam": (C.c_int, [C.POINTER(RdgPoseAdam), C.c_int32, c_ptr]),
     "rdg_l2_loss_workspace_bytes": (C.c_int64, [C.c_int32, C.c_int32, C.c_int32]),
     "rdg_l2_loss": (C.c_int, [c_ptr, c_ptr, C.c_int32, C.c_int32, C.c_int32, c_ptr, C.c_int32, c_ptr, c_ptr, c_ptr, C.c_int64,

@@ -9,6 +9,12 @@
 // Activations ping-pong between two NHWC buffers; the head runs straight after its tap, so a tap's features are dead before
 // the next layer overwrites them.  No float atomics: bit-identical from run to run and independent of the rest of the batch.
 //
+// Masked LPIPS (rdg_masked_lpips, DyCheck's mLPIPS) runs the same pass with three changes:
+//   scale       x_m = m != 0 ? m x : 0 before the scaling, likewise y_m
+//   head        writes sum_c w_c (...)^2 of every position as float32 to the tap's map in the workspace instead of summing it
+//   spatial     one pass over the H x W pixels: sum over taps of the bilinear upsample (align_corners=False) of each map,
+//               weighted by m, into per-CTA float64 slots of sum m map and sum m; a one-CTA finalize divides the two
+//
 // Conv GEMM: M = output pixels of both images, N = Cout, K = kh kw Cin ordered (ky, kx, c), so that with NHWC activations a
 // 32-wide K slice is a contiguous run of channels of one input pixel (every Cin but the first layer's 3 is a multiple of 32;
 // the first layer gathers element-wise and its K is zero-padded to a multiple of 32).  A CTA computes a 128 x BN tile:
@@ -34,6 +40,8 @@
 #define LP_HEAD_MAX_CTAS 1184        // 8 x 148
 #define LP_TAPS 5
 #define LP_MAX_LAYERS 18
+#define LP_SPATIAL_THREADS 256
+#define LP_SPATIAL_MAX_CTAS 1184     // 8 x 148
 
 // ---- network definitions -----------------------------------------------------------------------------------------------
 
@@ -96,11 +104,16 @@ static void lp_packed_layout(const LpNet& N, LpPacked* P) {
     P->total = off;
 }
 
-// Workspace of one pair: two activation buffers (the largest NHWC tensor of the pass, both images), then the head slots.
+// Workspace of one pair: two activation buffers (the largest NHWC tensor of the pass, both images), then the head slots;
+// masked, the five tap maps and the spatial pass's slots instead of the head slots.
 struct LpWork {
     int64_t act_bytes;
-    int64_t part_off[LP_TAPS];
+    int64_t part_off[LP_TAPS];   // unmasked: [head_ctas] float64 per tap
     int head_ctas[LP_TAPS];
+    int tap_h[LP_TAPS], tap_w[LP_TAPS];
+    int64_t map_off[LP_TAPS];    // masked: [tap_h][tap_w] float32 per tap
+    int64_t spatial_off;         // masked: [2][spatial_ctas] float64 (sum m map, then sum m)
+    int spatial_ctas;
     int64_t total;
 };
 
@@ -109,24 +122,39 @@ static int lp_head_ctas(int64_t positions) {
     return (int)(need < LP_HEAD_MAX_CTAS ? need : LP_HEAD_MAX_CTAS);
 }
 
-static void lp_work_layout(const LpNet& N, int H, int W, LpWork* Wk) {
+static void lp_work_layout(const LpNet& N, int H, int W, bool masked, LpWork* Wk) {
     int64_t big = 2LL * H * W * 3;
     int h = H, w = W, t = 0;
-    int64_t tap_pos[LP_TAPS];
     for (int i = 0; i < N.n; ++i) {
         const LpLayer& L = N.layers[i];
         h = (h + 2 * L.p - L.k) / L.s + 1;
         w = (w + 2 * L.p - L.k) / L.s + 1;
         const int64_t n = 2LL * h * w * L.cout;
         if (n > big) big = n;
-        if (L.conv && L.tap) tap_pos[t++] = (int64_t)h * w;
+        if (L.conv && L.tap) {
+            Wk->tap_h[t] = h;
+            Wk->tap_w[t] = w;
+            ++t;
+        }
     }
     Wk->act_bytes = rdg_align_up(big * (int64_t)sizeof(float), 256);
     int64_t off = 2 * Wk->act_bytes;
     for (int i = 0; i < LP_TAPS; ++i) {
-        Wk->head_ctas[i] = lp_head_ctas(tap_pos[i]);
-        Wk->part_off[i] = off;
-        off += rdg_align_up((int64_t)Wk->head_ctas[i] * (int64_t)sizeof(double), 256);
+        const int64_t positions = (int64_t)Wk->tap_h[i] * Wk->tap_w[i];
+        Wk->head_ctas[i] = lp_head_ctas(positions);
+        if (masked) {
+            Wk->map_off[i] = off;
+            off += rdg_align_up(positions * (int64_t)sizeof(float), 256);
+        } else {
+            Wk->part_off[i] = off;
+            off += rdg_align_up((int64_t)Wk->head_ctas[i] * (int64_t)sizeof(double), 256);
+        }
+    }
+    if (masked) {
+        const int64_t need = ((int64_t)H * W + LP_SPATIAL_THREADS - 1) / LP_SPATIAL_THREADS;
+        Wk->spatial_ctas = (int)(need < LP_SPATIAL_MAX_CTAS ? need : LP_SPATIAL_MAX_CTAS);
+        Wk->spatial_off = off;
+        off += rdg_align_up(2LL * Wk->spatial_ctas * (int64_t)sizeof(double), 256);
     }
     Wk->total = off;
 }
@@ -359,17 +387,23 @@ __global__ void lpips_copy_kernel(const float* __restrict__ src, float* __restri
 
 // ---- scaling, pooling, head, finalize ----------------------------------------------------------------------------------
 
-// pred, gt [3, H, W] -> out NHWC [2][H][W][3], (x / R - mu_c) / sigma_c
-__global__ void lpips_scale_kernel(const float* __restrict__ pred, const float* __restrict__ gt, int H, int W, float R,
-                                   float* __restrict__ out) {
+// pred, gt [3, H, W] -> out NHWC [2][H][W][3], (x / R - mu_c) / sigma_c; with a mask [H, W] (NULL: none), x is first
+// replaced by m != 0 ? m x : 0, so values under m = 0 take no part, NaN included
+__global__ void lpips_scale_kernel(const float* __restrict__ pred, const float* __restrict__ gt,
+                                   const float* __restrict__ mask, int H, int W, float R, float* __restrict__ out) {
     const int64_t hw = (int64_t)H * W;
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i >= 2 * hw) return;
     const float* src = i < hw ? pred : gt;
     const int64_t p = i < hw ? i : i - hw;
+    const float m = mask ? mask[p] : 1.f;
     const float mu[3] = {0.485f, 0.456f, 0.406f}, sd[3] = {0.229f, 0.224f, 0.225f};
 #pragma unroll
-    for (int ch = 0; ch < 3; ++ch) out[i * 3 + ch] = (src[ch * hw + p] / R - mu[ch]) / sd[ch];
+    for (int ch = 0; ch < 3; ++ch) {
+        float v = src[ch * hw + p];
+        if (mask) v = m != 0.f ? m * v : 0.f;
+        out[i * 3 + ch] = (v / R - mu[ch]) / sd[ch];
+    }
 }
 
 // NHWC [2][H][W][C] -> [2][Ho][Wo][C], window k, stride s, no padding, floor
@@ -402,10 +436,12 @@ __device__ __forceinline__ float lp_warp_sum(float v) {
     return v;
 }
 
-// f NHWC [2][positions][C] (C a multiple of 32, <= 512), one warp per position:
-// part[blockIdx.x] = sum over the CTA's positions of sum_c w_c (f0_c / (|f0| + 1e-10) - f1_c / (|f1| + 1e-10))^2
+// f NHWC [2][positions][C] (C a multiple of 32, <= 512), one warp per position, d[p] = sum_c w_c (f0_c / (|f0| + 1e-10) -
+// f1_c / (|f1| + 1e-10))^2:  part[blockIdx.x] = sum over the CTA's positions of d[p]; MAP: map[p] = d[p] (part unused)
+template <bool MAP>
 __global__ void __launch_bounds__(LP_HEAD_THREADS) lpips_head_kernel(const float* __restrict__ f, const float* __restrict__ lin,
-                                                                     int64_t positions, int C, double* __restrict__ part) {
+                                                                     int64_t positions, int C, double* __restrict__ part,
+                                                                     float* __restrict__ map) {
     __shared__ double red[LP_HEAD_THREADS / 32];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, per = C / 32;
     double acc = 0.0;
@@ -432,14 +468,21 @@ __global__ void __launch_bounds__(LP_HEAD_THREADS) lpips_head_kernel(const float
                 const float diff = va[i] / na - vb[i] / nb;
                 d = fmaf(lin[lane + 32 * i], diff * diff, d);
             }
-        acc += (double)lp_warp_sum(d);
+        const float dp = lp_warp_sum(d);
+        if constexpr (MAP) {
+            if (lane == 0) map[p] = dp;
+        } else {
+            acc += (double)dp;
+        }
     }
-    if (lane == 0) red[warp] = acc;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        double t = 0.0;
-        for (int w = 0; w < LP_HEAD_THREADS / 32; ++w) t += red[w];
-        part[blockIdx.x] = t;
+    if constexpr (!MAP) {
+        if (lane == 0) red[warp] = acc;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            double t = 0.0;
+            for (int w = 0; w < LP_HEAD_THREADS / 32; ++w) t += red[w];
+            part[blockIdx.x] = t;
+        }
     }
 }
 
@@ -465,6 +508,92 @@ __global__ void __launch_bounds__(256) lpips_finalize_kernel(LpFinal fin, float*
         __syncthreads();
     }
     if (threadIdx.x == 0) *out = (float)total;
+}
+
+struct LpSpatial {
+    const float* map[LP_TAPS];       // [h][w] float32
+    int h[LP_TAPS], w[LP_TAPS];
+    float sy[LP_TAPS], sx[LP_TAPS];  // in / out per axis, divided in float32 as ATen does for float32 input
+};
+
+// One axis of nn.Upsample(mode="bilinear", align_corners=False): src = max(scale (dst + 0.5) - 0.5, 0), taps i0 = floor(src)
+// and i1 = min(i0 + 1, in - 1) with weights 1 - l1 and l1 = src - i0
+__device__ __forceinline__ void lp_bilinear_axis(float scale, int dst, int in, int* i0, int* i1, float* l1) {
+    const float src = fmaxf(scale * ((float)dst + 0.5f) - 0.5f, 0.f);
+    *i0 = (int)src;   // src >= 0: truncation is floor
+    *i1 = *i0 < in - 1 ? *i0 + 1 : *i0;
+    *l1 = src - (float)*i0;
+}
+
+// mask [H][W]: part[blockIdx.x] = sum over the CTA's pixels of m map, part[gridDim.x + blockIdx.x] = sum of m, with map the
+// float32 sum over taps (in tap order) of each upsampled tap map.  Pixels with m = 0 are skipped: they add nothing to either
+// sum.  Fixed pixel-to-thread assignment and a fixed-order reduction: no atomics.
+__global__ void __launch_bounds__(LP_SPATIAL_THREADS) lpips_spatial_kernel(const LpSpatial sp, const float* __restrict__ mask,
+                                                                           int H, int W, double* __restrict__ part) {
+    __shared__ double red[2][LP_SPATIAL_THREADS / 32];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int hw = H * W;   // <= 2^26 (lp_check_size): 32-bit pixel indices
+    double am = 0.0, an = 0.0;
+    for (int p = blockIdx.x * LP_SPATIAL_THREADS + threadIdx.x; p < hw; p += gridDim.x * LP_SPATIAL_THREADS) {
+        const float m = __ldg(mask + p);
+        if (m == 0.f) continue;
+        const int y = p / W, x = p - y * W;
+        float v = 0.f;
+#pragma unroll
+        for (int l = 0; l < LP_TAPS; ++l) {
+            int y0, y1, x0, x1;
+            float ly1, lx1;
+            lp_bilinear_axis(sp.sy[l], y, sp.h[l], &y0, &y1, &ly1);
+            lp_bilinear_axis(sp.sx[l], x, sp.w[l], &x0, &x1, &lx1);
+            const float ly0 = 1.f - ly1, lx0 = 1.f - lx1;
+            const float* r0 = sp.map[l] + (int64_t)y0 * sp.w[l];
+            const float* r1 = sp.map[l] + (int64_t)y1 * sp.w[l];
+            v += ly0 * (lx0 * __ldg(r0 + x0) + lx1 * __ldg(r0 + x1)) + ly1 * (lx0 * __ldg(r1 + x0) + lx1 * __ldg(r1 + x1));
+        }
+        am += (double)m * (double)v;
+        an += (double)m;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        am += __shfl_xor_sync(0xffffffffu, am, o);
+        an += __shfl_xor_sync(0xffffffffu, an, o);
+    }
+    if (lane == 0) {
+        red[0][warp] = am;
+        red[1][warp] = an;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double a = 0.0, n = 0.0;
+        for (int w = 0; w < LP_SPATIAL_THREADS / 32; ++w) {
+            a += red[0][w];
+            n += red[1][w];
+        }
+        part[blockIdx.x] = a;
+        part[gridDim.x + blockIdx.x] = n;
+    }
+}
+
+// part [2][ctas] -> out = (sum of part[0]) / (sum of part[1]), each summed in a fixed order; an empty mask gives 0 / 0 = NaN
+__global__ void __launch_bounds__(256) lpips_masked_finalize_kernel(const double* __restrict__ part, int ctas,
+                                                                    float* __restrict__ out) {
+    __shared__ double sh[2][256];
+    double a = 0.0, n = 0.0;
+    for (int i = threadIdx.x; i < ctas; i += 256) {
+        a += part[i];
+        n += part[ctas + i];
+    }
+    sh[0][threadIdx.x] = a;
+    sh[1][threadIdx.x] = n;
+    __syncthreads();
+    for (int s = 128; s > 0; s >>= 1) {
+        if (threadIdx.x < s) {
+            sh[0][threadIdx.x] += sh[0][threadIdx.x + s];
+            sh[1][threadIdx.x] += sh[1][threadIdx.x + s];
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) *out = (float)(sh[0][0] / sh[1][0]);
 }
 
 // ---- host entry points -------------------------------------------------------------------------------------------------
@@ -532,55 +661,101 @@ static int lp_check_size(const char* fn, const LpNet& N, int32_t height, int32_t
     return RDG_OK;
 }
 
-extern "C" int64_t rdg_lpips_workspace_bytes(int32_t net, int32_t height, int32_t width) {
+static int64_t lp_workspace_bytes(const char* fn, int32_t net, int32_t height, int32_t width, bool masked) {
     LpNet N;
-    if (!lp_net(net, &N)) { rdg_set_error("%s: unknown net %d (RDG_LPIPS_ALEX or RDG_LPIPS_VGG)", __func__, net); return RDG_E_ARG; }
-    const int rc = lp_check_size(__func__, N, height, width);
+    if (!lp_net(net, &N)) { rdg_set_error("%s: unknown net %d (RDG_LPIPS_ALEX or RDG_LPIPS_VGG)", fn, net); return RDG_E_ARG; }
+    const int rc = lp_check_size(fn, N, height, width);
     if (rc != RDG_OK) return rc;
     LpWork Wk;
-    lp_work_layout(N, height, width, &Wk);
+    lp_work_layout(N, height, width, masked, &Wk);
     return Wk.total;
 }
 
-extern "C" int rdg_lpips(const float* pred, const float* gt, int32_t batch, int32_t channels, int32_t height, int32_t width,
-                         float value_range, int32_t net, const float* packed, int64_t packed_floats, float* out, void* workspace,
-                         int64_t workspace_bytes, void* stream) {
-    RDG_CHECK_ARG(pred, "pred is NULL");
-    RDG_CHECK_ARG(gt, "gt is NULL");
-    RDG_CHECK_ARG(packed, "packed is NULL");
-    RDG_CHECK_ARG(out, "out is NULL");
-    RDG_CHECK_ARG(workspace, "workspace is NULL");
+extern "C" int64_t rdg_lpips_workspace_bytes(int32_t net, int32_t height, int32_t width) {
+    return lp_workspace_bytes(__func__, net, height, width, false);
+}
+
+extern "C" int64_t rdg_masked_lpips_workspace_bytes(int32_t net, int32_t height, int32_t width) {
+    return lp_workspace_bytes(__func__, net, height, width, true);
+}
+
+#define LP_ARG(cond, msg)                                          \
+    do {                                                           \
+        if (!(cond)) {                                             \
+            rdg_set_error("%s: %s", fn, msg);                      \
+            return RDG_E_ARG;                                      \
+        }                                                          \
+    } while (0)
+
+#define LP_LAUNCHED()                                                                   \
+    do {                                                                                \
+        cudaError_t e__ = cudaGetLastError();                                           \
+        if (e__ != cudaSuccess) {                                                       \
+            rdg_set_error("%s: CUDA error: %s", fn, cudaGetErrorString(e__));           \
+            return RDG_E_CUDA;                                                          \
+        }                                                                               \
+    } while (0)
+
+// rdg_lpips (mask == NULL) and rdg_masked_lpips: checks every argument, then runs the pairs in turn
+static int lp_score(const char* fn, bool masked, const float* pred, const float* gt, const float* mask, int32_t batch,
+                    int32_t channels, int32_t height, int32_t width, float value_range, int32_t net, const float* packed,
+                    int64_t packed_floats, float* out, void* workspace, int64_t workspace_bytes, void* stream) {
+    LP_ARG(pred, "pred is NULL");
+    LP_ARG(gt, "gt is NULL");
+    if (masked) LP_ARG(mask, "mask is NULL");
+    LP_ARG(packed, "packed is NULL");
+    LP_ARG(out, "out is NULL");
+    LP_ARG(workspace, "workspace is NULL");
     LpNet N;
-    if (!lp_net(net, &N)) { rdg_set_error("%s: unknown net %d (RDG_LPIPS_ALEX or RDG_LPIPS_VGG)", __func__, net); return RDG_E_ARG; }
-    RDG_CHECK_ARG(batch >= 1, "batch must be >= 1");
-    RDG_CHECK_ARG(channels == 3, "channels must be 3 (LPIPS takes RGB images)");
-    const int rc = lp_check_size(__func__, N, height, width);
+    if (!lp_net(net, &N)) { rdg_set_error("%s: unknown net %d (RDG_LPIPS_ALEX or RDG_LPIPS_VGG)", fn, net); return RDG_E_ARG; }
+    LP_ARG(batch >= 1, "batch must be >= 1");
+    LP_ARG(channels == 3, "channels must be 3 (LPIPS takes RGB images)");
+    const int rc = lp_check_size(fn, N, height, width);
     if (rc != RDG_OK) return rc;
-    RDG_CHECK_ARG(value_range > 0.0f && isfinite(value_range), "value_range must be a finite value > 0");
+    LP_ARG(value_range > 0.0f && isfinite(value_range), "value_range must be a finite value > 0");
     LpPacked P;
     lp_packed_layout(N, &P);
-    RDG_CHECK_ARG(packed_floats == P.total, "packed_floats is not rdg_lpips_packed_floats(net)");
-    RDG_CHECK_ARG(((uintptr_t)packed & 15) == 0, "packed must be 16-byte aligned");
+    LP_ARG(packed_floats == P.total, "packed_floats is not rdg_lpips_packed_floats(net)");
+    LP_ARG(((uintptr_t)packed & 15) == 0, "packed must be 16-byte aligned");
     LpWork Wk;
-    lp_work_layout(N, height, width, &Wk);
-    RDG_CHECK_ARG(workspace_bytes >= Wk.total, "workspace_bytes is smaller than rdg_lpips_workspace_bytes()");
-    RDG_CHECK_ARG(((uintptr_t)workspace & 255) == 0, "workspace must be 256-byte aligned");
+    lp_work_layout(N, height, width, masked, &Wk);
+    LP_ARG(workspace_bytes >= Wk.total, masked ? "workspace_bytes is smaller than rdg_masked_lpips_workspace_bytes()"
+                                               : "workspace_bytes is smaller than rdg_lpips_workspace_bytes()");
+    LP_ARG(((uintptr_t)workspace & 255) == 0, "workspace must be 256-byte aligned");
 
     cudaStream_t s = (cudaStream_t)stream;
     char* ws = (char*)workspace;
     float* act[2] = {(float*)ws, (float*)(ws + Wk.act_bytes)};
-    RDG_CUDA(cudaFuncSetAttribute(lpips_conv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kConvSmem));
-    LpFinal fin = {};
-    for (int l = 0; l < LP_TAPS; ++l) {
-        fin.part[l] = (const double*)(ws + Wk.part_off[l]);
-        fin.ctas[l] = Wk.head_ctas[l];
+    {
+        const cudaError_t e = cudaFuncSetAttribute(lpips_conv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kConvSmem);
+        if (e != cudaSuccess) {
+            rdg_set_error("%s: cudaFuncSetAttribute(lpips_conv_kernel) failed: %s", fn, cudaGetErrorString(e));
+            return RDG_E_CUDA;
+        }
     }
+    LpFinal fin = {};
+    LpSpatial sp = {};
+    for (int l = 0; l < LP_TAPS; ++l) {
+        if (masked) {
+            sp.map[l] = (const float*)(ws + Wk.map_off[l]);
+            sp.h[l] = Wk.tap_h[l];
+            sp.w[l] = Wk.tap_w[l];
+            sp.sy[l] = (float)Wk.tap_h[l] / (float)height;
+            sp.sx[l] = (float)Wk.tap_w[l] / (float)width;
+        } else {
+            fin.part[l] = (const double*)(ws + Wk.part_off[l]);
+            fin.ctas[l] = Wk.head_ctas[l];
+            fin.positions[l] = (double)Wk.tap_h[l] * Wk.tap_w[l];
+        }
+    }
+    double* spatial_part = masked ? (double*)(ws + Wk.spatial_off) : nullptr;
     const int64_t hw = (int64_t)height * width;
     int launches = 0;
     for (int b = 0; b < batch; ++b) {
-        lpips_scale_kernel<<<(unsigned)((2 * hw + 255) / 256), 256, 0, s>>>(pred + b * 3 * hw, gt + b * 3 * hw, height, width,
+        lpips_scale_kernel<<<(unsigned)((2 * hw + 255) / 256), 256, 0, s>>>(pred + b * 3 * hw, gt + b * 3 * hw,
+                                                                              masked ? mask + b * hw : nullptr, height, width,
                                                                               value_range, act[0]);
-        RDG_CHECK_LAUNCH();
+        LP_LAUNCHED();
         ++launches;
         int cur = 0, h = height, w = width, t = 0;
         for (int i = 0; i < N.n; ++i) {
@@ -600,13 +775,16 @@ extern "C" int rdg_lpips(const float* pred, const float* gt, int32_t batch, int3
                 c.ntiles = L.cout / c.bn;
                 const int64_t ctas = (int64_t)rdg_div_up(c.M, LP_BM) * c.ntiles;
                 lpips_conv_kernel<<<(unsigned)ctas, LP_THREADS, kConvSmem, s>>>(c);
-                RDG_CHECK_LAUNCH();
+                LP_LAUNCHED();
                 ++launches;
                 if (L.tap) {
-                    lpips_head_kernel<<<Wk.head_ctas[t], LP_HEAD_THREADS, 0, s>>>(act[cur ^ 1], packed + P.lin_off[t],
-                                                                                 (int64_t)ho * wo, L.cout, (double*)fin.part[t]);
-                    RDG_CHECK_LAUNCH();
-                    fin.positions[t] = (double)ho * wo;
+                    if (masked)
+                        lpips_head_kernel<true><<<Wk.head_ctas[t], LP_HEAD_THREADS, 0, s>>>(
+                            act[cur ^ 1], packed + P.lin_off[t], (int64_t)ho * wo, L.cout, nullptr, (float*)sp.map[t]);
+                    else
+                        lpips_head_kernel<false><<<Wk.head_ctas[t], LP_HEAD_THREADS, 0, s>>>(
+                            act[cur ^ 1], packed + P.lin_off[t], (int64_t)ho * wo, L.cout, (double*)fin.part[t], nullptr);
+                    LP_LAUNCHED();
                     ++launches;
                     ++t;
                 }
@@ -614,17 +792,39 @@ extern "C" int rdg_lpips(const float* pred, const float* gt, int32_t batch, int3
                 const int64_t n = 2LL * ho * wo * (L.cin / 4);
                 lpips_pool_kernel<<<(unsigned)((n + 255) / 256 < 8192 ? (n + 255) / 256 : 8192), 256, 0, s>>>(
                     (const float4*)act[cur], (float4*)act[cur ^ 1], h, w, L.cin / 4, ho, wo, L.k, L.s);
-                RDG_CHECK_LAUNCH();
+                LP_LAUNCHED();
                 ++launches;
             }
             cur ^= 1;
             h = ho;
             w = wo;
         }
-        lpips_finalize_kernel<<<1, 256, 0, s>>>(fin, out + b);
-        RDG_CHECK_LAUNCH();
-        ++launches;
+        if (masked) {
+            lpips_spatial_kernel<<<Wk.spatial_ctas, LP_SPATIAL_THREADS, 0, s>>>(sp, mask + b * hw, height, width, spatial_part);
+            LP_LAUNCHED();
+            lpips_masked_finalize_kernel<<<1, 256, 0, s>>>(spatial_part, Wk.spatial_ctas, out + b);
+            LP_LAUNCHED();
+            launches += 2;
+        } else {
+            lpips_finalize_kernel<<<1, 256, 0, s>>>(fin, out + b);
+            LP_LAUNCHED();
+            ++launches;
+        }
     }
     rdg_count_launches(launches);
     return RDG_OK;
+}
+
+extern "C" int rdg_lpips(const float* pred, const float* gt, int32_t batch, int32_t channels, int32_t height, int32_t width,
+                         float value_range, int32_t net, const float* packed, int64_t packed_floats, float* out, void* workspace,
+                         int64_t workspace_bytes, void* stream) {
+    return lp_score(__func__, false, pred, gt, nullptr, batch, channels, height, width, value_range, net, packed, packed_floats,
+                    out, workspace, workspace_bytes, stream);
+}
+
+extern "C" int rdg_masked_lpips(const float* pred, const float* gt, const float* mask, int32_t batch, int32_t channels,
+                                int32_t height, int32_t width, float value_range, int32_t net, const float* packed,
+                                int64_t packed_floats, float* out, void* workspace, int64_t workspace_bytes, void* stream) {
+    return lp_score(__func__, true, pred, gt, mask, batch, channels, height, width, value_range, net, packed, packed_floats, out,
+                    workspace, workspace_bytes, stream);
 }

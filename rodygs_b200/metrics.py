@@ -1,5 +1,6 @@
-"""Evaluation image metrics on the device: MSE, PSNR, SSIM and MS-SSIM in one fused pass per scale (rdg_image_metrics), and
-their masked forms over a covisibility mask, mPSNR and mSSIM (rdg_masked_image_metrics).
+"""Evaluation image metrics on the device: MSE, PSNR, SSIM and MS-SSIM in one fused pass per scale (rdg_image_metrics),
+their masked forms over a covisibility mask, mPSNR and mSSIM (rdg_masked_image_metrics), LPIPS (rdg_lpips) and its masked
+form, mLPIPS (rdg_masked_lpips).
 
 These are the metrics the reference reports for held-out views (RoDyGSEvaluator.eval, VizScoreEvaluator, through piqa):
 an 11x11 Gaussian window (sigma 1.5) over the VALID region only, averaged per channel, and MS-SSIM over five scales.  They
@@ -80,13 +81,8 @@ def masked_image_metrics(pred: torch.Tensor, gt: torch.Tensor, mask: torch.Tenso
         raise TypeError(f"masked_image_metrics: mask must be a tensor, got {type(mask).__name__}")
     if not mask.is_cuda:
         raise RuntimeError(f"masked_image_metrics: mask is on {mask.device}; rodygs_b200 runs on CUDA tensors only (no CPU fallback)")
-    want = (B, 1, H, W) if pred.dim() == 4 else (1, H, W)
-    if tuple(mask.shape) != want:
-        raise ValueError(f"masked_image_metrics: mask must have shape {want} for pred of shape {tuple(pred.shape)}, "
-                         f"got {tuple(mask.shape)}")
-    if mask.device != x.device:
-        raise ValueError(f"masked_image_metrics: mask is on {mask.device} but pred on {x.device}")
-    m = mask.detach().to(torch.float32).reshape(B, H, W).contiguous()
+    _mask_shape("masked_image_metrics", mask, pred)
+    m = _mask_on("masked_image_metrics", mask, x)
     lib = _lib.load()
     nbytes = int(lib.rdg_masked_image_metrics_workspace_bytes(B, C, H, W))
     if nbytes < 0:
@@ -97,6 +93,22 @@ def masked_image_metrics(pred: torch.Tensor, gt: torch.Tensor, mask: torch.Tenso
         check(lib.rdg_masked_image_metrics(ptr(x), ptr(y), ptr(m), B, C, H, W, value_range, ptr(out), ptr(ws), nbytes,
                                            _lib.stream_ptr()))
     return out
+
+
+def _mask_shape(fn: str, mask: torch.Tensor, pred: torch.Tensor):
+    """mask must be [1, H, W] for pred [C, H, W] and [B, 1, H, W] for pred [B, C, H, W]."""
+    H, W = pred.shape[-2:]
+    want = (pred.shape[0], 1, H, W) if pred.dim() == 4 else (1, H, W)
+    if tuple(mask.shape) != want:
+        raise ValueError(f"{fn}: mask must have shape {want} for pred of shape {tuple(pred.shape)}, got {tuple(mask.shape)}")
+
+
+def _mask_on(fn: str, mask: torch.Tensor, x: torch.Tensor) -> torch.Tensor:
+    """The checked mask on x's device as contiguous float32 [B, H, W]."""
+    if mask.device != x.device:
+        raise ValueError(f"{fn}: mask is on {mask.device} but pred on {x.device}")
+    B, _, H, W = x.shape
+    return mask.detach().to(torch.float32).reshape(B, H, W).contiguous()
 
 
 # ---- LPIPS ---------------------------------------------------------------------------------------------------------------
@@ -174,6 +186,20 @@ def load_lpips(net: str, backbone, linear, device="cuda") -> LpipsWeights:
     return LpipsWeights(net, packed)
 
 
+def _lpips_shapes(fn: str, pred, gt, weights):
+    """The checks of lpips / masked_lpips that need no device: the weights' type, 3 channels, the backbone's least size."""
+    if not isinstance(weights, LpipsWeights):
+        raise TypeError(f"{fn}: weights must be an LpipsWeights from load_lpips, got {type(weights).__name__}")
+    for name, t in (("pred", pred), ("gt", gt)):
+        if torch.is_tensor(t) and t.dim() in (3, 4):
+            if t.shape[-3] != 3:
+                raise ValueError(f"{fn}: {name} must have 3 channels, got shape {tuple(t.shape)}")
+            edge = _LPIPS_MIN_EDGE[weights.net]
+            if min(t.shape[-2:]) < edge:
+                raise ValueError(f"{fn}: {name} is {t.shape[-2]}x{t.shape[-1]}; the {weights.net} backbone needs H and W "
+                                 f">= {edge}")
+
+
 def lpips(pred: torch.Tensor, gt: torch.Tensor, weights: LpipsWeights, value_range: float = 1.0) -> torch.Tensor:
     """LPIPS (the lpips package v0.1, lpips=True, spatial=False) of every image pair as a [B] float32 tensor on the inputs'
     device, without a host read.
@@ -182,16 +208,7 @@ def lpips(pred: torch.Tensor, gt: torch.Tensor, weights: LpipsWeights, value_ran
     float32.  H, W >= 31 for alex and >= 16 for vgg.  weights: from load_lpips, on the inputs' device.  The convolutions
     run on tensor cores in TF32 (the reference's arithmetic under cuDNN's default).  Not differentiable.  The result of a
     pair does not depend on the other pairs, and repeated calls give identical bits."""
-    if not isinstance(weights, LpipsWeights):
-        raise TypeError(f"lpips: weights must be an LpipsWeights from load_lpips, got {type(weights).__name__}")
-    for name, t in (("pred", pred), ("gt", gt)):      # shape checks first: they need no device
-        if torch.is_tensor(t) and t.dim() in (3, 4):
-            if t.shape[-3] != 3:
-                raise ValueError(f"lpips: {name} must have 3 channels, got shape {tuple(t.shape)}")
-            edge = _LPIPS_MIN_EDGE[weights.net]
-            if min(t.shape[-2:]) < edge:
-                raise ValueError(f"lpips: {name} is {t.shape[-2]}x{t.shape[-1]}; the {weights.net} backbone needs H and W "
-                                 f">= {edge}")
+    _lpips_shapes("lpips", pred, gt, weights)
     x, y, value_range = _pair("lpips", pred, gt, value_range)
     B, Cc, H, W = x.shape
     if weights.packed.device != x.device:
@@ -206,4 +223,43 @@ def lpips(pred: torch.Tensor, gt: torch.Tensor, weights: LpipsWeights, value_ran
         out = torch.empty(B, dtype=torch.float32, device=x.device)
         check(lib.rdg_lpips(ptr(x), ptr(y), B, Cc, H, W, value_range, code, ptr(weights.packed), weights.packed.numel(),
                             ptr(out), ptr(ws), nbytes, _lib.stream_ptr()))
+    return out
+
+
+def masked_lpips(pred: torch.Tensor, gt: torch.Tensor, mask: torch.Tensor, weights: LpipsWeights,
+                 value_range: float = 1.0) -> torch.Tensor:
+    """Masked LPIPS over a covisibility mask, DyCheck's mLPIPS (the iPhone protocol; DyCheck uses alex), of every image pair
+    as a [B] float32 tensor on the inputs' device, without a host read.
+
+    pred, gt, weights and value_range as for lpips; mask as for masked_image_metrics ([1, H, W] or [B, 1, H, W], shared by
+    the channels; bool, uint8, half and double converted to float32; applied as a weight, not validated).  Both images are
+    masked first (x_m = m x where m != 0, else 0), the lpips head of every tap position is upsampled bilinearly
+    (align_corners=False) to H x W and summed over the taps, and the result is sum m map / sum m.  An empty mask gives NaN;
+    values where the mask is 0 change no bit of the result (NaN and Inf included).  With an all-ones mask this equals lpips
+    only where every tap size divides the image size (vgg at 64x64): bilinear upsampling of a 15x15 alex tap to 64x64 does
+    not keep its mean.  Not differentiable.  The result of a pair does not depend on the other pairs, and repeated calls
+    give identical bits."""
+    fn = "masked_lpips"
+    _lpips_shapes(fn, pred, gt, weights)
+    if not torch.is_tensor(mask):
+        raise TypeError(f"{fn}: mask must be a tensor, got {type(mask).__name__}")
+    if torch.is_tensor(pred) and pred.dim() in (3, 4):
+        _mask_shape(fn, mask, pred)
+    x, y, value_range = _pair(fn, pred, gt, value_range)
+    if not mask.is_cuda:
+        raise RuntimeError(f"{fn}: mask is on {mask.device}; rodygs_b200 runs on CUDA tensors only (no CPU fallback)")
+    m = _mask_on(fn, mask, x)
+    B, Cc, H, W = x.shape
+    if weights.packed.device != x.device:
+        raise ValueError(f"{fn}: weights are on {weights.packed.device} but pred on {x.device}")
+    lib = _lib.load()
+    code = _LPIPS_NET[weights.net]
+    nbytes = int(lib.rdg_masked_lpips_workspace_bytes(code, H, W))
+    if nbytes < 0:
+        check(nbytes)
+    with torch.cuda.device(x.device):
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
+        out = torch.empty(B, dtype=torch.float32, device=x.device)
+        check(lib.rdg_masked_lpips(ptr(x), ptr(y), ptr(m), B, Cc, H, W, value_range, code, ptr(weights.packed),
+                                   weights.packed.numel(), ptr(out), ptr(ws), nbytes, _lib.stream_ptr()))
     return out

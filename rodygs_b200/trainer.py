@@ -971,14 +971,18 @@ class SplatTrainStep:
 
     # -- held-out views -------------------------------------------------------------------------------------------
     def evaluate(self, viewmats: torch.Tensor, projmats: torch.Tensor, tanfovx, tanfovy, basis_ts: Optional[torch.Tensor],
-                 gts: torch.Tensor, value_range: float = 1.0, masks: Optional[torch.Tensor] = None, lpips=None) -> torch.Tensor:
+                 gts: torch.Tensor, value_range: float = 1.0, masks: Optional[torch.Tensor] = None, lpips=None,
+                 masked_lpips=None) -> torch.Tensor:
         """Score V views against their ground truth: [V, 4] float32 on the device, row v = (mse, psnr, ssim, ms_ssim) of view v
         (rodygs_b200.metrics.image_metrics: the evaluation metrics, not the training SSIM of loss_parts[2]).  With masks
         [V, 1, H, W] (the test views' covisibility masks, any dtype masked_image_metrics takes) the table is [V, 7]: columns
         0-3 as without masks, columns 4-6 = (mmse, mpsnr, mssim) of rodygs_b200.metrics.masked_image_metrics over the mask,
         DyCheck's iPhone protocol.  lpips: None, or one rodygs_b200.metrics.LpipsWeights or a sequence of them (the
         reference reports alex and vgg); each adds one column after the others, in the given order, holding
-        rodygs_b200.metrics.lpips of the same clamped render: [V, 4 + L], or [V, 7 + L] with masks.
+        rodygs_b200.metrics.lpips of the same clamped render: [V, 4 + L], or [V, 7 + L] with masks.  masked_lpips (needs
+        masks): None, or one LpipsWeights or a sequence of them (DyCheck reports alex); each adds one column after the lpips
+        columns, in the given order, holding rodygs_b200.metrics.masked_lpips of the same clamped render under masks[v]
+        (mLPIPS): [V, 7 + L + M].
 
         viewmats / projmats [V, 4, 4] in glm storage; tanfovx / tanfovy a float or a length-V sequence; basis_ts [V, K, 7]
         the B(t) of each view (from BasisMLP.query_and_table or the table: no MLP runs here; None without dynamic
@@ -1011,14 +1015,20 @@ class SplatTrainStep:
             return vals
 
         fovx, fovy = per_view("tanfovx", tanfovx), per_view("tanfovy", tanfovy)
-        from .metrics import LpipsWeights, image_metrics, lpips as lpips_metric, masked_image_metrics
+        from .metrics import LpipsWeights, image_metrics, lpips as lpips_metric, masked_image_metrics, masked_lpips as mlpips
         nets = [] if lpips is None else [lpips] if isinstance(lpips, LpipsWeights) else list(lpips)
         if not all(isinstance(w, LpipsWeights) for w in nets):
             raise ValueError("SplatTrainStep.evaluate: lpips must be an LpipsWeights (rodygs_b200.metrics.load_lpips) or a "
                              "sequence of them")
+        mnets = [] if masked_lpips is None else [masked_lpips] if isinstance(masked_lpips, LpipsWeights) else list(masked_lpips)
+        if not all(isinstance(w, LpipsWeights) for w in mnets):
+            raise ValueError("SplatTrainStep.evaluate: masked_lpips must be an LpipsWeights (rodygs_b200.metrics.load_lpips) "
+                             "or a sequence of them")
+        if mnets and masks is None:
+            raise ValueError("SplatTrainStep.evaluate: masked_lpips scores under the covisibility masks; pass masks as well")
         rank, world = self._dp_rank_world()
         cols = 4 if masks is None else 7
-        table = torch.zeros(V, cols + len(nets), dtype=torch.float32, device=self.dev)
+        table = torch.zeros(V, cols + len(nets) + len(mnets), dtype=torch.float32, device=self.dev)
         cap = engine._cap_state(self.params.device, self.ns + self.nd)
         saved = engine.config.sync_free, cap["pending"]          # a training step's unread duplicate count stays for it
         engine.config.sync_free, cap["pending"] = False, None
@@ -1031,6 +1041,8 @@ class SplatTrainStep:
                     table[v, 4:7] = masked_image_metrics(color, gts[v], masks[v], value_range)[0]
                 for j, w in enumerate(nets):
                     table[v, cols + j] = lpips_metric(color, gts[v], w, value_range)[0]
+                for j, w in enumerate(mnets):
+                    table[v, cols + len(nets) + j] = mlpips(color, gts[v], masks[v], w, value_range)[0]
         finally:
             engine.config.sync_free, cap["pending"] = saved
         allreduce_flat(table, None, self.pg)

@@ -1,12 +1,14 @@
 """Time rdg_lpips (AlexNet and VGG-16 LPIPS, convolutions on tcgen05 tensor cores in TF32) per image pair, its conv
 kernel per layer, and a float32 F.conv2d restatement of the same definition with cuDNN's TF32 allowed (the reference's
-arithmetic) and disallowed; print one JSON line per backbone with the GPU's name, power limit and SM clock.
+arithmetic) and disallowed; in the same run, rdg_masked_lpips (mLPIPS) of the same pair under a seeded covisibility mask,
+alternating with rdg_lpips call by call.  Prints one JSON line per backbone with the GPU's name, power limit and SM clock.
 
     python tools/lpips_bench.py [--height 1080] [--width 1920] [--iters 100] [--warmup 20] [--out FILE]
 
 Weights are seeded random ones under the real key names (nothing is downloaded; the time does not depend on the values).
 One seeded render-like pair at 1920x1080.  Per-pair times: CUDA events around each of `iters` calls after `warmup` calls,
-reported as median / p10 / p90.  Per-layer conv times: device time of each lpips_conv_kernel launch from a torch.profiler
+reported as median / p10 / p90; rdg_lpips and rdg_masked_lpips are timed alternately in one loop, so both see the same
+clocks.  The masked path's own kernels (the spatial pass and its finalize) are also timed from a torch.profiler run.  Per-layer conv times: device time of each lpips_conv_kernel launch from a torch.profiler
 run of its own, median over 20 pairs.  Achieved TFLOP/s = 2 MAC / time, set against the data-sheet dense TF32 rate of
 one HGX B200 GPU (1,125 TFLOP/s; a data-sheet figure, not one measured here).  The VGG pair's activations (1.06 GB for
 relu1_2 of the pair) exceed the 126 MB L2."""
@@ -22,7 +24,7 @@ import torch.nn.functional as F
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 
-from rodygs_b200.metrics import LPIPS_CONVS, LPIPS_TAPS, load_lpips, lpips  # noqa: E402
+from rodygs_b200.metrics import LPIPS_CONVS, LPIPS_TAPS, load_lpips, lpips, masked_lpips  # noqa: E402
 
 TF32_DATASHEET_TFLOPS = 1125.0
 POOLS = {"alex": {3: 3, 6: 3}, "vgg": {5: 2, 10: 2, 17: 2, 24: 2}}   # features.{i} -> kernel of the stride-2 pool before it
@@ -83,19 +85,39 @@ def gpu_identity():
     return {"gpu": name, "power_limit": power, "sm_clock_at_query": sm, "sm_clock_max": sm_max}
 
 
-def event_times(fn, iters, warmup):
-    for _ in range(warmup):
-        fn()
-    torch.cuda.synchronize()
-    ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(iters)]
-    for a, b in ev:
-        a.record()
-        fn()
-        b.record()
-    torch.cuda.synchronize()
-    ts = sorted(a.elapsed_time(b) for a, b in ev)
+def _summary(ts):
+    ts = sorted(ts)
     q = lambda f: ts[min(len(ts) - 1, int(f * len(ts)))]   # noqa: E731
     return {"median": round(statistics.median(ts), 4), "p10": round(q(0.1), 4), "p90": round(q(0.9), 4)}
+
+
+def event_times(fn, iters, warmup):
+    return alternating_event_times([fn], iters, warmup)[0]
+
+
+def alternating_event_times(fns, iters, warmup):
+    """CUDA-event times of each of fns, called in turn `iters` times after `warmup` rounds."""
+    for _ in range(warmup):
+        for fn in fns:
+            fn()
+    torch.cuda.synchronize()
+    ev = [[(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in fns] for _ in range(iters)]
+    for row in ev:
+        for fn, (a, b) in zip(fns, row):
+            a.record()
+            fn()
+            b.record()
+    torch.cuda.synchronize()
+    return [_summary([row[k][0].elapsed_time(row[k][1]) for row in ev]) for k in range(len(fns))]
+
+
+def covisibility_mask(H, W, g):
+    """[1, 1, H, W]: blobs with ragged edges and single-pixel holes, about half the image covisible."""
+    low = torch.rand(1, 1, H // 40 + 2, W // 40 + 2, device="cuda", generator=g)
+    smooth = F.interpolate(low, size=(H, W), mode="bilinear", align_corners=False)
+    ragged = smooth + 0.1 * torch.rand(1, 1, H, W, device="cuda", generator=g)
+    holes = torch.rand(1, 1, H, W, device="cuda", generator=g) < 0.01
+    return ((ragged > 0.55) & ~holes).float()
 
 
 def conv_layer_ms(fn, nconv, pairs=20):
@@ -113,6 +135,23 @@ def conv_layer_ms(fn, nconv, pairs=20):
     return [statistics.median(ev[p * nconv + l].time_range.elapsed_us() for p in range(pairs)) / 1e3 for l in range(nconv)]
 
 
+def kernels_ms(fn, names, pairs=20):
+    """Median device time per pair of the launches whose kernel name holds one of `names`, from a profiler run."""
+    from torch.profiler import ProfilerActivity, profile
+    fn()
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(pairs):
+            fn()
+        torch.cuda.synchronize()
+    out = {}
+    for name in names:
+        ev = sorted((e for e in prof.events() if name in e.name), key=lambda e: e.time_range.start)
+        assert len(ev) == pairs, (name, len(ev), pairs)
+        out[name] = round(statistics.median(e.time_range.elapsed_us() for e in ev) / 1e3, 4)
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--height", type=int, default=1080)
@@ -128,6 +167,7 @@ def main():
     low = torch.rand(1, 3, H // 60 + 2, W // 60 + 2, device="cuda", generator=g)
     pred = F.interpolate(low, size=(H, W), mode="bilinear", align_corners=False)
     gt = (pred + 0.05 * torch.randn(pred.shape, device="cuda", generator=g)).clamp(0, 1)
+    mask = covisibility_mask(H, W, torch.Generator(device="cuda").manual_seed(1))
     ident = gpu_identity()
     lines = []
     saved = torch.backends.cudnn.allow_tf32
@@ -137,8 +177,11 @@ def main():
         dev_w = {key: v.cuda() for key, v in {**bb, **lin}.items()}
         shapes = layer_shapes(net, H, W)
         macs = [2 * ho * wo * cout * cin * kk * kk for (_, cout, cin, kk, _, _, _, _, ho, wo) in shapes]
-        kern = event_times(lambda: lpips(pred, gt, w), args.iters, args.warmup)
+        kern, mkern = alternating_event_times([lambda: lpips(pred, gt, w), lambda: masked_lpips(pred, gt, mask, w)],
+                                              args.iters, args.warmup)
         per_layer = conv_layer_ms(lambda: lpips(pred, gt, w), len(shapes))
+        masked_own = kernels_ms(lambda: masked_lpips(pred, gt, mask, w),
+                                ("lpips_spatial_kernel", "lpips_masked_finalize_kernel"))
         res = {}
         for tf32 in (True, False):
             torch.backends.cudnn.allow_tf32 = tf32
@@ -157,6 +200,7 @@ def main():
             res[f"value_{tf32}"] = ref.item()
         torch.backends.cudnn.allow_tf32 = saved
         got = lpips(pred, gt, w).item()
+        got_masked = masked_lpips(pred, gt, mask, w).item()
         layers = []
         for (i, cout, cin, kk, s, p, h, ww, ho, wo), mac, ms, ctf, cfp in zip(shapes, macs, per_layer, res["layers_True"],
                                                                                res["layers_False"]):
@@ -171,7 +215,10 @@ def main():
                 "kernel_ms_per_pair": kern, "cudnn_tf32_ms_per_pair": res[True], "cudnn_fp32_ms_per_pair": res[False],
                 "kernel_tflops_whole_pair": round(2 * total_mac / (kern["median"] * 1e-3) / 1e12, 1),
                 "datasheet_dense_tf32_tflops": TF32_DATASHEET_TFLOPS, "layers": layers,
-                "value_kernel": got, "value_cudnn_tf32": res["value_True"], "value_cudnn_fp32": res["value_False"]}
+                "value_kernel": got, "value_cudnn_tf32": res["value_True"], "value_cudnn_fp32": res["value_False"],
+                "mask_covisible": round(mask.mean().item(), 4), "masked_kernel_ms_per_pair": mkern,
+                "masked_minus_plain_ms_median": round(mkern["median"] - kern["median"], 4),
+                "masked_own_kernels_ms": masked_own, "value_masked_kernel": got_masked}
         lines.append(json.dumps(line))
         print(lines[-1], flush=True)
     if args.out:
