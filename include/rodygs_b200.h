@@ -405,6 +405,27 @@ typedef struct RdgPoseAdam {
  * One warp, one launch, no host synchronisation. */
 int rdg_pose_adam(const RdgPoseAdam* args, int32_t update, void* stream);
 
+/* ---- learning the training cameras (INTEGRATION.md "Learning the training cameras") ------------------------------------ */
+
+/* A table of C cameras: param [C, 7] rows (q_r, q_x, q_y, q_z, T_x, T_y, T_z) as in RdgPoseAdam, V(q, T) the same formula.
+ * rdg_camera_grad: grad [C, 7] = for each camera c, the sum in slot order over the slots s with cam_idx[s] == c of
+ * dL_dV_slots[s] (16 floats, glm storage, as rdg_preprocess_bwd wrote it) pulled back through V(q_c, T_c) - the arithmetic of
+ * rdg_pose_adam's grad output; rows no slot names are 0.  No float atomics: bit-identical from run to run.  *error receives 1 +
+ * the first slot whose index lies outside [0, C), or 0; such a slot is skipped (nothing is written out of bounds).
+ * n_slots = 0 only zeroes grad.  One launch. */
+int rdg_camera_grad(int32_t n_slots, const int32_t* cam_idx, const float* dL_dV_slots, const float* param, int32_t C,
+                    float* grad, int32_t* error, void* stream);
+
+/* One dense torch.optim.Adam step over every row (no weight decay; bias correction from step >= 1, the step count the whole
+ * table shares): the gradient is grad * grad_scale, q moves with lr_q and T with lr_T (doubles, like torch's Python
+ * hyperparameters).  Then V(q, T) of every camera in glm storage into viewmats [C, 16], what the next rdg_preprocess_fwd
+ * reads.  One launch. */
+int rdg_camera_adam(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int32_t C, int32_t step, double lr_q,
+                    double lr_T, double beta1, double beta2, double eps, float grad_scale, float* viewmats, void* stream);
+
+/* viewmats [C, 16] = V(q, T) of every row of param [C, 7], glm storage, nothing else (the table before its first step). */
+int rdg_camera_views(const float* param, int32_t C, float* viewmats, void* stream);
+
 /* loss = mean((pred - gt)^2) over channels x height x width; dL_dpred = 2 (pred - gt) / n (overwritten); the loss goes to
  * history[*step] (device step counter, the slot of the pose the image was rendered at) when 0 <= *step < max_steps.  Per-CTA
  * float64 partials in fixed workspace slots and a fixed-order finalize, no float atomics: bit-identical from run to run.

@@ -155,6 +155,10 @@ SYMBOLS = {
     "rdg_masked_lpips": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_int32, c_ptr,
                                    C.c_int64, c_ptr, c_ptr, C.c_int64, c_ptr]),
     "rdg_pose_adam": (C.c_int, [C.POINTER(RdgPoseAdam), C.c_int32, c_ptr]),
+    "rdg_camera_grad": (C.c_int, [C.c_int32, c_ptr, c_ptr, c_ptr, C.c_int32, c_ptr, c_ptr, c_ptr]),
+    "rdg_camera_adam": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, C.c_int32, C.c_int32, C.c_double, C.c_double, C.c_double,
+                                  C.c_double, C.c_double, C.c_float, c_ptr, c_ptr]),
+    "rdg_camera_views": (C.c_int, [c_ptr, C.c_int32, c_ptr, c_ptr]),
     "rdg_l2_loss_workspace_bytes": (C.c_int64, [C.c_int32, C.c_int32, C.c_int32]),
     "rdg_l2_loss": (C.c_int, [c_ptr, c_ptr, C.c_int32, C.c_int32, C.c_int32, c_ptr, C.c_int32, c_ptr, c_ptr, c_ptr, C.c_int64,
                               c_ptr]),

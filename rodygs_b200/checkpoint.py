@@ -14,6 +14,9 @@ not in this tree, so it is recalled, not pinned: map the dicts into and out of a
 The step holds three things no reference model does: the motion table B(t_i) [T,K,7] (the MLP's output at the training
 times, or a free tensor when no MLP is attached), B(t) [K,7] of the last query time and `spatial_lr_scale`.  They travel
 under the separate key "motion" so that the round trip is lossless.
+
+With camera learning enabled (`SplatTrainStep.enable_camera_learning`), the learned training cameras travel under "cameras" with
+the reference's `LearnableCamera` attribute names: `R_c2ws_quat [C, 4]` and `T_c2ws [C, 3]`, both camera to world.
 """
 from __future__ import annotations
 
@@ -27,7 +30,8 @@ TAGS = ("static", "dynamic")
 
 
 def export_models(step) -> Dict[str, Dict]:
-    """{"static": {...}, "dynamic": {...}, "motion": {"table", "basis_t", "spatial_lr_scale"}}; tensors are copies on the
+    """{"static": {...}, "dynamic": {...}, "motion": {"table", "basis_t", "spatial_lr_scale"}} (+ "cameras": {"R_c2ws_quat",
+    "T_c2ws"} when the step learns its cameras); tensors are copies on the
     step's device (they outlive the next densification, which replaces the flat buffers)."""
     out = {tag: {f"_{k}": step.p(f"{tag}.{k}").detach().clone() for k in PARAM_ORDER} for tag in TAGS}
     dyn = out["dynamic"]
@@ -40,6 +44,9 @@ def export_models(step) -> Dict[str, Dict]:
         dyn["_deform_network"] = mlp.state_dict()
     out["motion"] = {"table": step.p("table").detach().clone(), "basis_t": step.p("basis_t").detach().clone(),
                      "spatial_lr_scale": float(step.spatial_lr_scale)}
+    cam = getattr(step, "cameras", None)
+    if cam is not None:
+        out["cameras"] = {"R_c2ws_quat": cam["param"][:, :4].clone(), "T_c2ws": cam["param"][:, 4:].clone()}
     return out
 
 
@@ -49,7 +56,8 @@ def import_models(d: Dict[str, Dict], table: Optional[torch.Tensor] = None, basi
     reference trained).  table / basis_t / spatial_lr_scale override d["motion"]; without d["motion"] the table is
     required (compute it with `BasisMLP.query_and_table(t, train_times)` after loading `_deform_network`) and
     spatial_lr_scale defaults to 1.  `_deform_network` itself goes to `BasisMLP.load_state_dict` +
-    `SplatTrainStep.attach_basis_mlp`."""
+    `SplatTrainStep.attach_basis_mlp`.  d["cameras"] ({"R_c2ws_quat": [C, 4], "T_c2ws": [C, 3]}), when present, is checked
+    and passed on as scene["cameras"], which `SplatTrainStep.enable_camera_learning(scene["cameras"], lrs)` takes."""
     motion = d.get("motion", {})
     table = motion.get("table") if table is None else table
     if table is None:
@@ -85,4 +93,11 @@ def import_models(d: Dict[str, Dict], table: Optional[torch.Tensor] = None, basi
                  spatial_lr_scale=float(spatial_lr_scale))
     if basis_t is not None:
         scene["basis_t"] = basis_t.detach().to(torch.float32)
+    if "cameras" in d:
+        q, T = d["cameras"].get("R_c2ws_quat"), d["cameras"].get("T_c2ws")
+        C = q.shape[0] if torch.is_tensor(q) and q.dim() == 2 else 0
+        if C < 1 or tuple(q.shape) != (C, 4) or not torch.is_tensor(T) or tuple(T.shape) != (C, 3):
+            got = [tuple(t.shape) if torch.is_tensor(t) else type(t).__name__ for t in (q, T)]
+            raise ValueError(f"import_models: cameras needs R_c2ws_quat [C,4] and T_c2ws [C,3] with C >= 1, got {got}")
+        scene["cameras"] = {"R_c2ws_quat": q.detach().to(torch.float32), "T_c2ws": T.detach().to(torch.float32)}
     return scene

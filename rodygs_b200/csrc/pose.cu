@@ -3,41 +3,13 @@
 // model, L2 photometric loss, backward, Adam step on one LearnableCamera) device-resident, so that the whole loop is
 // replays of one CUDA graph with no host read.  Definitions: INTEGRATION.md "Refining held-out camera poses".
 //
-// Pose parameters (q, T): q = (r, x, y, z) the camera-to-world rotation (any norm; it is normalised here), T the
-// camera-to-world translation.  R = rot(q / |q|),  V = [[R^T, -R^T T], [0, 0, 0, 1]].  In glm storage (the 16 floats of
-// V^T row-major) the rotation block reads R row-major: V_glm[4 k + r] = V[r][k] = R[k][r] for r, k < 3.
+// The pose arithmetic (V(q, T), dL/dV -> dL/d(q, T), the Adam element) is in pose.cuh, shared with the camera table below.
 #include <math.h>
 #include "common.cuh"
+#include "pose.cuh"
 
 #define PL_THREADS 256
 #define PL_MAX_CTAS 592            // 4 per SM: enough to stream the image at full bandwidth
-
-// R (row-major) of the normalised quaternion; qn receives q / |q|, the return value is 1 / |q|.
-__device__ __forceinline__ float pose_rot(const float* q, float* qn, float* R) {
-    const float inv = 1.0f / sqrtf(q[0] * q[0] + q[1] * q[1] + q[2] * q[2] + q[3] * q[3]);
-    const float r = q[0] * inv, x = q[1] * inv, y = q[2] * inv, z = q[3] * inv;
-    qn[0] = r; qn[1] = x; qn[2] = y; qn[3] = z;
-    R[0] = 1.f - 2.f * (y * y + z * z); R[1] = 2.f * (x * y - r * z);       R[2] = 2.f * (x * z + r * y);
-    R[3] = 2.f * (x * y + r * z);       R[4] = 1.f - 2.f * (x * x + z * z); R[5] = 2.f * (y * z - r * x);
-    R[6] = 2.f * (x * z - r * y);       R[7] = 2.f * (y * z + r * x);       R[8] = 1.f - 2.f * (x * x + y * y);
-    return inv;
-}
-
-// V(q, T) in glm storage (16 floats)
-__device__ void pose_write_view(const float* prm, float* __restrict__ vm) {
-    float qn[4], R[9];
-    pose_rot(prm, qn, R);
-    const float* T = prm + 4;
-#pragma unroll
-    for (int k = 0; k < 3; ++k) {
-#pragma unroll
-        for (int r = 0; r < 3; ++r) vm[4 * k + r] = R[3 * k + r];
-        vm[4 * k + 3] = 0.f;
-    }
-#pragma unroll
-    for (int r = 0; r < 3; ++r) vm[12 + r] = -(R[r] * T[0] + R[3 + r] * T[1] + R[6 + r] * T[2]);
-    vm[15] = 1.f;
-}
 
 // One warp.  Lanes 0..15 own one float of dL/dV (read, then zeroed for the next iteration's rdg_preprocess_bwd), lanes 0..6
 // one Adam parameter; lane 0 chains dL/dV to dL/d(q, T) in between.
@@ -63,42 +35,14 @@ __global__ void __launch_bounds__(32) pose_adam_kernel(RdgPoseAdam a, int update
             a.overflow[1] = a.num_rendered[0];
         }
         apply = !overflow && step < a.max_steps;
-        float qn[4], R[9];
-        const float inv = pose_rot(a.param, qn, R);
-        const float* T = a.param + 4;
-        // V[r][k] = R[k][r], V[r][3] = -sum_k R[k][r] T[k]; dL/dV[r][k] = gv[4 k + r]
-        float dR[9];
-#pragma unroll
-        for (int k = 0; k < 3; ++k)
-#pragma unroll
-            for (int r = 0; r < 3; ++r) dR[3 * k + r] = gv[4 * k + r] - T[k] * gv[12 + r];
-#pragma unroll
-        for (int k = 0; k < 3; ++k) g7[4 + k] = -(R[3 * k] * gv[12] + R[3 * k + 1] * gv[13] + R[3 * k + 2] * gv[14]);
-        const float r = qn[0], x = qn[1], y = qn[2], z = qn[3];
-        float dq[4];
-        dq[0] = 2.f * (-z * dR[1] + y * dR[2] + z * dR[3] - x * dR[5] - y * dR[6] + x * dR[7]);
-        dq[1] = 2.f * (y * dR[1] + z * dR[2] + y * dR[3] - 2.f * x * dR[4] - r * dR[5] + z * dR[6] + r * dR[7] - 2.f * x * dR[8]);
-        dq[2] = 2.f * (-2.f * y * dR[0] + x * dR[1] + r * dR[2] + x * dR[3] + z * dR[5] - r * dR[6] + z * dR[7] - 2.f * y * dR[8]);
-        dq[3] = 2.f * (-2.f * z * dR[0] - r * dR[1] + x * dR[2] + r * dR[3] - 2.f * z * dR[4] + y * dR[5] + x * dR[6] + y * dR[7]);
-        // through q / |q|: (I - qn qn^T) / |q|
-        const float dot = r * dq[0] + x * dq[1] + y * dq[2] + z * dq[3];
-#pragma unroll
-        for (int k = 0; k < 4; ++k) g7[k] = (dq[k] - qn[k] * dot) * inv;
+        pose_pullback(a.param, gv, g7);
     }
     __syncwarp();
     if (lane < 7 && a.grad) a.grad[lane] = g7[lane];
     if (apply && lane < 7) {
-        // torch.optim.Adam (no weight decay, no amsgrad): scalars in double as torch takes them on the host, each rounded to
-        // float where the float32 tensor op consumes it
-        const int t = *a.step + 1;
-        const double bc1 = 1.0 - pow(a.beta1, (double)t);
-        const double bc2_sqrt = sqrt(1.0 - pow(a.beta2, (double)t));
-        const float g = g7[lane];
-        float m = a.exp_avg[lane], v = a.exp_avg_sq[lane];
-        m = m + (float)(1.0 - a.beta1) * (g - m);                     // exp_avg.lerp_(grad, 1 - beta1)
-        v = v * (float)a.beta2 + (float)(1.0 - a.beta2) * g * g;      // exp_avg_sq.mul_(beta2).addcmul_(grad, grad, 1 - beta2)
-        const float denom = sqrtf(v) / (float)bc2_sqrt + (float)a.eps;
-        a.param[lane] = a.param[lane] + (float)(-(a.lr / bc1)) * (m / denom);
+        float p = a.param[lane], m = a.exp_avg[lane], v = a.exp_avg_sq[lane];
+        pose_adam_elem(p, g7[lane], m, v, *a.step + 1, a.lr, a.beta1, a.beta2, a.eps);
+        a.param[lane] = p;
         a.exp_avg[lane] = m;
         a.exp_avg_sq[lane] = v;
     }
@@ -127,6 +71,120 @@ extern "C" int rdg_pose_adam(const RdgPoseAdam* args, int32_t update, void* stre
         RDG_CHECK_ARG(!args->num_rendered || args->overflow, "overflow is NULL (required with num_rendered)");
     }
     pose_adam_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(*args, update);
+    RDG_CHECK_LAUNCH();
+    rdg_count_launches(1);
+    return RDG_OK;
+}
+
+// ---- the table of training cameras (INTEGRATION.md "Learning the training cameras") --------------------------------------
+// C is at most a few thousand rows of 7 floats: each launch below is one thread per camera and takes microseconds, so
+// none of them is tuned.
+
+#define CAM_THREADS 128
+
+// One thread per camera: its row of dL/d(q, T) is the slot-order sum of the pulled-back dL/dV of every slot naming it (no
+// atomics, so the result is bit-identical from run to run; a row no slot names is 0).  Thread 0 also scans the indices and
+// writes 1 + the first slot whose camera lies outside [0, C) into *error, or 0; such a slot adds to no row.
+__global__ void __launch_bounds__(CAM_THREADS) camera_grad_kernel(int n_slots, const int32_t* __restrict__ cam_idx,
+                                                                  const float* __restrict__ dV, const float* __restrict__ param,
+                                                                  int C, float* __restrict__ grad, int32_t* __restrict__ error) {
+    const int c = blockIdx.x * CAM_THREADS + threadIdx.x;
+    if (c == 0) {
+        int bad = 0;
+        for (int s = 0; s < n_slots && !bad; ++s)
+            if (cam_idx[s] < 0 || cam_idx[s] >= C) bad = s + 1;
+        *error = bad;
+    }
+    if (c >= C) return;
+    float prm[7], acc[7];
+#pragma unroll
+    for (int k = 0; k < 7; ++k) prm[k] = param[7 * c + k];
+    bool have = false;
+    for (int s = 0; s < n_slots; ++s) {
+        if (cam_idx[s] != c) continue;
+        float gv[16], g7[7];
+#pragma unroll
+        for (int k = 0; k < 16; ++k) gv[k] = dV[16 * s + k];
+        pose_pullback(prm, gv, g7);
+        // the first term is taken as it is (0 + x would turn a -0 into +0): one slot gives rdg_pose_adam's bits
+#pragma unroll
+        for (int k = 0; k < 7; ++k) acc[k] = have ? acc[k] + g7[k] : g7[k];
+        have = true;
+    }
+#pragma unroll
+    for (int k = 0; k < 7; ++k) grad[7 * c + k] = have ? acc[k] : 0.f;
+}
+
+// One thread per camera: one Adam step of all 7 parameters (q with lr_q, T with lr_T), then V(q, T) of the new pose
+__global__ void __launch_bounds__(CAM_THREADS) camera_adam_kernel(float* __restrict__ param, const float* __restrict__ grad,
+                                                                  float* __restrict__ exp_avg, float* __restrict__ exp_avg_sq, int C,
+                                                                  int step, double lr_q, double lr_T, double beta1, double beta2,
+                                                                  double eps, float grad_scale, float* __restrict__ viewmats) {
+    const int c = blockIdx.x * CAM_THREADS + threadIdx.x;
+    if (c >= C) return;
+    float prm[7];
+#pragma unroll
+    for (int k = 0; k < 7; ++k) {
+        const int i = 7 * c + k;
+        float p = param[i], m = exp_avg[i], v = exp_avg_sq[i];
+        pose_adam_elem(p, grad[i] * grad_scale, m, v, step, k < 4 ? lr_q : lr_T, beta1, beta2, eps);
+        param[i] = prm[k] = p;
+        exp_avg[i] = m;
+        exp_avg_sq[i] = v;
+    }
+    pose_write_view(prm, viewmats + 16 * c);
+}
+
+__global__ void __launch_bounds__(CAM_THREADS) camera_views_kernel(const float* __restrict__ param, int C,
+                                                                   float* __restrict__ viewmats) {
+    const int c = blockIdx.x * CAM_THREADS + threadIdx.x;
+    if (c < C) pose_write_view(param + 7 * c, viewmats + 16 * c);
+}
+
+extern "C" int rdg_camera_grad(int32_t n_slots, const int32_t* cam_idx, const float* dL_dV_slots, const float* param, int32_t C,
+                               float* grad, int32_t* error, void* stream) {
+    RDG_CHECK_ARG(cam_idx, "cam_idx is NULL");
+    RDG_CHECK_ARG(dL_dV_slots, "dL_dV_slots is NULL");
+    RDG_CHECK_ARG(param, "param is NULL");
+    RDG_CHECK_ARG(grad, "grad is NULL");
+    RDG_CHECK_ARG(error, "error is NULL");
+    RDG_CHECK_ARG(n_slots >= 0, "n_slots must be >= 0");
+    RDG_CHECK_ARG(C >= 1, "C must be >= 1");
+    camera_grad_kernel<<<rdg_div_up(C, CAM_THREADS), CAM_THREADS, 0, (cudaStream_t)stream>>>(n_slots, cam_idx, dL_dV_slots,
+                                                                                            param, C, grad, error);
+    RDG_CHECK_LAUNCH();
+    rdg_count_launches(1);
+    return RDG_OK;
+}
+
+extern "C" int rdg_camera_adam(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int32_t C, int32_t step,
+                               double lr_q, double lr_T, double beta1, double beta2, double eps, float grad_scale, float* viewmats,
+                               void* stream) {
+    RDG_CHECK_ARG(param, "param is NULL");
+    RDG_CHECK_ARG(grad, "grad is NULL");
+    RDG_CHECK_ARG(exp_avg, "exp_avg is NULL");
+    RDG_CHECK_ARG(exp_avg_sq, "exp_avg_sq is NULL");
+    RDG_CHECK_ARG(viewmats, "viewmats is NULL");
+    RDG_CHECK_ARG(C >= 1, "C must be >= 1");
+    RDG_CHECK_ARG(step >= 1, "step must be >= 1");
+    RDG_CHECK_ARG(lr_q >= 0.0 && isfinite(lr_q), "lr_q must be a finite value >= 0");
+    RDG_CHECK_ARG(lr_T >= 0.0 && isfinite(lr_T), "lr_T must be a finite value >= 0");
+    RDG_CHECK_ARG(beta1 >= 0.0 && beta1 < 1.0, "beta1 must be in [0, 1)");
+    RDG_CHECK_ARG(beta2 >= 0.0 && beta2 < 1.0, "beta2 must be in [0, 1)");
+    RDG_CHECK_ARG(eps >= 0.0 && isfinite(eps), "eps must be a finite value >= 0");
+    RDG_CHECK_ARG(isfinite(grad_scale), "grad_scale must be finite");
+    camera_adam_kernel<<<rdg_div_up(C, CAM_THREADS), CAM_THREADS, 0, (cudaStream_t)stream>>>(
+        param, grad, exp_avg, exp_avg_sq, C, step, lr_q, lr_T, beta1, beta2, eps, grad_scale, viewmats);
+    RDG_CHECK_LAUNCH();
+    rdg_count_launches(1);
+    return RDG_OK;
+}
+
+extern "C" int rdg_camera_views(const float* param, int32_t C, float* viewmats, void* stream) {
+    RDG_CHECK_ARG(param, "param is NULL");
+    RDG_CHECK_ARG(viewmats, "viewmats is NULL");
+    RDG_CHECK_ARG(C >= 1, "C must be >= 1");
+    camera_views_kernel<<<rdg_div_up(C, CAM_THREADS), CAM_THREADS, 0, (cudaStream_t)stream>>>(param, C, viewmats);
     RDG_CHECK_LAUNCH();
     rdg_count_launches(1);
     return RDG_OK;

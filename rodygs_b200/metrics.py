@@ -1,6 +1,6 @@
 """Evaluation image metrics on the device: MSE, PSNR, SSIM and MS-SSIM in one fused pass per scale (rdg_image_metrics),
 their masked forms over a covisibility mask, mPSNR and mSSIM (rdg_masked_image_metrics), LPIPS (rdg_lpips) and its masked
-form, mLPIPS (rdg_masked_lpips).
+form, mLPIPS (rdg_masked_lpips); and the trajectory errors ATE / RPE of learned cameras (trajectory_errors, float64 torch).
 
 These are the metrics the reference reports for held-out views (RoDyGSEvaluator.eval, VizScoreEvaluator, through piqa):
 an 11x11 Gaussian window (sigma 1.5) over the VALID region only, averaged per channel, and MS-SSIM over five scales.  They
@@ -263,3 +263,44 @@ def masked_lpips(pred: torch.Tensor, gt: torch.Tensor, mask: torch.Tensor, weigh
         check(lib.rdg_masked_lpips(ptr(x), ptr(y), ptr(m), B, Cc, H, W, value_range, code, ptr(weights.packed),
                                    weights.packed.numel(), ptr(out), ptr(ws), nbytes, _lib.stream_ptr()))
     return out
+
+
+def trajectory_errors(pred_c2w: torch.Tensor, gt_c2w: torch.Tensor):
+    """(ate, rpe_trans, rpe_rot_deg) of a learned camera trajectory, three float64 scalars on the inputs' device (no host
+    read).  pred_c2w / gt_c2w: [C, 4, 4] camera-to-world matrices (mathematical row-major layout, C >= 2), in the same order.
+
+    The predicted camera centres are aligned to the ground-truth ones by the Umeyama Sim(3) (rotation, translation and
+    scale); ATE is the RMSE of the aligned centres.  The aligned predicted poses (R pred_R, s R pred_t + t) then give RPE over
+    consecutive pairs: rel = inv(inv(gt_i) gt_{i+1}) (inv(pred_i) pred_{i+1}), rpe_trans the mean of |rel[:3, 3]|, rpe_rot_deg
+    the mean of arccos(clamp((tr rel[:3, :3] - 1) / 2, -1, 1)) in degrees.  These are the compute_ATE / compute_rpe
+    conventions of Nope-NeRF / CF-3DGS as recalled, not pinned (INTEGRATION.md "Learning the training cameras").  Computed
+    in float64 with torch: C is at most a few thousand 4x4 matrices."""
+    if not (torch.is_tensor(pred_c2w) and torch.is_tensor(gt_c2w) and pred_c2w.dim() == 3 and pred_c2w.shape[0] >= 2
+            and tuple(pred_c2w.shape[1:]) == (4, 4) and pred_c2w.shape == gt_c2w.shape and pred_c2w.device == gt_c2w.device):
+        got = [tuple(t.shape) if torch.is_tensor(t) else type(t).__name__ for t in (pred_c2w, gt_c2w)]
+        raise ValueError(f"trajectory_errors: pred_c2w and gt_c2w must be [C, 4, 4] tensors on one device with C >= 2, got {got}")
+    pred, gt = pred_c2w.double(), gt_c2w.double()
+    n = pred.shape[0]
+    # Umeyama: gt_centre ~ s R pred_centre + t
+    x, y = pred[:, :3, 3], gt[:, :3, 3]
+    mx, my = x.mean(0), y.mean(0)
+    xc, yc = x - mx, y - my
+    U, D, Vh = torch.linalg.svd(yc.t() @ xc / n)
+    S = torch.ones(3, dtype=torch.float64, device=pred.device)
+    S[2] = torch.where(torch.linalg.det(U) * torch.linalg.det(Vh) < 0, -1.0, 1.0)
+    R = U @ torch.diag(S) @ Vh
+    s = (D * S).sum() / ((xc * xc).sum() / n)
+    t = my - s * (R @ mx)
+    aligned = pred.clone()
+    aligned[:, :3, :3] = R @ pred[:, :3, :3]
+    aligned[:, :3, 3] = s * x @ R.t() + t
+    ate = ((aligned[:, :3, 3] - y) ** 2).sum(-1).mean().sqrt()
+    inv_gt, inv_pred = torch.linalg.inv(gt), torch.linalg.inv(aligned)
+    rel = torch.linalg.inv(inv_gt[:-1] @ gt[1:]) @ (inv_pred[:-1] @ aligned[1:])
+    rpe_trans = rel[:, :3, 3].norm(dim=-1).mean()
+    # the arccos of the definition as atan2(sin, cos): the same angle for a rotation, but without arccos' loss of precision
+    # near 0 (arccos(1 - 1e-16) is already 1.4e-8)
+    cos = ((rel[:, 0, 0] + rel[:, 1, 1] + rel[:, 2, 2] - 1.0) / 2.0).clamp(-1.0, 1.0)
+    sin = torch.stack([rel[:, 2, 1] - rel[:, 1, 2], rel[:, 0, 2] - rel[:, 2, 0], rel[:, 1, 0] - rel[:, 0, 1]], -1).norm(dim=-1) / 2.0
+    rpe_rot = torch.rad2deg(torch.atan2(sin, cos)).mean()
+    return ate, rpe_trans, rpe_rot

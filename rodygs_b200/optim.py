@@ -61,6 +61,44 @@ class GaussianLRs:
         return lrs
 
 
+@dataclass
+class CameraLRs:
+    """Learning rates of the training-camera table (SplatTrainStep.enable_camera_learning): lr_q for the quaternions, lr_T for
+    the translations, both scaled by the warmup + cosine factor
+
+        f(it) = min(1, it / warmup_steps) * (final_ratio + (1 - final_ratio) * 0.5 * (1 + cos(pi * p))),
+        p = clamp((it - warmup_steps) / (max_steps - warmup_steps), 0, 1)
+
+    (f = 1 for the warmup factor when warmup_steps = 0).  The formula of the reference's CameraQuatOptimizer is recalled, not
+    pinned (INTEGRATION.md "Learning the training cameras"), and its default values are not known: the two rates are
+    required, and the other defaults give constant rates."""
+    lr_q: float
+    lr_T: float
+    warmup_steps: int = 0
+    max_steps: int = 1
+    final_ratio: float = 1.0
+
+    def __post_init__(self):
+        for name in ("lr_q", "lr_T", "final_ratio"):
+            v = float(getattr(self, name))
+            if not (v >= 0.0 and math.isfinite(v)):
+                raise ValueError(f"CameraLRs: {name} must be a finite value >= 0, got {getattr(self, name)}")
+        if int(self.warmup_steps) != self.warmup_steps or self.warmup_steps < 0:
+            raise ValueError(f"CameraLRs: warmup_steps must be an integer >= 0, got {self.warmup_steps}")
+        if int(self.max_steps) != self.max_steps or self.max_steps <= self.warmup_steps:
+            raise ValueError(f"CameraLRs: max_steps must be an integer > warmup_steps, got {self.max_steps}")
+
+    def factor(self, it: int) -> float:
+        warm = 1.0 if self.warmup_steps == 0 else min(1.0, it / self.warmup_steps)
+        p = min(max((it - self.warmup_steps) / (self.max_steps - self.warmup_steps), 0.0), 1.0)
+        return warm * (self.final_ratio + (1.0 - self.final_ratio) * 0.5 * (1.0 + math.cos(math.pi * p)))
+
+    def rates(self, it: int) -> Tuple[float, float]:
+        """(lr_q, lr_T) at iteration `it`."""
+        f = self.factor(it)
+        return self.lr_q * f, self.lr_T * f
+
+
 class GaussianAdam:
     """torch.optim.Adam(groups, lr=0.0, eps=1e-15) of ONE model ("static" or "dynamic") living in the flat buffers
     of a SplatTrainStep.  `ranges`: reference group name -> (float offset, numel) inside those buffers."""

@@ -162,6 +162,7 @@ class SplatTrainStep:
         self.last_state: Optional[engine.FwdState] = None
         self._deferred = None      # exchange_grads(defer_sh=True): the factors the next optimizer_step consumes
         self.stage_events = None   # set by enable_stage_timing()
+        self.cameras = None        # enable_camera_learning(): the table of training cameras
 
     def _alloc_boxes(self):
         if self.n_local > 0:
@@ -274,14 +275,21 @@ class SplatTrainStep:
                         sh_degree=self.sh_degree, viewmatrix=viewmatrix, projmatrix=projmatrix, bg=self.bg)
         return scene, view
 
-    def forward_backward(self, viewmatrix: torch.Tensor, projmatrix: torch.Tensor, tanfovx: float, tanfovy: float,
+    def forward_backward(self, viewmatrix: Optional[torch.Tensor], projmatrix: torch.Tensor, tanfovx: float, tanfovy: float,
                          basis_t: torch.Tensor, gt_image: torch.Tensor, gt_depth: Optional[torch.Tensor],
-                         accumulate: bool = False, forward_only: bool = False, dcolor_slot: Optional[int] = None):
+                         accumulate: bool = False, forward_only: bool = False, dcolor_slot: Optional[int] = None,
+                         camera: Optional[int] = None):
         """viewmatrix / projmatrix in glm storage (V^T, P^T).  Gradients land in self.grads
         (overwritten unless accumulate=True, in which case a second flat buffer is summed in).
         dcolor_slot: data-parallel mode - do not write dL/dSH; write its 12-byte factors dL/d(rgb) into
         self.dcolor_local[dcolor_slot] instead (exchange_grads() rebuilds dL/dSH of all views from them).
+        camera: render at camera_viewmatrix(camera) of the learned camera table instead of a given viewmatrix (pass None
+        for it) and, after the backward, collect this view's dL/dV for the next camera_step (collect_camera_grad).
         Returns self.loss_parts (device tensor; no host sync)."""
+        if camera is not None:
+            if viewmatrix is not None:
+                raise ValueError("SplatTrainStep.forward_backward: pass either camera= or a viewmatrix, not both")
+            viewmatrix = self.camera_viewmatrix(camera)
         lib = _lib.load()
         stream = _lib.stream_ptr()
         deform = self.nd > 0
@@ -366,6 +374,8 @@ class SplatTrainStep:
             self.grads = saved
         if accumulate:
             self.grads.add_(target)
+        if camera is not None:
+            self.collect_camera_grad(camera)
         return self.loss_parts
 
     def capture_forward_backward(self, viewmatrix, projmatrix, tanfovx, tanfovy, basis_t, gt_image, gt_depth) -> "CapturedStep":
@@ -969,6 +979,103 @@ class SplatTrainStep:
         lp = self.loss_parts
         return lp[0] + self.w[2] * lp[3] + lp[4] + (self.w_local * lp[5] if self.n_local > 0 else 0.0)
 
+    # -- learning the training cameras (INTEGRATION.md "Learning the training cameras") ------------------------------------
+    def enable_camera_learning(self, viewmats, lrs) -> None:
+        """Learn the poses of C training cameras (the reference's CameraQuatOptimizer): a table of (q, T) rows, both camera to
+        world, with torch.optim.Adam moments (betas (0.9, 0.999), eps 1e-15), one step count shared by the table, and the
+        [C, 16] table of V(q, T) that forward_backward(camera=c) renders at.  viewmats: the initial cameras as [C, 4, 4]
+        float32 glm-storage view matrices on the step's device (converted by rodygs_b200.pose.pose_from_viewmatrix, which
+        refuses a non-rotation), or the {"R_c2ws_quat": [C, 4], "T_c2ws": [C, 3]} dict of checkpoint.export_models /
+        import_models.  lrs: rodygs_b200.optim.CameraLRs.  Replaces a table enabled before."""
+        from .optim import CameraLRs
+        from .pose import pose_from_viewmatrix
+        pre = "SplatTrainStep.enable_camera_learning"
+        if not isinstance(lrs, CameraLRs):
+            raise ValueError(f"{pre}: lrs must be a rodygs_b200.optim.CameraLRs, got {type(lrs).__name__}")
+        if isinstance(viewmats, dict):
+            q, T = viewmats.get("R_c2ws_quat"), viewmats.get("T_c2ws")
+            n = q.shape[0] if torch.is_tensor(q) and q.dim() == 2 else 0
+            if n < 1 or tuple(q.shape) != (n, 4) or not torch.is_tensor(T) or tuple(T.shape) != (n, 3):
+                raise ValueError(f"{pre}: the cameras dict needs R_c2ws_quat [C, 4] and T_c2ws [C, 3] tensors with C >= 1")
+            param = torch.cat([q.detach(), T.detach()], 1).to(self.dev, torch.float32)
+        else:
+            n = viewmats.shape[0] if torch.is_tensor(viewmats) and viewmats.dim() == 3 else 0
+            if n < 1:
+                raise ValueError(f"{pre}: viewmats must be a [C, 4, 4] tensor with C >= 1")
+            self._check_input("viewmats", viewmats, (n, 4, 4))
+            param = pose_from_viewmatrix(viewmats)
+        self._init_cameras(param, lrs)
+
+    def _init_cameras(self, param: torch.Tensor, lrs, exp_avg=None, exp_avg_sq=None, steps: int = 0):
+        f32 = dict(dtype=torch.float32, device=self.dev)
+        n = param.shape[0]
+        self.cameras = {
+            "param": param.to(**f32).contiguous().clone(),
+            "exp_avg": torch.zeros(n, 7, **f32) if exp_avg is None else exp_avg.to(**f32).contiguous().clone(),
+            "exp_avg_sq": torch.zeros(n, 7, **f32) if exp_avg_sq is None else exp_avg_sq.to(**f32).contiguous().clone(),
+            "steps": int(steps), "lrs": lrs,
+            "viewmats": torch.zeros(n, 16, **f32), "grad": torch.zeros(n, 7, **f32),
+            # dL/dV of the views collected since the last camera_step (slot s belongs to camera pending[s])
+            "slots": torch.zeros(max(1, int(getattr(self, "views_per_rank", 1))), 16, **f32), "pending": [],
+            "error": torch.zeros(1, dtype=torch.int32, device=self.dev)}
+        self._camera_views()
+
+    def _camera_views(self):
+        cam = self.cameras
+        check(_lib.load().rdg_camera_views(ptr(cam["param"]), cam["param"].shape[0], ptr(cam["viewmats"]), _lib.stream_ptr()))
+
+    def _camera(self, camera: int, fn: str) -> int:
+        if getattr(self, "cameras", None) is None:
+            raise RuntimeError(f"SplatTrainStep.{fn}: camera learning is not enabled (enable_camera_learning)")
+        n = self.cameras["param"].shape[0]
+        if isinstance(camera, bool) or int(camera) != camera or not 0 <= camera < n:
+            raise ValueError(f"SplatTrainStep.{fn}: camera must be an integer in [0, {n}), got {camera!r}")
+        return int(camera)
+
+    def camera_viewmatrix(self, camera: int) -> torch.Tensor:
+        """V(q, T) of the learned camera as a [4, 4] glm-storage view of the table (what forward_backward takes).  It changes
+        in place at every camera_step: copy it to keep a value."""
+        c = self._camera(camera, "camera_viewmatrix")
+        return self.cameras["viewmats"][c].view(4, 4)
+
+    def collect_camera_grad(self, camera: int):
+        """Queue the dL/dV of the last backward (self.view_grad) for the next camera_step, as a view of `camera`.
+        forward_backward(camera=c) does this itself; call it after a CapturedStep.replay() whose static viewmatrix buffer
+        held camera_viewmatrix(c).  The queue grows as needed; camera_step empties it."""
+        cam = self.cameras
+        c = self._camera(camera, "collect_camera_grad")
+        k = len(cam["pending"])
+        if k == cam["slots"].shape[0]:
+            grown = torch.zeros(2 * k, 16, dtype=torch.float32, device=self.dev)
+            grown[:k].copy_(cam["slots"])
+            cam["slots"] = grown
+        cam["slots"][k].copy_(self.view_grad.view(16))
+        cam["pending"].append(c)
+
+    def camera_step(self, iteration: int, grad_scale: float = 1.0) -> Tuple[float, float]:
+        """One Adam step of the whole camera table: dL/d(q, T) of every camera from the collected views (rdg_camera_grad, a
+        zero row for a camera without one, so its moments decay and momentum still moves it), a sum all-reduce over the
+        step's process group (every rank keeps the same table), then rdg_camera_adam at CameraLRs.rates(iteration) with the
+        gradient times grad_scale, which also rewrites the V(q, T) table.  Empties the queue.  One host read (the index
+        error word).  Returns (lr_q, lr_T)."""
+        self._camera(0, "camera_step")
+        cam = self.cameras
+        lib, stream = _lib.load(), _lib.stream_ptr()
+        n = cam["param"].shape[0]
+        idx = torch.tensor(cam["pending"] or [0], dtype=torch.int32).to(self.dev)
+        check(lib.rdg_camera_grad(len(cam["pending"]), ptr(idx), ptr(cam["slots"]), ptr(cam["param"]), n, ptr(cam["grad"]),
+                                  ptr(cam["error"]), stream))
+        cam["pending"] = []
+        bad = int(cam["error"])
+        if bad:
+            raise RuntimeError(f"SplatTrainStep.camera_step: slot {bad - 1} names a camera outside [0, {n}); nothing was applied")
+        allreduce_flat(cam["grad"], None, self.pg)
+        lr_q, lr_T = cam["lrs"].rates(iteration)
+        cam["steps"] += 1
+        check(lib.rdg_camera_adam(ptr(cam["param"]), ptr(cam["grad"]), ptr(cam["exp_avg"]), ptr(cam["exp_avg_sq"]), n,
+                                  cam["steps"], lr_q, lr_T, 0.9, 0.999, 1e-15, float(grad_scale), ptr(cam["viewmats"]), stream))
+        return lr_q, lr_T
+
     # -- held-out views -------------------------------------------------------------------------------------------
     def evaluate(self, viewmats: torch.Tensor, projmats: torch.Tensor, tanfovx, tanfovy, basis_ts: Optional[torch.Tensor],
                  gts: torch.Tensor, value_range: float = 1.0, masks: Optional[torch.Tensor] = None, lpips=None,
@@ -1091,6 +1198,10 @@ class SplatTrainStep:
         if d is not None and d["pending"]:
             raise RuntimeError("SplatTrainStep.state_dict: exchange_grads(defer_sh=True) left the SH gradient factors of "
                                f"{sorted(d['pending'])} pending; call optimizer_step for them first")
+        cam = getattr(self, "cameras", None)
+        if cam is not None and cam["pending"]:
+            raise RuntimeError(f"SplatTrainStep.state_dict: {len(cam['pending'])} collected camera gradients are pending; call "
+                               "camera_step first")
 
     def _dp_rank_world(self) -> Tuple[int, int]:
         import torch.distributed as dist
@@ -1135,6 +1246,10 @@ class SplatTrainStep:
                                 "betas": [float(b) for b in opt.betas], "eps": float(opt.eps), "steps": int(opt.steps),
                                 "exp_avg": {g: cpu(m.view(shapes[g])) for g, (m, _) in moments.items()},
                                 "exp_avg_sq": {g: cpu(v.view(shapes[g])) for g, (_, v) in moments.items()}}
+        cam = getattr(self, "cameras", None)
+        if cam is not None:
+            sd["cameras"] = {"param": cpu(cam["param"]), "exp_avg": cpu(cam["exp_avg"]), "exp_avg_sq": cpu(cam["exp_avg_sq"]),
+                             "steps": int(cam["steps"]), "lrs": asdict(cam["lrs"])}
         mlp = getattr(self, "mlp", None)
         if mlp is not None:
             sd["mlp"] = {"args": dict(mlp.init_args), "state_dict": {k: cpu(v) for k, v in mlp.state_dict().items()},
@@ -1210,6 +1325,18 @@ class SplatTrainStep:
             for f in STATS_FIELDS:
                 if tuple(s[f].shape) != (n,):
                     raise ValueError(f"{pre}: statistics {tag}.{f} have shape {tuple(s[f].shape)}, expected ({n},)")
+        cams = sd.get("cameras")
+        if cams is not None:
+            from .optim import CameraLRs
+            n = cams["param"].shape[0] if cams["param"].dim() == 2 else 0
+            for kind in ("param", "exp_avg", "exp_avg_sq"):
+                if n < 1 or tuple(cams[kind].shape) != (n, 7):
+                    raise ValueError(f"{pre}: cameras[{kind!r}] has shape {tuple(cams[kind].shape)}, expected [C, 7] with C >= 1")
+            have = getattr(self, "cameras", None)
+            if have is not None and have["param"].shape[0] != n:
+                raise ValueError(f"{pre}: cameras['param'] holds {n} cameras in the state dict but the camera table of this step "
+                                 f"has {have['param'].shape[0]}")
+            cams = dict(cams, lrs=CameraLRs(**cams["lrs"]), steps=int(cams["steps"]))
         if "mlp" in sd:
             m = sd["mlp"]
             if m["train_times"].numel() != T:
@@ -1217,22 +1344,23 @@ class SplatTrainStep:
             missing = [k for k in ("args", "state_dict", "lr", "steps") if k not in m]
             if missing:
                 raise ValueError(f"{pre}: the basis MLP entry has no {missing}")
-        return scene, optims, stats, rng
+        return scene, optims, stats, rng, cams
 
     def load_state_dict(self, sd: Dict):
         """Restore a state_dict(): the flat buffers are rebuilt at the saved Gaussian counts (this step may have been built
         for any other N), then the loss configuration, the optimisers, the pending post-densification skips, the
-        densification statistics, the basis MLP (built from the saved arguments when none is attached) and the CUDA
-        generator that draws the local Pearson boxes.  Every check runs before anything changes; it refuses what it cannot
+        densification statistics, the basis MLP (built from the saved arguments when none is attached), the learned camera
+        table (a state with one enables camera learning here; a state without one leaves this step's table as it is) and
+        the CUDA generator that draws the local Pearson boxes.  Every check runs before anything changes; it refuses what it cannot
         repair, naming the field: another image size, a num_basis / T / network that differs from the MLP attached to this
-        step, or a state without an MLP while one is attached.  Like densify_and_prune this replaces every buffer: a
+        step, a state without an MLP while one is attached, or a camera count that differs from this step's camera table.  Like densify_and_prune this replaces every buffer: a
         CapturedStep taken before must be captured again, and an enabled factored exchange is set up again."""
         pre = "SplatTrainStep.load_state_dict"
         if not isinstance(sd, dict) or sd.get("format") != CHECKPOINT_FORMAT or sd.get("version") != CHECKPOINT_VERSION:
             got = (sd.get("format"), sd.get("version")) if isinstance(sd, dict) else type(sd).__name__
             raise ValueError(f"{pre}: not a {CHECKPOINT_FORMAT} v{CHECKPOINT_VERSION} state dict ({got!r})")
         try:
-            scene, optims, stats, rng = self._parse_state(sd)
+            scene, optims, stats, rng, cams = self._parse_state(sd)
         except (KeyError, TypeError, AttributeError) as e:
             raise ValueError(f"{pre}: malformed state dict ({type(e).__name__}: {e})") from None
         from .densify import DensifyStats
@@ -1269,6 +1397,8 @@ class SplatTrainStep:
             self._mlp_steps = int(m["steps"])
             if "exp_avg" in m:
                 self._mlp_moments = (m["exp_avg"].to(self.dev), m["exp_avg_sq"].to(self.dev))
+        if cams is not None:
+            self._init_cameras(cams["param"], cams["lrs"], cams["exp_avg"], cams["exp_avg_sq"], cams["steps"])
         torch.cuda.set_rng_state(rng, self.dev)
         if getattr(self, "_fx_args", None) is not None:          # the exchange buffers are sized by the Gaussian count
             self.enable_factored_exchange(*self._fx_args)
