@@ -195,6 +195,15 @@ int rdg_set_tunable(const char* name, int32_t value);
 /* deformation + activations + EWA projection + SH->RGB (SURVEY.md §8 a2-a7). */
 int rdg_preprocess_fwd(const RdgScene* scene, const RdgView* view, const RdgGeom* geom, void* stream);
 
+/* rdg_preprocess_fwd of num_views (1..8) views of one scene in ONE launch: each 256-Gaussian chunk's parameters are read
+ * once and projected into every view.  geoms[v] receives exactly what rdg_preprocess_fwd(scene with basis_t = basis_ts + v
+ * * num_basis * 7, &views[v], &geoms[v]) writes, bit for bit.  The views must share height, width, sh_degree and
+ * scale_modifier; viewmatrix, projmatrix, tanfovx / tanfovy and bg may differ.  scene->basis_t must be NULL: B(t) of view v
+ * is row v of basis_ts [num_views, num_basis, 7] (needed with deformation only).  Returns RDG_E_ARG before any launch
+ * when one of these does not hold. */
+int rdg_preprocess_fwd_views(const RdgScene* scene, const float* basis_ts, int32_t num_views, const RdgView* views,
+                             const RdgGeom* geoms, void* stream);
+
 /* bytes of scratch rdg_bin needs for N Gaussians and at most d_cap duplicates. */
 int64_t rdg_bin_workspace_bytes(int64_t n, int64_t d_cap, int32_t height, int32_t width);
 

@@ -111,6 +111,8 @@ SYMBOLS = {
     "rdg_set_tunable": (C.c_int, [C.c_char_p, C.c_int32]),
     "rdg_alpha_reg": (C.c_int, [c_ptr, C.c_int64, C.c_float, c_ptr, c_ptr, c_ptr]),
     "rdg_preprocess_fwd": (C.c_int, [C.POINTER(RdgScene), C.POINTER(RdgView), C.POINTER(RdgGeom), c_ptr]),
+    "rdg_preprocess_fwd_views": (C.c_int, [C.POINTER(RdgScene), c_ptr, C.c_int32, C.POINTER(RdgView), C.POINTER(RdgGeom),
+                                           c_ptr]),
     "rdg_bin_workspace_bytes": (C.c_int64, [C.c_int64, C.c_int64, C.c_int32, C.c_int32]),
     "rdg_bin": (C.c_int, [C.c_int64, C.POINTER(RdgGeom), C.c_int32, C.c_int32, C.c_int64, C.POINTER(RdgBins),
                           c_ptr, C.c_int64, c_ptr]),

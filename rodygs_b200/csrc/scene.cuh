@@ -89,7 +89,37 @@ __device__ __forceinline__ void rdg_deform_delta(const RdgScene& sc, const float
     }
 }
 
-template <bool RAW>
+// delta[j] = sum_k c_k (B(t)[k][j] - table[ti][k][j]) from a table row staged in shared memory (stride RDG_DIFF_STRIDE,
+// num_basis == RDG_NUM_BASIS_MAX) and B(t) kept apart: the batched forward stages the table once for all its views.  The
+// difference is rounded on its own before the FMA, so the result has the bits of rdg_deform_delta's.
+__device__ __forceinline__ void rdg_deform_delta_rows(const float* basis_t, const float* row_s, const float* c, float* d) {
+#pragma unroll
+    for (int j = 0; j < 7; ++j) d[j] = 0.f;
+    const float4* row4 = reinterpret_cast<const float4*>(row_s);
+    const float4* bt4 = reinterpret_cast<const float4*>(basis_t);
+#pragma unroll
+    for (int q = 0; q < 28; ++q) {
+        const float4 v = row4[q], b = bt4[q];
+        const float r[4] = {v.x, v.y, v.z, v.w}, bb[4] = {b.x, b.y, b.z, b.w};
+#pragma unroll
+        for (int m = 0; m < 4; ++m) {
+            const int e = 4 * q + m;
+            d[e % 7] = fmaf(c[e / 7], bb[m] - r[m], d[e % 7]);
+        }
+    }
+}
+
+// The deformation delta (rdg_deform_delta) applied to the activated parameters.
+__device__ __forceinline__ void rdg_apply_deform(const RdgScene& sc, const float* d, RdgAct& a) {
+    a.x += d[0] * sc.spatial_lr_scale;
+    a.y += d[1] * sc.spatial_lr_scale;
+    a.z += d[2] * sc.spatial_lr_scale;
+    a.q[0] += d[3]; a.q[1] += d[4]; a.q[2] += d[5]; a.q[3] += d[6];
+}
+
+// Loads, activations and (DEFORM) the deformation of one Gaussian.  DEFORM = false stops at the canonical mean and
+// quaternion and leaves a.c / a.ti loaded: the batched forward deforms each view's copy itself.
+template <bool RAW, bool DEFORM = true>
 __device__ __forceinline__ void rdg_fetch(const RdgScene& sc, bool dyn, int64_t local, const float* basis_t, RdgAct& a,
                                           const float* diff_s = nullptr) {
     a.dyn = dyn;
@@ -124,12 +154,11 @@ __device__ __forceinline__ void rdg_fetch(const RdgScene& sc, bool dyn, int64_t 
 #pragma unroll
                 for (int k = 0; k < RDG_NUM_BASIS_MAX; ++k) a.c[k] = k < sc.num_basis ? __ldg(pc + k) : 0.f;
             }
-            float d[7];
-            rdg_deform_delta(sc, basis_t, a.ti, a.c, d, diff_s);
-            a.x += d[0] * sc.spatial_lr_scale;
-            a.y += d[1] * sc.spatial_lr_scale;
-            a.z += d[2] * sc.spatial_lr_scale;
-            a.q[0] += d[3]; a.q[1] += d[4]; a.q[2] += d[5]; a.q[3] += d[6];
+            if (DEFORM) {
+                float d[7];
+                rdg_deform_delta(sc, basis_t, a.ti, a.c, d, diff_s);
+                rdg_apply_deform(sc, d, a);
+            }
         }
     } else {
         a.s[0] = s0; a.s[1] = s1; a.s[2] = s2;

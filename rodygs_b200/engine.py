@@ -358,6 +358,74 @@ def render_forward(scene: SceneArgs, view: ViewArgs, keep_for_backward: bool = T
     return color, depth, alpha, geom["radii"], state
 
 
+VIEWS_PER_LAUNCH = 8   # rdg_preprocess_fwd_views
+
+
+def render_views(scene: SceneArgs, views, basis_ts: Optional[torch.Tensor], stage_hook=None):
+    """render_forward of every view in `views` (ViewArgs sharing height, width, sh_degree and scale_modifier; scene.basis_t
+    None, B(t) of view v = basis_ts[v]), with the same bits.  Passes of up to 8 views: ONE rdg_preprocess_fwd_views, ONE host
+    read of the pass's duplicate counts (sums of each view's tile counts), then binning buffers of exactly that size and
+    rdg_bin_tiles + rdg_blend_fwd per view, so nothing overflows or is re-binned.  The duplicate-capacity state
+    (_capacity, a pending sync-free count) is neither read nor changed.
+    Returns (color [V,3,H,W], depth [V,1,H,W], alpha [V,1,H,W], radii [V,N] int32)."""
+    lib = _lib.load()
+    ns, nd = scene.counts()
+    n = ns + nd
+    V = len(views)
+    dev = views[0].viewmatrix.device
+    if dev.type != "cuda":
+        raise RuntimeError("rodygs_b200 runs on CUDA tensors only (no CPU fallback)")
+    stream = _lib.stream_ptr()
+    H, W = int(views[0].height), int(views[0].width)
+    ntiles = tiles_of(H, W)
+    f32 = dict(dtype=torch.float32, device=dev)
+    color = torch.empty(V, 3, H, W, **f32)
+    depth = torch.empty(V, 1, H, W, **f32)
+    alpha = torch.empty(V, 1, H, W, **f32)
+    radii = torch.empty(V, n, dtype=torch.int32, device=dev)
+    sc_s = _scene_struct(scene)
+    final_T = torch.empty(H, W, **f32)
+    n_contrib = torch.empty(H, W, dtype=torch.int32, device=dev)
+    ranges = torch.empty(ntiles, 2, dtype=torch.int32, device=dev)
+    num_rendered = torch.empty(2, dtype=torch.int32, device=dev)
+    region_count = torch.empty(2 * ntiles, dtype=torch.int32, device=dev)
+    for lo in range(0, V, VIEWS_PER_LAUNCH):
+        pv = views[lo:lo + VIEWS_PER_LAUNCH]
+        k = len(pv)
+        # zeroed here as well: without Gaussians the kernel returns before it zeroes them, and the counts must still read 0
+        tile_count = torch.zeros(k, ntiles + 1, dtype=torch.int32, device=dev)
+        geoms = [{"radii": radii[lo + j], "tiles_touched": torch.empty(n, dtype=torch.int32, device=dev),
+                  "p0": torch.empty(n, 4, **f32), "p1": torch.empty(n, 4, **f32), "p2": torch.empty(n, 2, **f32),
+                  "clamped": torch.empty(n, dtype=torch.uint8, device=dev), "tile_count": tile_count[j]} for j in range(k)]
+        vw_s = (RdgView * k)(*[_view_struct(v) for v in pv])
+        gm_s = (RdgGeom * k)(*[_geom_struct(g) for g in geoms])
+        bts = None if basis_ts is None else basis_ts[lo:lo + k].contiguous()
+        check(lib.rdg_preprocess_fwd_views(C.byref(sc_s), ptr(bts), k, vw_s, gm_s, stream))
+        if stage_hook:
+            stage_hook("preprocess_fwd")
+        counts = tile_count[:, :ntiles].sum(1).tolist()          # the pass's one host read
+        for j in range(k):
+            d_cap = max(int(counts[j]), 1)
+            vals = torch.empty(d_cap, dtype=torch.int32, device=dev)
+            region_ids = torch.empty(2 * d_cap, dtype=torch.int32, device=dev)
+            region_masks = torch.empty(2 * d_cap, dtype=torch.uint8, device=dev)
+            ws_bytes = int(lib.rdg_bin_tiles_workspace_bytes(n, d_cap, H, W))
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+            bins = RdgBins()
+            bins.vals_sorted, bins.ranges, bins.num_rendered = ptr(vals), ptr(ranges), ptr(num_rendered)
+            bins.region_ids, bins.region_masks, bins.region_count = ptr(region_ids), ptr(region_masks), ptr(region_count)
+            bins.region_stride = d_cap
+            check(lib.rdg_bin_tiles(n, C.byref(gm_s[j]), H, W, d_cap, C.byref(bins), ptr(ws), ws_bytes, stream))
+            img = RdgImage()
+            v = lo + j
+            img.color, img.depth, img.alpha = ptr(color[v]), ptr(depth[v]), ptr(alpha[v])
+            img.final_T, img.n_contrib = ptr(final_T), ptr(n_contrib)
+            check(lib.rdg_blend_fwd(n, C.byref(gm_s[j]), C.byref(bins), C.byref(vw_s[j]), C.byref(img), stream))
+        if stage_hook:
+            stage_hook("bin_blend")
+    return color, depth, alpha, radii
+
+
 @dataclass
 class SetGrads:
     xyz: Optional[torch.Tensor] = None

@@ -1155,6 +1155,39 @@ class SplatTrainStep:
         allreduce_flat(table, None, self.pg)
         return table
 
+    def render_views(self, viewmats: torch.Tensor, projmats: torch.Tensor, tanfovx, tanfovy,
+                     basis_ts: Optional[torch.Tensor]) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+        """Render V views with this step's background, SH degree and scale_modifier 1: returns (color [V, 3, H, W],
+        depth [V, 1, H, W], alpha [V, 1, H, W], radii [V, N] int32), the colour not clamped.  Bit for bit what
+        engine.render_forward returns for each view on its own.
+
+        Arguments as for evaluate, without gts: viewmats / projmats [V, 4, 4] in glm storage, tanfovx / tanfovy a float or
+        V values, basis_ts [V, K, 7] (None without dynamic Gaussians).  Views go through rdg_preprocess_fwd_views 8 at a
+        time, so each pass reads the Gaussians once; each pass then makes one host read of its duplicate counts and bins
+        every view in buffers of exactly that size.
+
+        No training state changes (the list of evaluate, plus the camera table and engine's duplicate capacity): a pending
+        sync-free duplicate count stays pending for the training step that owns it.  Data parallel: no collective; every
+        rank renders the views it is given (shard them with shard_views)."""
+        V = viewmats.shape[0] if torch.is_tensor(viewmats) else 0
+        if V < 1:
+            raise ValueError("SplatTrainStep.render_views: viewmats must be a [V, 4, 4] tensor with V >= 1")
+        self._check_input("viewmats", viewmats, (V, 4, 4))
+        self._check_input("projmats", projmats, (V, 4, 4))
+        if self.nd > 0:
+            self._check_input("basis_ts", basis_ts, (V, self.num_basis, 7))
+
+        def per_view(name, v):
+            vals = [float(t) for t in v] if hasattr(v, "__len__") else [float(v)] * V
+            if len(vals) != V:
+                raise ValueError(f"SplatTrainStep.render_views: {name} must be a float or {V} values, got {len(vals)}")
+            return vals
+
+        fovx, fovy = per_view("tanfovx", tanfovx), per_view("tanfovy", tanfovy)
+        scene, _ = self._scene_view(viewmats[0], projmats[0], fovx[0], fovy[0], None)
+        views = [self._scene_view(viewmats[v], projmats[v], fovx[v], fovy[v], None)[1] for v in range(V)]
+        return engine.render_views(scene, views, basis_ts if self.nd > 0 else None)
+
     def refine_poses(self, viewmats: torch.Tensor, projmats: torch.Tensor, tanfovx, tanfovy, gts: torch.Tensor, lr: float,
                      iters: int = 1000) -> Tuple[torch.Tensor, torch.Tensor]:
         """Test-time pose refinement of V held-out views (the reference's PoseOptimizer; rodygs_b200.pose.refine_poses) with
