@@ -204,6 +204,33 @@ int rdg_preprocess_fwd(const RdgScene* scene, const RdgView* view, const RdgGeom
 int rdg_preprocess_fwd_views(const RdgScene* scene, const float* basis_ts, int32_t num_views, const RdgView* views,
                              const RdgGeom* geoms, void* stream);
 
+/* ---- point tracking (INTEGRATION.md §10) ---------------------------------- */
+
+/* For every Gaussian with geom->radii > 0, its centre at the target time, mu_k(t_m) = xyz (static), or xyz +
+ * spatial_lr_scale * sum_b c_kb (B(t_m) - table[t_k])_b[0:3] (dynamic, raw = 1 with use_deform; the preprocess's
+ * deformation in its operation order), is written into the record's colour slots p1.z, p1.w, p2.x; no other field
+ * changes.  rdg_blend_fwd over the source view's bins with a zero background then blends S_m(p) = sum_k w_k(p) mu_k(t_m)
+ * with the source render's weights.  geom: the source view's rdg_preprocess_fwd output (radii, p1, p2 required).
+ * basis_t_target [num_basis, 7] = B(t_m) (needed with deformation only); scene->basis_t must be NULL.  positions_out:
+ * optional [N, 3], static rows first, receives mu_k(t_m) of EVERY Gaussian.  Returns RDG_E_ARG before any launch on a
+ * bad argument. */
+int rdg_track_attrs(const RdgScene* scene, const float* basis_t_target, const RdgGeom* geom, float* positions_out,
+                    void* stream);
+
+/* Tracked points X = S_m / A of M targets, projected into target m with rdg_preprocess_fwd's arithmetic: v = V_m X,
+ * c = P_m v, ndc = c.xy / (c.w + 1e-7), px = ((ndc.x + 1) W - 1) / 2, py = ((ndc.y + 1) H - 1) / 2, depth = v.z (as
+ * is, also behind the camera).  Where A == 0 every output is NaN.  S [M, 3, H, W] (rdg_blend_fwd colour of each
+ * target's rdg_track_attrs), A [H, W] (the source alpha), viewmats / projmats [M, 16] glm storage, M = 1..65535.
+ *   points == NULL (dense): xy_out [M, 2, H, W], depth_out [M, 1, H, W]; P and alpha_out are not used.
+ *   points [P, 2] (sparse, pixel (x, y) centred at integer x, y): S_m and A are sampled bilinearly between pixel centres,
+ *   clamped to the image, each interpolation written a + f (b - a) (an integer point reads its pixel's bits), then
+ *   normalised and projected: xy_out [M, P, 2], depth_out [M, P], alpha_out (optional) [P] the sampled A.
+ * One thread per output position, no atomics: bit-identical from run to run.  Returns RDG_E_ARG before any launch on a bad
+ * argument (P < 0 included). */
+int rdg_track_project(const float* S, const float* A, int32_t M, int32_t height, int32_t width, const float* viewmats,
+                      const float* projmats, const float* points, int64_t P, float* xy_out, float* depth_out,
+                      float* alpha_out, void* stream);
+
 /* bytes of scratch rdg_bin needs for N Gaussians and at most d_cap duplicates. */
 int64_t rdg_bin_workspace_bytes(int64_t n, int64_t d_cap, int32_t height, int32_t width);
 

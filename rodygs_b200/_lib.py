@@ -113,6 +113,9 @@ SYMBOLS = {
     "rdg_preprocess_fwd": (C.c_int, [C.POINTER(RdgScene), C.POINTER(RdgView), C.POINTER(RdgGeom), c_ptr]),
     "rdg_preprocess_fwd_views": (C.c_int, [C.POINTER(RdgScene), c_ptr, C.c_int32, C.POINTER(RdgView), C.POINTER(RdgGeom),
                                            c_ptr]),
+    "rdg_track_attrs": (C.c_int, [C.POINTER(RdgScene), c_ptr, C.POINTER(RdgGeom), c_ptr, c_ptr]),
+    "rdg_track_project": (C.c_int, [c_ptr, c_ptr, C.c_int32, C.c_int32, C.c_int32, c_ptr, c_ptr, c_ptr, C.c_int64, c_ptr,
+                                    c_ptr, c_ptr, c_ptr]),
     "rdg_bin_workspace_bytes": (C.c_int64, [C.c_int64, C.c_int64, C.c_int32, C.c_int32]),
     "rdg_bin": (C.c_int, [C.c_int64, C.POINTER(RdgGeom), C.c_int32, C.c_int32, C.c_int64, C.POINTER(RdgBins),
                           c_ptr, C.c_int64, c_ptr]),

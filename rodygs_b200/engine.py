@@ -426,6 +426,107 @@ def render_views(scene: SceneArgs, views, basis_ts: Optional[torch.Tensor], stag
     return color, depth, alpha, radii
 
 
+TARGETS_PER_PASS = 8   # engine.track: bounds the blended maps at 8 x 3 x H x W floats
+
+
+def track(scene: SceneArgs, view_src: ViewArgs, basis_t_src: Optional[torch.Tensor], target_viewmats: torch.Tensor,
+          target_projmats: torch.Tensor, target_basis_ts: Optional[torch.Tensor], points: Optional[torch.Tensor] = None,
+          stage_hook=None, keep_maps: bool = False):
+    """Where each pixel (or query point) of the source render goes at M target camera-times (INTEGRATION.md §10).
+    scene.basis_t None; B(t_s) = basis_t_src, B(t_m) = target_basis_ts[m] (both None without deformation);
+    target_viewmats / target_projmats [M, 4, 4] glm storage; points None or [P, 2] pixel coordinates.
+
+    One rdg_preprocess_fwd of the source view, ONE host read of its duplicate count, exactly sized binning buffers
+    (rdg_bin_tiles); then targets in passes of at most 8: per target rdg_track_attrs + rdg_blend_fwd (zero background) into
+    S [k, 3, H, W], and one rdg_track_project per pass.  The duplicate-capacity state (_capacity, a pending sync-free count)
+    is neither read nor changed.  stage_hook(name) is called after "source" (preprocess + binning) and after every "attrs",
+    "blend" and "project" launch.  keep_maps (tests): also return S_m of every target [M, 3, H, W] and mu_k(t_m)
+    [M, N, 3] (rdg_track_attrs' positions_out).
+    Returns dense (xy [M, 2, H, W], depth [M, 1, H, W], alpha [1, H, W]) or sparse (xy [M, P, 2], depth [M, P],
+    alpha [P]), then (S, positions) with keep_maps."""
+    lib = _lib.load()
+    ns, nd = scene.counts()
+    n = ns + nd
+    M = target_viewmats.shape[0]
+    dev = view_src.viewmatrix.device
+    if dev.type != "cuda":
+        raise RuntimeError("rodygs_b200 runs on CUDA tensors only (no CPU fallback)")
+    stream = _lib.stream_ptr()
+    H, W = int(view_src.height), int(view_src.width)
+    ntiles = tiles_of(H, W)
+    f32 = dict(dtype=torch.float32, device=dev)
+    # the source render: its records, bins and alpha are shared by every target
+    geom = {"radii": torch.empty(n, dtype=torch.int32, device=dev), "tiles_touched": torch.empty(n, dtype=torch.int32, device=dev),
+            "p0": torch.empty(n, 4, **f32), "p1": torch.empty(n, 4, **f32), "p2": torch.empty(n, 2, **f32),
+            "clamped": torch.empty(n, dtype=torch.uint8, device=dev),
+            # zeroed here as well: without Gaussians preprocess returns before it zeroes them
+            "tile_count": torch.zeros(ntiles + 1, dtype=torch.int32, device=dev)}
+    sc_s, gm_s = _scene_struct(scene), _geom_struct(geom)
+    sc_s.basis_t = ptr(basis_t_src) if sc_s.use_deform else None
+    check(lib.rdg_preprocess_fwd(C.byref(sc_s), C.byref(_view_struct(view_src)), C.byref(gm_s), stream))
+    sc_s.basis_t = None                                          # rdg_track_attrs takes B(t_m) on its own
+    d_cap = max(int(geom["tile_count"][:ntiles].sum()), 1)      # the call's one host read
+    vals = torch.empty(d_cap, dtype=torch.int32, device=dev)
+    ranges = torch.empty(ntiles, 2, dtype=torch.int32, device=dev)
+    num_rendered = torch.empty(2, dtype=torch.int32, device=dev)
+    region_ids = torch.empty(2 * d_cap, dtype=torch.int32, device=dev)
+    region_masks = torch.empty(2 * d_cap, dtype=torch.uint8, device=dev)
+    region_count = torch.empty(2 * ntiles, dtype=torch.int32, device=dev)
+    ws_bytes = int(lib.rdg_bin_tiles_workspace_bytes(n, d_cap, H, W))
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    bins = RdgBins()
+    bins.vals_sorted, bins.ranges, bins.num_rendered = ptr(vals), ptr(ranges), ptr(num_rendered)
+    bins.region_ids, bins.region_masks, bins.region_count = ptr(region_ids), ptr(region_masks), ptr(region_count)
+    bins.region_stride = d_cap
+    check(lib.rdg_bin_tiles(n, C.byref(gm_s), H, W, d_cap, C.byref(bins), ptr(ws), ws_bytes, stream))
+    if stage_hook:
+        stage_hook("source")
+
+    zero_bg = torch.zeros(3, **f32)
+    vw_blend = _view_struct(view_src)
+    vw_blend.bg = ptr(zero_bg)
+    alpha = torch.empty(1, H, W, **f32)
+    blend_depth = torch.empty(1, H, W, **f32)
+    final_T = torch.empty(H, W, **f32)
+    n_contrib = torch.empty(H, W, dtype=torch.int32, device=dev)
+    vms, pms = target_viewmats.contiguous(), target_projmats.contiguous()
+    sparse = points is not None
+    P = points.shape[0] if sparse else 0
+    if sparse:
+        xy, depth = torch.empty(M, P, 2, **f32), torch.empty(M, P, **f32)
+        alpha_pts = torch.empty(P, **f32)
+    else:
+        xy, depth = torch.empty(M, 2, H, W, **f32), torch.empty(M, 1, H, W, **f32)
+    S_all = torch.empty(M, 3, H, W, **f32) if keep_maps else None
+    positions = torch.empty(M, n, 3, **f32) if keep_maps else None
+    S_pass = None if keep_maps else torch.empty(min(M, TARGETS_PER_PASS), 3, H, W, **f32)
+    for lo in range(0, M, TARGETS_PER_PASS):
+        k = min(TARGETS_PER_PASS, M - lo)
+        S = S_all[lo:lo + k] if keep_maps else S_pass[:k]
+        for j in range(k):
+            m = lo + j
+            bt = None if target_basis_ts is None or not sc_s.use_deform else target_basis_ts[m]
+            check(lib.rdg_track_attrs(C.byref(sc_s), ptr(bt), C.byref(gm_s), ptr(positions[m]) if keep_maps else None, stream))
+            if stage_hook:
+                stage_hook("attrs")
+            img = RdgImage()
+            img.color, img.depth, img.alpha = ptr(S[j]), ptr(blend_depth), ptr(alpha)
+            img.final_T, img.n_contrib = ptr(final_T), ptr(n_contrib)
+            check(lib.rdg_blend_fwd(n, C.byref(gm_s), C.byref(bins), C.byref(vw_blend), C.byref(img), stream))
+            if stage_hook:
+                stage_hook("blend")
+        if not sparse:
+            check(lib.rdg_track_project(ptr(S), ptr(alpha), k, H, W, ptr(vms[lo:lo + k]), ptr(pms[lo:lo + k]), None, 0,
+                                        ptr(xy[lo:lo + k]), ptr(depth[lo:lo + k]), None, stream))
+        elif P > 0:                                              # without query points the empty outputs have no storage
+            check(lib.rdg_track_project(ptr(S), ptr(alpha), k, H, W, ptr(vms[lo:lo + k]), ptr(pms[lo:lo + k]), ptr(points), P,
+                                        ptr(xy[lo:lo + k]), ptr(depth[lo:lo + k]), ptr(alpha_pts), stream))
+        if stage_hook:
+            stage_hook("project")
+    out = (xy, depth, alpha_pts if sparse else alpha)
+    return out + (S_all, positions) if keep_maps else out
+
+
 @dataclass
 class SetGrads:
     xyz: Optional[torch.Tensor] = None

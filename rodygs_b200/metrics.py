@@ -304,3 +304,26 @@ def trajectory_errors(pred_c2w: torch.Tensor, gt_c2w: torch.Tensor):
     sin = torch.stack([rel[:, 2, 1] - rel[:, 1, 2], rel[:, 0, 2] - rel[:, 2, 0], rel[:, 1, 0] - rel[:, 0, 1]], -1).norm(dim=-1) / 2.0
     rpe_rot = torch.rad2deg(torch.atan2(sin, cos)).mean()
     return ate, rpe_trans, rpe_rot
+
+
+def pck(pred: torch.Tensor, gt: torch.Tensor, visible: torch.Tensor, height: int, width: int, ratio: float = 0.05):
+    """PCK-T (percentage of correct keypoint transfers), [B] float64 on the inputs' device (no host read): for each row b
+    the fraction of the points with visible[b] != 0 whose prediction lies strictly within ratio * max(height, width) pixels
+    of the ground truth, |pred - gt|_2 < ratio * max(H, W).  pred / gt [B, P, 2] pixel coordinates, visible [B, P] (bool or
+    numbers).  A NaN prediction counts as wrong; a row without a visible point is NaN.
+
+    DyCheck's keypoint-transfer protocol, as recalled and not pinned (INTEGRATION.md §10): a ratio of 0.05 of the longer
+    side, pairs of training frames, keypoints counted where they are visible in both frames; the caller converts DyCheck's
+    keypoint pixel convention to the rasterizer's (pixel (x, y) centred at integer x, y) before tracking.  Computed in
+    float64 with torch, as trajectory_errors: B x P is at most a few thousand points."""
+    if not (torch.is_tensor(pred) and torch.is_tensor(gt) and torch.is_tensor(visible) and pred.dim() == 3
+            and pred.shape[-1] == 2 and pred.shape == gt.shape and tuple(visible.shape) == tuple(pred.shape[:2])
+            and pred.device == gt.device == visible.device):
+        got = [f"{tuple(t.shape)} {t.device}" if torch.is_tensor(t) else type(t).__name__ for t in (pred, gt, visible)]
+        raise ValueError(f"pck: pred and gt must be [B, P, 2] and visible [B, P] tensors on one device, got {got}")
+    if not (int(height) > 0 and int(width) > 0 and ratio > 0):
+        raise ValueError(f"pck: height, width and ratio must be positive, got {height}, {width}, {ratio}")
+    vis = visible != 0
+    dist = torch.linalg.vector_norm(pred.double() - gt.double(), dim=-1)
+    correct = (dist < ratio * max(int(height), int(width))) & vis        # NaN < x is False: a NaN prediction is wrong
+    return correct.sum(-1).double() / vis.sum(-1).double()                 # 0 / 0 = NaN: no visible point

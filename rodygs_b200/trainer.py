@@ -1188,6 +1188,55 @@ class SplatTrainStep:
         views = [self._scene_view(viewmats[v], projmats[v], fovx[v], fovy[v], None)[1] for v in range(V)]
         return engine.render_views(scene, views, basis_ts if self.nd > 0 else None)
 
+    def track_maps(self, viewmat: torch.Tensor, projmat: torch.Tensor, tanfovx: float, tanfovy: float,
+                   basis_t: Optional[torch.Tensor], target_viewmats: torch.Tensor, target_projmats: torch.Tensor,
+                   target_basis_ts: Optional[torch.Tensor]) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        """Where every pixel of a source view goes at M target camera-times, through the learned motion (INTEGRATION.md
+        §10): returns (xy [M, 2, H, W] pixel coordinates in target m, depth [M, 1, H, W] view-space z in target m,
+        alpha [1, H, W] the source render's alpha).  Where alpha == 0 every output is NaN; filter on alpha as you need.
+
+        The source view is (viewmat, projmat [4, 4] glm storage, tanfovx, tanfovy, basis_t [K, 7] = B(t_s)); target m is
+        (target_viewmats[m], target_projmats[m] [M, 4, 4], target_basis_ts[m] [M, K, 7] = B(t_m)).  The basis arguments are
+        None without dynamic Gaussians.  A learned training camera c comes in as camera_viewmatrix(c).  The tracked point
+        is the source render's weighted mean of the Gaussians' centres at t_m (the weights of the render with this step's
+        background, SH degree and scale_modifier 1), projected into target m.
+
+        No training state changes (the list of render_views, the camera table included).  Data parallel: no collective;
+        every rank tracks the pairs it is given."""
+        return self._track("track_maps", viewmat, projmat, tanfovx, tanfovy, basis_t, target_viewmats, target_projmats,
+                           target_basis_ts, None)
+
+    def track_points(self, viewmat: torch.Tensor, projmat: torch.Tensor, tanfovx: float, tanfovy: float,
+                     basis_t: Optional[torch.Tensor], target_viewmats: torch.Tensor, target_projmats: torch.Tensor,
+                     target_basis_ts: Optional[torch.Tensor], points: torch.Tensor
+                     ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        """track_maps at P query points of the source view: points [P, 2] float32 (x, y) in the rasterizer's pixel
+        convention (pixel (x, y) is centred at integer x, y).  The blended maps are sampled bilinearly between pixel
+        centres, clamped to the image, then normalised and projected; an integer point returns what track_maps gives at
+        that pixel, bit for bit.  Returns (xy [M, P, 2], depth [M, P], alpha [P] the sampled source alpha)."""
+        return self._track("track_points", viewmat, projmat, tanfovx, tanfovy, basis_t, target_viewmats, target_projmats,
+                           target_basis_ts, points)
+
+    def _track(self, fn, viewmat, projmat, tanfovx, tanfovy, basis_t, target_viewmats, target_projmats, target_basis_ts,
+               points):
+        M = target_viewmats.shape[0] if torch.is_tensor(target_viewmats) and target_viewmats.dim() == 3 else 0
+        if M < 1:
+            raise ValueError(f"SplatTrainStep.{fn}: target_viewmats must be a [M, 4, 4] tensor with M >= 1")
+        self._check_input("viewmat", viewmat, (4, 4))
+        self._check_input("projmat", projmat, (4, 4))
+        self._check_input("target_viewmats", target_viewmats, (M, 4, 4))
+        self._check_input("target_projmats", target_projmats, (M, 4, 4))
+        if self.nd > 0:
+            self._check_input("basis_t", basis_t, (self.num_basis, 7))
+            self._check_input("target_basis_ts", target_basis_ts, (M, self.num_basis, 7))
+        if points is not None or fn == "track_points":
+            P = points.shape[0] if torch.is_tensor(points) and points.dim() == 2 else 0
+            self._check_input("points", points, (P, 2))
+        scene, view = self._scene_view(viewmat, projmat, float(tanfovx), float(tanfovy), None)
+        deform = self.nd > 0
+        return engine.track(scene, view, basis_t if deform else None, target_viewmats, target_projmats,
+                            target_basis_ts if deform else None, points)
+
     def refine_poses(self, viewmats: torch.Tensor, projmats: torch.Tensor, tanfovx, tanfovy, gts: torch.Tensor, lr: float,
                      iters: int = 1000) -> Tuple[torch.Tensor, torch.Tensor]:
         """Test-time pose refinement of V held-out views (the reference's PoseOptimizer; rodygs_b200.pose.refine_poses) with
