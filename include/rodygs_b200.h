@@ -231,6 +231,30 @@ int rdg_track_project(const float* S, const float* A, int32_t M, int32_t height,
                       const float* projmats, const float* points, int64_t P, float* xy_out, float* depth_out,
                       float* alpha_out, void* stream);
 
+/* ---- export as a 3D Gaussian Splatting PLY (INTEGRATION.md §11) ---------- */
+
+#define RDG_3DGS_RECORD_FLOATS 62
+
+/* The scene at the time of scene->basis_t = B(t), as the vertex records of 3DGS's PLY file (save_ply): records [N, 62]
+ * float32, static Gaussians first, then dynamic ones (the order of radii), each in the property order of 3DGS's
+ * construct_list_of_attributes:
+ *   x y z nx ny nz f_dc_0..2 f_rest_0..44 opacity scale_0..2 rot_0..3
+ * f_dc_c = sh_dc[c]; f_rest_{15 c + k - 1} = sh_rest[3 (k - 1) + c] (channel-major, the transpose of RdgSet's
+ * coefficient-major rows; strides honoured), 0 for coefficients of degree above sh_degree (0..3); nx ny nz = 0; opacity is
+ * the raw logit.
+ *   static:  x y z, scale (log), rot (un-normalised) and opacity are the raw parameters, bit for bit.
+ *   dynamic: x y z is the deformed mean, with the bits of rdg_preprocess_fwd's.  The quaternion q' = normalize(q) + dq(t)
+ *            is not re-normalised and R(q') (rdg_preprocess_fwd's unit-quaternion formula) is no rotation when |q'| != 1,
+ *            so the record factors the covariance the rasterizer draws: Sigma = M M^T, M = R(q') diag(exp(scaling)) from
+ *            the float32 q' and scales, formed in float64 and decomposed Sigma = U diag(lambda) U^T (float64 Jacobi,
+ *            deterministic, det U = +1); rot = the unit quaternion of U with rot_0 >= 0, scale_j = 0.5 log(max(lambda_j,
+ *            FLT_MIN)).  The FLT_MIN floor keeps singular and rounding-negative lambda finite: such an axis is written
+ *            as scale -43.67, which a viewer draws as flat.
+ * raw must be 1 and colors_precomp NULL; with deformation, scene->basis_t, motion_coeff, time_ind and table are required.
+ * N == 0 returns RDG_OK without a launch (records may then be NULL).  Returns RDG_E_ARG before any launch on a bad
+ * argument. */
+int rdg_export_3dgs(const RdgScene* scene, int32_t sh_degree, float* records, void* stream);
+
 /* bytes of scratch rdg_bin needs for N Gaussians and at most d_cap duplicates. */
 int64_t rdg_bin_workspace_bytes(int64_t n, int64_t d_cap, int32_t height, int32_t width);
 

@@ -116,6 +116,7 @@ SYMBOLS = {
     "rdg_track_attrs": (C.c_int, [C.POINTER(RdgScene), c_ptr, C.POINTER(RdgGeom), c_ptr, c_ptr]),
     "rdg_track_project": (C.c_int, [c_ptr, c_ptr, C.c_int32, C.c_int32, C.c_int32, c_ptr, c_ptr, c_ptr, C.c_int64, c_ptr,
                                     c_ptr, c_ptr, c_ptr]),
+    "rdg_export_3dgs": (C.c_int, [C.POINTER(RdgScene), C.c_int32, c_ptr, c_ptr]),
     "rdg_bin_workspace_bytes": (C.c_int64, [C.c_int64, C.c_int64, C.c_int32, C.c_int32]),
     "rdg_bin": (C.c_int, [C.c_int64, C.POINTER(RdgGeom), C.c_int32, C.c_int32, C.c_int64, C.POINTER(RdgBins),
                           c_ptr, C.c_int64, c_ptr]),

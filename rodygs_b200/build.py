@@ -44,6 +44,7 @@ SOURCES = {
     "pose.cu": [],
     "lpips.cu": [],
     "track.cu": ["-fmad=false"],
+    "export.cu": ["-fmad=false"],
 }
 # every header the sources include takes part in the digest, so that editing one rebuilds the library
 HEADERS = sorted(f for f in os.listdir(CSRC) if f.endswith(".cuh")) + [os.path.join("..", "..", "include", "rodygs_b200.h")]

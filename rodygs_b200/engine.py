@@ -527,6 +527,22 @@ def track(scene: SceneArgs, view_src: ViewArgs, basis_t_src: Optional[torch.Tens
     return out + (S_all, positions) if keep_maps else out
 
 
+RECORD_FLOATS = 62   # RDG_3DGS_RECORD_FLOATS: x y z nx ny nz f_dc_0..2 f_rest_0..44 opacity scale_0..2 rot_0..3
+
+
+def export_3dgs(scene: SceneArgs, sh_degree: int, device: torch.device) -> torch.Tensor:
+    """The scene at B(t) = scene.basis_t as 3DGS PLY vertex records [N, 62] float32 on the device, static rows first
+    (rdg_export_3dgs, INTEGRATION.md §11).  scene: raw parameters, no colors_precomp.  One launch, no host read."""
+    ns, nd = scene.counts()
+    dev = torch.device(device)
+    if dev.type != "cuda":
+        raise RuntimeError("rodygs_b200 runs on CUDA tensors only (no CPU fallback)")
+    records = torch.empty(ns + nd, RECORD_FLOATS, dtype=torch.float32, device=dev)
+    sc = _scene_struct(scene)
+    check(_lib.load().rdg_export_3dgs(C.byref(sc), int(sh_degree), ptr(records), _lib.stream_ptr()))
+    return records
+
+
 @dataclass
 class SetGrads:
     xyz: Optional[torch.Tensor] = None

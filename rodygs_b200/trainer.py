@@ -264,13 +264,16 @@ class SplatTrainStep:
             raise ValueError(f"SplatTrainStep: {name} must be a contiguous float32 tensor of shape {tuple(shape)} on {self.params.device}, got {got}")
 
     # -- one view --------------------------------------------------------------------------------
-    def _scene_view(self, viewmatrix, projmatrix, tanfovx, tanfovy, basis_t) -> Tuple[SceneArgs, ViewArgs]:
+    def _scene(self, basis_t) -> SceneArgs:
         deform = self.nd > 0
-        scene = SceneArgs(st=self._set("static"), dy=self._set("dynamic"), raw=True, use_deform=deform,
-                          motion_coeff=self.p("motion_coeff").view(self.nd, self.num_basis) if deform else None,
-                          time_ind=self.time_ind if deform else None, basis_t=basis_t if deform else None,
-                          table=self.p("table") if deform else None, spatial_lr_scale=self.spatial_lr_scale,
-                          frame_order=self.frame_order, frame_offsets=self.frame_offsets)
+        return SceneArgs(st=self._set("static"), dy=self._set("dynamic"), raw=True, use_deform=deform,
+                         motion_coeff=self.p("motion_coeff").view(self.nd, self.num_basis) if deform else None,
+                         time_ind=self.time_ind if deform else None, basis_t=basis_t if deform else None,
+                         table=self.p("table") if deform else None, spatial_lr_scale=self.spatial_lr_scale,
+                         frame_order=self.frame_order, frame_offsets=self.frame_offsets)
+
+    def _scene_view(self, viewmatrix, projmatrix, tanfovx, tanfovy, basis_t) -> Tuple[SceneArgs, ViewArgs]:
+        scene = self._scene(basis_t)
         view = ViewArgs(height=self.H, width=self.W, tanfovx=tanfovx, tanfovy=tanfovy, scale_modifier=1.0,
                         sh_degree=self.sh_degree, viewmatrix=viewmatrix, projmatrix=projmatrix, bg=self.bg)
         return scene, view
@@ -1236,6 +1239,22 @@ class SplatTrainStep:
         deform = self.nd > 0
         return engine.track(scene, view, basis_t if deform else None, target_viewmats, target_projmats,
                             target_basis_ts if deform else None, points)
+
+    def export_3dgs(self, basis_t: Optional[torch.Tensor]) -> torch.Tensor:
+        """The scene at time t as the vertex records of 3D Gaussian Splatting's PLY file: [N, 62] float32 on the device,
+        static Gaussians first, columns in the order of rodygs_b200.ply.PLY_PROPERTIES (rdg_export_3dgs, INTEGRATION.md
+        §11).  rodygs_b200.ply.write_ply(path, records) writes the file a 3DGS viewer opens.
+
+        basis_t [K, 7] = B(t) (basis_forward(t), a row of the motion table, or BasisMLP.query_and_table); None without
+        dynamic Gaussians.  SH coefficients above this step's SH degree are written as 0, so that a viewer draws what
+        render_views draws.  A dynamic Gaussian's record holds its deformed mean and the covariance the rasterizer draws,
+        re-factored into a unit quaternion and log-scales; static records are the raw parameters, bit for bit.
+
+        No training state changes (the list of render_views).  Data parallel: no collective; every rank holds the whole
+        model, so call it on one rank."""
+        if self.nd > 0:
+            self._check_input("basis_t", basis_t, (self.num_basis, 7))
+        return engine.export_3dgs(self._scene(basis_t), self.sh_degree, self.params.device)
 
     def refine_poses(self, viewmats: torch.Tensor, projmats: torch.Tensor, tanfovx, tanfovy, gts: torch.Tensor, lr: float,
                      iters: int = 1000) -> Tuple[torch.Tensor, torch.Tensor]:
