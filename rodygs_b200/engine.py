@@ -15,7 +15,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 from dataclasses import dataclass, field
-from typing import Dict, Optional
+from typing import Dict, List, Optional
 
 import torch
 
@@ -159,6 +159,7 @@ class FwdState:
     n_contrib: torch.Tensor
     d_cap: int
     extras: dict = field(default_factory=dict)
+    bins: Optional[RdgBins] = None    # the RdgBins the forward filled (its buffers are the tensors above)
 
 
 def _set_struct(s: Optional[SetArgs]) -> RdgSet:
@@ -223,6 +224,113 @@ def _geom_struct(g: dict) -> RdgGeom:
     return out
 
 
+def _image_struct(color, depth, alpha, final_T, n_contrib) -> RdgImage:
+    out = RdgImage()
+    out.color, out.depth, out.alpha, out.final_T, out.n_contrib = ptr(color), ptr(depth), ptr(alpha), ptr(final_T), ptr(n_contrib)
+    return out
+
+
+def _alloc_geom(n: int, dev: torch.device, radii: Optional[torch.Tensor] = None,
+                tile_count: Optional[torch.Tensor] = None) -> dict:
+    """The per-Gaussian records rdg_preprocess_fwd writes for one view, as the dict _geom_struct reads.  radii [n] int32 and
+    tile_count [tiles + 1] int32 may be the caller's (render_views hands in rows of its [V, n] / [k, tiles + 1] outputs);
+    without a tile_count the records have none (rdg_bin needs none)."""
+    f32 = dict(dtype=torch.float32, device=dev)
+    geom = {"radii": torch.empty(n, dtype=torch.int32, device=dev) if radii is None else radii,
+            "tiles_touched": torch.empty(n, dtype=torch.int32, device=dev),
+            "p0": torch.empty(n, 4, **f32), "p1": torch.empty(n, 4, **f32), "p2": torch.empty(n, 2, **f32),
+            "clamped": torch.empty(n, dtype=torch.uint8, device=dev)}
+    if tile_count is not None:
+        geom["tile_count"] = tile_count
+    return geom
+
+
+class Bins:
+    """The buffers of one frame's binning at duplicate capacity `cap` and the RdgBins over them (`s`).
+
+    ranges [tiles, 2], num_rendered [2] and region_count [2 * tiles] are frame-sized and the caller's: render_views and the
+    pose loop keep them across views and re-allocations.  Allocated here at `cap`: vals, keys (keys=True), the region lists
+    of the blend kernels (two 16x8 regions per tile, region_stride = cap; rdg_blend_fwd writes them, rdg_blend_bwd reads
+    them) and the binning workspace.  bin() runs rdg_bin_tiles or, with lsd, rdg_bin (scan + duplicateWithKeys + global LSD
+    radix sort), which also needs the keys and point_offsets [n], and under config.debug_keep_unsorted keeps
+    duplicateWithKeys' output in keys_unsorted / vals_unsorted."""
+
+    def __init__(self, n: int, H: int, W: int, cap: int, ranges: torch.Tensor, num_rendered: torch.Tensor,
+                 region_count: torch.Tensor, keys: bool = False, lsd: bool = False,
+                 point_offsets: Optional[torch.Tensor] = None):
+        lib = _lib.load()
+        dev = ranges.device
+        self.n, self.H, self.W, self.cap, self.lsd = n, H, W, cap, lsd
+        self.keys = torch.empty(cap, dtype=torch.int64, device=dev) if keys or lsd else None
+        self.vals = torch.empty(cap, dtype=torch.int32, device=dev)
+        self.region_ids = torch.empty(2 * cap, dtype=torch.int32, device=dev)
+        self.region_masks = torch.empty(2 * cap, dtype=torch.uint8, device=dev)
+        self.ws_bytes = int((lib.rdg_bin_workspace_bytes if lsd else lib.rdg_bin_tiles_workspace_bytes)(n, cap, H, W))
+        self.ws = torch.empty(self.ws_bytes, dtype=torch.uint8, device=dev)
+        s = RdgBins()
+        s.keys_sorted, s.vals_sorted = ptr(self.keys), ptr(self.vals)
+        s.ranges, s.point_offsets, s.num_rendered = ptr(ranges), ptr(point_offsets), ptr(num_rendered)
+        s.region_ids, s.region_masks, s.region_count = ptr(self.region_ids), ptr(self.region_masks), ptr(region_count)
+        s.region_stride = cap
+        self.keys_unsorted = self.vals_unsorted = None
+        if lsd and config.debug_keep_unsorted:
+            self.keys_unsorted = torch.empty(cap, dtype=torch.int64, device=dev)
+            self.vals_unsorted = torch.empty(cap, dtype=torch.int32, device=dev)
+            s.keys_unsorted, s.vals_unsorted = ptr(self.keys_unsorted), ptr(self.vals_unsorted)
+        self.s = s
+
+    def bin(self, gm_s: RdgGeom):
+        lib = _lib.load()
+        check((lib.rdg_bin if self.lsd else lib.rdg_bin_tiles)(self.n, C.byref(gm_s), self.H, self.W, self.cap, C.byref(self.s),
+                                                                ptr(self.ws), self.ws_bytes, _lib.stream_ptr()))
+
+
+def _exact_bins(n: int, gm_s, tile_count: torch.Tensor, H: int, W: int, ranges: torch.Tensor, num_rendered: torch.Tensor,
+                region_count: torch.Tensor):
+    """Bins of k views at exactly their duplicate counts, the sums of the per-tile counts preprocess wrote into tile_count
+    [k, tiles + 1] (gm_s[j]: the RdgGeom of view j), read in ONE host read for all k.  View j is binned (rdg_bin_tiles) in
+    buffers of max(count, 1) when the generator reaches it, so that the k views' buffers are not all alive at once.  Nothing
+    overflows or is re-binned, and the duplicate-capacity state (_capacity, a pending sync-free count) is neither read nor
+    changed."""
+    counts = tile_count[:, :tiles_of(H, W)].sum(1).tolist()
+    for j, d in enumerate(counts):
+        bins = Bins(n, H, W, max(int(d), 1), ranges, num_rendered, region_count)
+        bins.bin(gm_s[j])
+        yield bins
+
+
+def _blend_bwd_scratch(n: int, dev: torch.device) -> Optional[torch.Tensor]:
+    """rdg_blend_bwd_deterministic's scratch for n Gaussians under config.deterministic, else None."""
+    if not config.deterministic:
+        return None
+    return torch.empty(max(int(_lib.load().rdg_blend_bwd_deterministic_scratch_bytes(n)), 8), dtype=torch.uint8, device=dev)
+
+
+def _blend_bwd(n: int, gm_s: RdgGeom, bins_s: RdgBins, vw_s: RdgView, img_s: RdgImage, dL_dcolor, dL_ddepth, dL_dalpha,
+               acc: torch.Tensor, scratch: Optional[torch.Tensor] = None):
+    """The blend backward into acc [n, NACC]: rdg_blend_bwd, or under config.deterministic rdg_blend_bwd_deterministic, with
+    the "deterministic" tunable (which also puts the per-Gaussian backward on one CTA) set to match.  scratch: from
+    _blend_bwd_scratch; allocated here when None, so a caller that captures a CUDA graph passes its own."""
+    lib, stream = _lib.load(), _lib.stream_ptr()
+    _lib.set_tunable("deterministic", 1 if config.deterministic else 0)
+    args = (n, C.byref(gm_s), C.byref(bins_s), C.byref(vw_s), C.byref(img_s), ptr(dL_dcolor), ptr(dL_ddepth), ptr(dL_dalpha),
+            ptr(acc))
+    if config.deterministic:
+        if scratch is None:
+            scratch = _blend_bwd_scratch(n, acc.device)
+        check(lib.rdg_blend_bwd_deterministic(*args, ptr(scratch), scratch.numel(), stream))
+    else:
+        check(lib.rdg_blend_bwd(*args, stream))
+
+
+def per_view(fn: str, name: str, value, n: int) -> List[float]:
+    """A float, or one float per view, as a list of n floats; ValueError prefixed with the caller fn otherwise."""
+    vals = [float(t) for t in value] if hasattr(value, "__len__") else [float(value)] * n
+    if len(vals) != n:
+        raise ValueError(f"{fn}: {name} must be a float or {n} values, got {len(vals)}")
+    return vals
+
+
 _csr_cache: Dict[tuple, tuple] = {}
 
 
@@ -274,18 +382,12 @@ def render_forward(scene: SceneArgs, view: ViewArgs, keep_for_backward: bool = T
         raise RuntimeError("rodygs_b200 runs on CUDA tensors only (no CPU fallback)")
     stream = _lib.stream_ptr()
     H, W = int(view.height), int(view.width)
+    ntiles = tiles_of(H, W)
     f32 = dict(dtype=torch.float32, device=dev)
-    geom = {
-        "radii": torch.empty(n, dtype=torch.int32, device=dev),
-        "tiles_touched": torch.empty(n, dtype=torch.int32, device=dev),
-        "p0": torch.empty(n, 4, **f32), "p1": torch.empty(n, 4, **f32), "p2": torch.empty(n, 2, **f32),
-        "clamped": torch.empty(n, dtype=torch.uint8, device=dev),
-    }
+    use_tiles = config.binning == "tiles" and not config.debug_keep_unsorted
+    geom = _alloc_geom(n, dev, tile_count=torch.empty(ntiles + 1, dtype=torch.int32, device=dev) if use_tiles else None)
     if config.debug_activated:
         geom["dbg_activated"] = torch.zeros(n, 11, **f32)
-    use_tiles = config.binning == "tiles" and not config.debug_keep_unsorted
-    if use_tiles:
-        geom["tile_count"] = torch.empty(tiles_of(H, W) + 1, dtype=torch.int32, device=dev)
     sc_s, vw_s, gm_s = _scene_struct(scene), _view_struct(view), _geom_struct(geom)
     check(lib.rdg_preprocess_fwd(C.byref(sc_s), C.byref(vw_s), C.byref(gm_s), stream))
     if stage_hook:
@@ -294,33 +396,14 @@ def render_forward(scene: SceneArgs, view: ViewArgs, keep_for_backward: bool = T
     st = _cap_state(dev, n)
     if not config.capturing:
         _check_pending(st)
-    ntiles = tiles_of(H, W)
     ranges = torch.empty(ntiles, 2, dtype=torch.int32, device=dev)
     point_offsets = torch.empty(n, dtype=torch.int32, device=dev)
     num_rendered = torch.empty(2, dtype=torch.int32, device=dev)
-    extras = {}
+    region_count = torch.empty(2 * ntiles, dtype=torch.int32, device=dev)
     while True:
-        d_cap = int(st["cap"])
-        want_keys = config.emit_sorted_keys or not use_tiles
-        keys = torch.empty(d_cap, dtype=torch.int64, device=dev) if want_keys else None
-        vals = torch.empty(d_cap, dtype=torch.int32, device=dev)
-        # region lists of the blend kernels (two 16x8 regions per tile; rdg_blend_fwd writes, rdg_blend_bwd reads)
-        region_ids = torch.empty(2 * d_cap, dtype=torch.int32, device=dev)
-        region_masks = torch.empty(2 * d_cap, dtype=torch.uint8, device=dev)
-        region_count = torch.empty(2 * ntiles, dtype=torch.int32, device=dev)
-        ws_bytes = int((lib.rdg_bin_tiles_workspace_bytes if use_tiles else lib.rdg_bin_workspace_bytes)(n, d_cap, H, W))
-        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-        bins = RdgBins()
-        bins.keys_sorted, bins.vals_sorted = ptr(keys), ptr(vals)
-        bins.ranges, bins.point_offsets, bins.num_rendered = ptr(ranges), ptr(point_offsets), ptr(num_rendered)
-        bins.region_ids, bins.region_masks, bins.region_count = ptr(region_ids), ptr(region_masks), ptr(region_count)
-        bins.region_stride = d_cap
-        if config.debug_keep_unsorted:
-            extras["keys_unsorted"] = torch.empty(d_cap, dtype=torch.int64, device=dev)
-            extras["vals_unsorted"] = torch.empty(d_cap, dtype=torch.int32, device=dev)
-            bins.keys_unsorted, bins.vals_unsorted = ptr(extras["keys_unsorted"]), ptr(extras["vals_unsorted"])
-        check((lib.rdg_bin_tiles if use_tiles else lib.rdg_bin)(n, C.byref(gm_s), H, W, d_cap, C.byref(bins), ptr(ws),
-                                                                ws_bytes, stream))
+        bins = Bins(n, H, W, int(st["cap"]), ranges, num_rendered, region_count, keys=config.emit_sorted_keys,
+                    lsd=not use_tiles, point_offsets=point_offsets)
+        bins.bin(gm_s)
         if config.sync_free:
             # (under graph capture the pinned buffer was allocated beforehand: no cudaHostAlloc inside a capture)
             host = config.capture_host if config.capturing else torch.empty(2, dtype=torch.int32, pin_memory=True)
@@ -329,11 +412,11 @@ def render_forward(scene: SceneArgs, view: ViewArgs, keep_for_backward: bool = T
             if not config.capturing:
                 ev = torch.cuda.Event()
                 ev.record()
-            st["pending"] = (host, ev, d_cap)
+            st["pending"] = (host, ev, bins.cap)
             break
         d = int(num_rendered[0].item())          # the reference's one host read per forward
-        if d <= d_cap:
-            if d * config.headroom > d_cap:
+        if d <= bins.cap:
+            if d * config.headroom > bins.cap:
                 st["cap"] = int(d * config.headroom) + 1
             break
         st["cap"] = int(d * config.headroom) + 1  # overflow: re-bin with a larger buffer
@@ -345,16 +428,18 @@ def render_forward(scene: SceneArgs, view: ViewArgs, keep_for_backward: bool = T
     alpha = torch.empty(1, H, W, **f32)
     final_T = torch.empty(H, W, **f32)
     n_contrib = torch.empty(H, W, dtype=torch.int32, device=dev)
-    img = RdgImage()
-    img.color, img.depth, img.alpha, img.final_T, img.n_contrib = ptr(color), ptr(depth), ptr(alpha), ptr(final_T), ptr(n_contrib)
-    check(lib.rdg_blend_fwd(n, C.byref(gm_s), C.byref(bins), C.byref(vw_s), C.byref(img), stream))
+    img = _image_struct(color, depth, alpha, final_T, n_contrib)
+    check(lib.rdg_blend_fwd(n, C.byref(gm_s), C.byref(bins.s), C.byref(vw_s), C.byref(img), stream))
     if stage_hook:
         stage_hook("blend_fwd")
 
-    extras.update({"keys_sorted": keys, "point_offsets": point_offsets, "region_ids": region_ids, "region_masks": region_masks,
-                   "region_count": region_count})
-    state = FwdState(scene=scene, view=view, n=n, geom=geom, vals_sorted=vals, ranges=ranges,
-                     num_rendered=num_rendered, final_T=final_T, n_contrib=n_contrib, d_cap=d_cap, extras=extras)
+    extras = {"keys_sorted": bins.keys, "point_offsets": point_offsets, "region_ids": bins.region_ids,
+              "region_masks": bins.region_masks, "region_count": region_count}
+    if config.debug_keep_unsorted:
+        extras["keys_unsorted"], extras["vals_unsorted"] = bins.keys_unsorted, bins.vals_unsorted
+    state = FwdState(scene=scene, view=view, n=n, geom=geom, vals_sorted=bins.vals, ranges=ranges,
+                     num_rendered=num_rendered, final_T=final_T, n_contrib=n_contrib, d_cap=bins.cap, extras=extras,
+                     bins=bins.s)
     return color, depth, alpha, geom["radii"], state
 
 
@@ -394,33 +479,17 @@ def render_views(scene: SceneArgs, views, basis_ts: Optional[torch.Tensor], stag
         k = len(pv)
         # zeroed here as well: without Gaussians the kernel returns before it zeroes them, and the counts must still read 0
         tile_count = torch.zeros(k, ntiles + 1, dtype=torch.int32, device=dev)
-        geoms = [{"radii": radii[lo + j], "tiles_touched": torch.empty(n, dtype=torch.int32, device=dev),
-                  "p0": torch.empty(n, 4, **f32), "p1": torch.empty(n, 4, **f32), "p2": torch.empty(n, 2, **f32),
-                  "clamped": torch.empty(n, dtype=torch.uint8, device=dev), "tile_count": tile_count[j]} for j in range(k)]
+        geoms = [_alloc_geom(n, dev, radii=radii[lo + j], tile_count=tile_count[j]) for j in range(k)]
         vw_s = (RdgView * k)(*[_view_struct(v) for v in pv])
         gm_s = (RdgGeom * k)(*[_geom_struct(g) for g in geoms])
         bts = None if basis_ts is None else basis_ts[lo:lo + k].contiguous()
         check(lib.rdg_preprocess_fwd_views(C.byref(sc_s), ptr(bts), k, vw_s, gm_s, stream))
         if stage_hook:
             stage_hook("preprocess_fwd")
-        counts = tile_count[:, :ntiles].sum(1).tolist()          # the pass's one host read
-        for j in range(k):
-            d_cap = max(int(counts[j]), 1)
-            vals = torch.empty(d_cap, dtype=torch.int32, device=dev)
-            region_ids = torch.empty(2 * d_cap, dtype=torch.int32, device=dev)
-            region_masks = torch.empty(2 * d_cap, dtype=torch.uint8, device=dev)
-            ws_bytes = int(lib.rdg_bin_tiles_workspace_bytes(n, d_cap, H, W))
-            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-            bins = RdgBins()
-            bins.vals_sorted, bins.ranges, bins.num_rendered = ptr(vals), ptr(ranges), ptr(num_rendered)
-            bins.region_ids, bins.region_masks, bins.region_count = ptr(region_ids), ptr(region_masks), ptr(region_count)
-            bins.region_stride = d_cap
-            check(lib.rdg_bin_tiles(n, C.byref(gm_s[j]), H, W, d_cap, C.byref(bins), ptr(ws), ws_bytes, stream))
-            img = RdgImage()
+        for j, bins in enumerate(_exact_bins(n, gm_s, tile_count, H, W, ranges, num_rendered, region_count)):
             v = lo + j
-            img.color, img.depth, img.alpha = ptr(color[v]), ptr(depth[v]), ptr(alpha[v])
-            img.final_T, img.n_contrib = ptr(final_T), ptr(n_contrib)
-            check(lib.rdg_blend_fwd(n, C.byref(gm_s[j]), C.byref(bins), C.byref(vw_s[j]), C.byref(img), stream))
+            img = _image_struct(color[v], depth[v], alpha[v], final_T, n_contrib)
+            check(lib.rdg_blend_fwd(n, C.byref(gm_s[j]), C.byref(bins.s), C.byref(vw_s[j]), C.byref(img), stream))
         if stage_hook:
             stage_hook("bin_blend")
     return color, depth, alpha, radii
@@ -456,29 +525,17 @@ def track(scene: SceneArgs, view_src: ViewArgs, basis_t_src: Optional[torch.Tens
     ntiles = tiles_of(H, W)
     f32 = dict(dtype=torch.float32, device=dev)
     # the source render: its records, bins and alpha are shared by every target
-    geom = {"radii": torch.empty(n, dtype=torch.int32, device=dev), "tiles_touched": torch.empty(n, dtype=torch.int32, device=dev),
-            "p0": torch.empty(n, 4, **f32), "p1": torch.empty(n, 4, **f32), "p2": torch.empty(n, 2, **f32),
-            "clamped": torch.empty(n, dtype=torch.uint8, device=dev),
-            # zeroed here as well: without Gaussians preprocess returns before it zeroes them
-            "tile_count": torch.zeros(ntiles + 1, dtype=torch.int32, device=dev)}
+    # (tile_count zeroed here as well: without Gaussians preprocess returns before it zeroes it)
+    tile_count = torch.zeros(1, ntiles + 1, dtype=torch.int32, device=dev)
+    geom = _alloc_geom(n, dev, tile_count=tile_count[0])
     sc_s, gm_s = _scene_struct(scene), _geom_struct(geom)
     sc_s.basis_t = ptr(basis_t_src) if sc_s.use_deform else None
     check(lib.rdg_preprocess_fwd(C.byref(sc_s), C.byref(_view_struct(view_src)), C.byref(gm_s), stream))
     sc_s.basis_t = None                                          # rdg_track_attrs takes B(t_m) on its own
-    d_cap = max(int(geom["tile_count"][:ntiles].sum()), 1)      # the call's one host read
-    vals = torch.empty(d_cap, dtype=torch.int32, device=dev)
     ranges = torch.empty(ntiles, 2, dtype=torch.int32, device=dev)
     num_rendered = torch.empty(2, dtype=torch.int32, device=dev)
-    region_ids = torch.empty(2 * d_cap, dtype=torch.int32, device=dev)
-    region_masks = torch.empty(2 * d_cap, dtype=torch.uint8, device=dev)
     region_count = torch.empty(2 * ntiles, dtype=torch.int32, device=dev)
-    ws_bytes = int(lib.rdg_bin_tiles_workspace_bytes(n, d_cap, H, W))
-    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-    bins = RdgBins()
-    bins.vals_sorted, bins.ranges, bins.num_rendered = ptr(vals), ptr(ranges), ptr(num_rendered)
-    bins.region_ids, bins.region_masks, bins.region_count = ptr(region_ids), ptr(region_masks), ptr(region_count)
-    bins.region_stride = d_cap
-    check(lib.rdg_bin_tiles(n, C.byref(gm_s), H, W, d_cap, C.byref(bins), ptr(ws), ws_bytes, stream))
+    (bins,) = _exact_bins(n, [gm_s], tile_count, H, W, ranges, num_rendered, region_count)
     if stage_hook:
         stage_hook("source")
 
@@ -509,10 +566,8 @@ def track(scene: SceneArgs, view_src: ViewArgs, basis_t_src: Optional[torch.Tens
             check(lib.rdg_track_attrs(C.byref(sc_s), ptr(bt), C.byref(gm_s), ptr(positions[m]) if keep_maps else None, stream))
             if stage_hook:
                 stage_hook("attrs")
-            img = RdgImage()
-            img.color, img.depth, img.alpha = ptr(S[j]), ptr(blend_depth), ptr(alpha)
-            img.final_T, img.n_contrib = ptr(final_T), ptr(n_contrib)
-            check(lib.rdg_blend_fwd(n, C.byref(gm_s), C.byref(bins), C.byref(vw_blend), C.byref(img), stream))
+            img = _image_struct(S[j], blend_depth, alpha, final_T, n_contrib)
+            check(lib.rdg_blend_fwd(n, C.byref(gm_s), C.byref(bins.s), C.byref(vw_blend), C.byref(img), stream))
             if stage_hook:
                 stage_hook("blend")
         if not sparse:
@@ -595,26 +650,13 @@ def render_backward(state: FwdState, dL_dcolor, dL_ddepth, dL_dalpha, grads: Sce
     n = state.n
     acc = torch.zeros(max(n, 1), NACC, dtype=torch.float32, device=dev)
     sc_s, vw_s, gm_s = _scene_struct(state.scene), _view_struct(state.view), _geom_struct(state.geom)
-    bins = RdgBins()
-    bins.vals_sorted, bins.ranges, bins.num_rendered = ptr(state.vals_sorted), ptr(state.ranges), ptr(state.num_rendered)
-    bins.region_ids, bins.region_masks = ptr(state.extras["region_ids"]), ptr(state.extras["region_masks"])
-    bins.region_count, bins.region_stride = ptr(state.extras["region_count"]), state.d_cap
-    img = RdgImage()
-    img.final_T, img.n_contrib = ptr(state.final_T), ptr(state.n_contrib)
+    img = _image_struct(None, None, None, state.final_T, state.n_contrib)
 
     def c(t):
         return None if t is None else t.contiguous()
 
     dL_dcolor, dL_ddepth, dL_dalpha = c(dL_dcolor), c(dL_ddepth), c(dL_dalpha)
-    _lib.set_tunable("deterministic", 1 if config.deterministic else 0)
-    if config.deterministic:
-        nb = int(lib.rdg_blend_bwd_deterministic_scratch_bytes(n))
-        scratch = torch.empty(max(nb, 8), dtype=torch.uint8, device=dev)
-        check(lib.rdg_blend_bwd_deterministic(n, C.byref(gm_s), C.byref(bins), C.byref(vw_s), C.byref(img), ptr(dL_dcolor),
-                                              ptr(dL_ddepth), ptr(dL_dalpha), ptr(acc), ptr(scratch), nb, stream))
-    else:
-        check(lib.rdg_blend_bwd(n, C.byref(gm_s), C.byref(bins), C.byref(vw_s), C.byref(img),
-                                ptr(dL_dcolor), ptr(dL_ddepth), ptr(dL_dalpha), ptr(acc), stream))
+    _blend_bwd(n, gm_s, state.bins, vw_s, img, dL_dcolor, dL_ddepth, dL_dalpha, acc)
     early = after_blend is not None and grads.dcolor is not None and state.scene.colors_precomp is None
     if early:
         if grads.dcolor_mc:

@@ -11,12 +11,12 @@ pending sync-free count included).
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, List, Sequence, Tuple, Union
+from typing import Dict, Sequence, Tuple, Union
 
 import torch
 
 from . import _lib, engine
-from ._lib import RdgBins, RdgPoseAdam, RdgSceneGrad, check, ptr
+from ._lib import RdgPoseAdam, RdgSceneGrad, check, ptr
 from .engine import NACC, SceneArgs, SetArgs, ViewArgs
 
 BETAS = (0.9, 0.999)            # torch.optim.Adam defaults
@@ -25,14 +25,6 @@ ORTHONORMAL_TOL = 1e-4
 CHUNK = 100                     # graph replays between two host reads of the step counter and the overflow latch
 STATIC_FIELDS = {"xyz": (3,), "features_dc": (1, 3), "features_rest": (15, 3), "scaling": (3,), "rotation": (4,),
                  "opacity": (1,)}
-
-
-def per_view(name: str, v, n_views: int) -> List[float]:
-    """A float, or one float per view, as a list of n_views floats."""
-    vals = [float(t) for t in v] if hasattr(v, "__len__") else [float(v)] * n_views
-    if len(vals) != n_views:
-        raise ValueError(f"refine_poses: {name} must be a float or {n_views} values, got {len(vals)}")
-    return vals
 
 
 def pose_from_viewmatrix(viewmats: torch.Tensor) -> torch.Tensor:
@@ -108,9 +100,7 @@ class _PoseLoop:
         i32 = dict(dtype=torch.int32, device=dev)
         n, H, W = self.n, self.H, self.W
         self.scene = engine._scene_struct(SceneArgs(st=st, raw=True))
-        self.geom = {"radii": torch.empty(n, **i32), "tiles_touched": torch.empty(n, **i32), "p0": torch.empty(n, 4, **f32),
-                     "p1": torch.empty(n, 4, **f32), "p2": torch.empty(n, 2, **f32),
-                     "clamped": torch.empty(n, dtype=torch.uint8, device=dev), "tile_count": torch.empty(self.tiles + 1, **i32)}
+        self.geom = engine._alloc_geom(n, dev, tile_count=torch.empty(self.tiles + 1, **i32))
         self.geom_s = engine._geom_struct(self.geom)
         self.ranges = torch.empty(self.tiles, 2, **i32)
         self.num_rendered = torch.zeros(2, **i32)
@@ -119,8 +109,7 @@ class _PoseLoop:
         self.final_T, self.n_contrib = torch.empty(H, W, **f32), torch.empty(H, W, **i32)
         self.gt, self.dL_dcolor = gt, torch.empty(3, H, W, **f32)
         self.acc = torch.zeros(n, NACC, **f32)
-        self.det_bytes = int(self.lib.rdg_blend_bwd_deterministic_scratch_bytes(n)) if engine.config.deterministic else 0
-        self.det_scratch = torch.empty(self.det_bytes, dtype=torch.uint8, device=dev) if self.det_bytes else None
+        self.det_scratch = engine._blend_bwd_scratch(n, dev)
         self.loss_bytes = int(self.lib.rdg_l2_loss_workspace_bytes(3, H, W))
         self.loss_ws = torch.empty(self.loss_bytes, dtype=torch.uint8, device=dev)
         self.history = torch.zeros(iters, **f32)
@@ -144,51 +133,31 @@ class _PoseLoop:
         self.graph = None
 
     def _alloc_bins(self, cap: int):
-        dev = self.gt.device
         self.cap = int(cap)
-        self.vals = torch.empty(self.cap, dtype=torch.int32, device=dev)
-        self.region_ids = torch.empty(2 * self.cap, dtype=torch.int32, device=dev)
-        self.region_masks = torch.empty(2 * self.cap, dtype=torch.uint8, device=dev)
-        self.bin_bytes = int(self.lib.rdg_bin_tiles_workspace_bytes(self.n, self.cap, self.H, self.W))
-        self.bin_ws = torch.empty(self.bin_bytes, dtype=torch.uint8, device=dev)
-        b = RdgBins()
-        b.vals_sorted, b.ranges, b.num_rendered = ptr(self.vals), ptr(self.ranges), ptr(self.num_rendered)
-        b.region_ids, b.region_masks, b.region_count = ptr(self.region_ids), ptr(self.region_masks), ptr(self.region_count)
-        b.region_stride = self.cap
-        self.bins = b
+        self.bins = engine.Bins(self.n, self.H, self.W, self.cap, self.ranges, self.num_rendered, self.region_count)
 
     def _write_view(self):
         check(self.lib.rdg_pose_adam(C.byref(self.adam), 0, _lib.stream_ptr()))
 
-    def _forward_bins(self):
-        s = _lib.stream_ptr()
-        check(self.lib.rdg_preprocess_fwd(C.byref(self.scene), C.byref(self.view_s), C.byref(self.geom_s), s))
-        check(self.lib.rdg_bin_tiles(self.n, C.byref(self.geom_s), self.H, self.W, self.cap, C.byref(self.bins), ptr(self.bin_ws),
-                                     self.bin_bytes, s))
+    def _preprocess(self):
+        check(self.lib.rdg_preprocess_fwd(C.byref(self.scene), C.byref(self.view_s), C.byref(self.geom_s), _lib.stream_ptr()))
 
     def _iteration(self):
         lib, s = self.lib, _lib.stream_ptr()
-        self._forward_bins()
-        img = _lib.RdgImage()
-        img.color, img.depth, img.alpha = ptr(self.color), ptr(self.depth), ptr(self.alpha)
-        img.final_T, img.n_contrib = ptr(self.final_T), ptr(self.n_contrib)
-        check(lib.rdg_blend_fwd(self.n, C.byref(self.geom_s), C.byref(self.bins), C.byref(self.view_s), C.byref(img), s))
+        self._preprocess()
+        self.bins.bin(self.geom_s)
+        img = engine._image_struct(self.color, self.depth, self.alpha, self.final_T, self.n_contrib)
+        check(lib.rdg_blend_fwd(self.n, C.byref(self.geom_s), C.byref(self.bins.s), C.byref(self.view_s), C.byref(img), s))
         check(lib.rdg_l2_loss(ptr(self.color), ptr(self.gt), 3, self.H, self.W, ptr(self.step), self.iters, ptr(self.history),
                               ptr(self.dL_dcolor), ptr(self.loss_ws), self.loss_bytes, s))
         self.acc.zero_()
-        if engine.config.deterministic:
-            check(lib.rdg_blend_bwd_deterministic(self.n, C.byref(self.geom_s), C.byref(self.bins), C.byref(self.view_s),
-                                                  C.byref(img), ptr(self.dL_dcolor), None, None, ptr(self.acc),
-                                                  ptr(self.det_scratch), self.det_bytes, s))
-        else:
-            check(lib.rdg_blend_bwd(self.n, C.byref(self.geom_s), C.byref(self.bins), C.byref(self.view_s), C.byref(img),
-                                    ptr(self.dL_dcolor), None, None, ptr(self.acc), s))
+        engine._blend_bwd(self.n, self.geom_s, self.bins.s, self.view_s, img, self.dL_dcolor, None, None, self.acc,
+                          self.det_scratch)
         check(lib.rdg_preprocess_bwd(C.byref(self.scene), C.byref(self.view_s), C.byref(self.geom_s), ptr(self.acc),
                                      C.byref(self.grads), s))
         check(lib.rdg_pose_adam(C.byref(self.adam), 1, s))
 
     def _capture(self):
-        _lib.set_tunable("deterministic", 1 if engine.config.deterministic else 0)
         self.graph = None
         graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(graph):
@@ -197,13 +166,11 @@ class _PoseLoop:
 
     def run(self) -> Tuple[torch.Tensor, torch.Tensor]:
         headroom = max(float(engine.config.headroom), 1.0)
-        # duplicate capacity: one host read of the count at the initial pose (tile_scan counts past a full buffer)
+        # duplicate capacity: one host read of the count preprocess makes at the initial pose (the sum of its tile counts)
         self._write_view()
-        self._alloc_bins(1)
-        self._forward_bins()
-        self._alloc_bins(int(int(self.num_rendered[0]) * headroom) + 1)
+        self._preprocess()
+        self._alloc_bins(int(int(self.geom["tile_count"][:self.tiles].sum()) * headroom) + 1)
         # one eager iteration loads every kernel outside the capture; then the pose state starts over
-        _lib.set_tunable("deterministic", 1 if engine.config.deterministic else 0)
         self._iteration()
         self.param.copy_(self.pose0)
         for t in (self.exp_avg, self.exp_avg_sq, self.step, self.dV, self.overflow):
@@ -252,7 +219,7 @@ def refine_poses(static: Dict[str, torch.Tensor], height: int, width: int, sh_de
         raise ValueError(f"refine_poses: iters must be an integer >= 1, got {iters}")
     if not lr > 0 or lr == float("inf"):
         raise ValueError(f"refine_poses: lr must be a finite value > 0, got {lr}")
-    fovx, fovy = per_view("tanfovx", tanfovx, V), per_view("tanfovy", tanfovy, V)
+    fovx, fovy = engine.per_view("refine_poses", "tanfovx", tanfovx, V), engine.per_view("refine_poses", "tanfovy", tanfovy, V)
     st = _static_set(static)
     if st.xyz.device != dev:
         raise ValueError(f"refine_poses: the static model is on {st.xyz.device}, the views on {dev}")

@@ -1101,9 +1101,9 @@ class SplatTrainStep:
         Data parallel: every rank renders its shard_views() share and one sum all-reduce over the step's group gives every
         rank the whole table; all ranks call this with the same views.  No training state changes: parameters, gradients,
         moments, densification statistics, loss_parts, last_state / last_outputs, means2D_grad, the CUDA generator and
-        pending exchange_grads(defer_sh=True) factors stay as they were.  The views are binned with a host read of their
-        duplicate count even under config.sync_free, so that a view which overflows the buffers is re-binned here instead
-        of leaving an overflow for the next training step to raise."""
+        pending exchange_grads(defer_sh=True) factors stay as they were.  The views are rendered through engine.render_views
+        in passes of up to 8, each view binned at exactly its duplicate count, so engine's duplicate capacity and a pending
+        sync-free count of the training step are neither read nor changed."""
         V = viewmats.shape[0] if torch.is_tensor(viewmats) else 0
         if V < 1:
             raise ValueError("SplatTrainStep.evaluate: viewmats must be a [V, 4, 4] tensor with V >= 1")
@@ -1117,14 +1117,8 @@ class SplatTrainStep:
             got = f"{tuple(masks.shape)} {masks.device}" if torch.is_tensor(masks) else type(masks).__name__
             raise ValueError(f"SplatTrainStep.evaluate: masks must be a {(V, 1, self.H, self.W)} tensor on {self.params.device}, "
                              f"got {got}")
-
-        def per_view(name, v):
-            vals = [float(t) for t in v] if hasattr(v, "__len__") else [float(v)] * V
-            if len(vals) != V:
-                raise ValueError(f"SplatTrainStep.evaluate: {name} must be a float or {V} values, got {len(vals)}")
-            return vals
-
-        fovx, fovy = per_view("tanfovx", tanfovx), per_view("tanfovy", tanfovy)
+        fn = "SplatTrainStep.evaluate"
+        fovx, fovy = engine.per_view(fn, "tanfovx", tanfovx, V), engine.per_view(fn, "tanfovy", tanfovy, V)
         from .metrics import LpipsWeights, image_metrics, lpips as lpips_metric, masked_image_metrics, masked_lpips as mlpips
         nets = [] if lpips is None else [lpips] if isinstance(lpips, LpipsWeights) else list(lpips)
         if not all(isinstance(w, LpipsWeights) for w in nets):
@@ -1139,13 +1133,13 @@ class SplatTrainStep:
         rank, world = self._dp_rank_world()
         cols = 4 if masks is None else 7
         table = torch.zeros(V, cols + len(nets) + len(mnets), dtype=torch.float32, device=self.dev)
-        cap = engine._cap_state(self.params.device, self.ns + self.nd)
-        saved = engine.config.sync_free, cap["pending"]          # a training step's unread duplicate count stays for it
-        engine.config.sync_free, cap["pending"] = False, None
-        try:
-            for v in shard_views(V, world, rank):
-                scene, view = self._scene_view(viewmats[v], projmats[v], fovx[v], fovy[v], basis_ts[v] if self.nd > 0 else None)
-                color = engine.render_forward(scene, view)[0].clamp_(0.0, 1.0)
+        scene = self._scene(None)
+        mine = shard_views(V, world, rank)
+        for lo in range(0, len(mine), engine.VIEWS_PER_LAUNCH):      # passes of up to 8 bound the renders held at once
+            vs = mine[lo:lo + engine.VIEWS_PER_LAUNCH]
+            views = [self._scene_view(viewmats[v], projmats[v], fovx[v], fovy[v], None)[1] for v in vs]
+            colors = engine.render_views(scene, views, basis_ts[vs] if self.nd > 0 else None)[0].clamp_(0.0, 1.0)
+            for color, v in zip(colors, vs):
                 table[v, :4] = image_metrics(color, gts[v], value_range)[0]
                 if masks is not None:
                     table[v, 4:7] = masked_image_metrics(color, gts[v], masks[v], value_range)[0]
@@ -1153,8 +1147,6 @@ class SplatTrainStep:
                     table[v, cols + j] = lpips_metric(color, gts[v], w, value_range)[0]
                 for j, w in enumerate(mnets):
                     table[v, cols + len(nets) + j] = mlpips(color, gts[v], masks[v], w, value_range)[0]
-        finally:
-            engine.config.sync_free, cap["pending"] = saved
         allreduce_flat(table, None, self.pg)
         return table
 
@@ -1179,14 +1171,8 @@ class SplatTrainStep:
         self._check_input("projmats", projmats, (V, 4, 4))
         if self.nd > 0:
             self._check_input("basis_ts", basis_ts, (V, self.num_basis, 7))
-
-        def per_view(name, v):
-            vals = [float(t) for t in v] if hasattr(v, "__len__") else [float(v)] * V
-            if len(vals) != V:
-                raise ValueError(f"SplatTrainStep.render_views: {name} must be a float or {V} values, got {len(vals)}")
-            return vals
-
-        fovx, fovy = per_view("tanfovx", tanfovx), per_view("tanfovy", tanfovy)
+        fn = "SplatTrainStep.render_views"
+        fovx, fovy = engine.per_view(fn, "tanfovx", tanfovx, V), engine.per_view(fn, "tanfovy", tanfovy, V)
         scene, _ = self._scene_view(viewmats[0], projmats[0], fovx[0], fovy[0], None)
         views = [self._scene_view(viewmats[v], projmats[v], fovx[v], fovy[v], None)[1] for v in range(V)]
         return engine.render_views(scene, views, basis_ts if self.nd > 0 else None)
@@ -1277,7 +1263,7 @@ class SplatTrainStep:
             raise ValueError(f"SplatTrainStep.refine_poses: iters must be an integer >= 1, got {iters}")
         if not lr > 0 or lr == float("inf"):
             raise ValueError(f"SplatTrainStep.refine_poses: lr must be a finite value > 0, got {lr}")
-        fovx, fovy = pose.per_view("tanfovx", tanfovx, V), pose.per_view("tanfovy", tanfovy, V)
+        fovx, fovy = engine.per_view("refine_poses", "tanfovx", tanfovx, V), engine.per_view("refine_poses", "tanfovy", tanfovy, V)
         pose.pose_from_viewmatrix(viewmats)              # every rank refuses a bad view, not only the one that holds it
         rank, world = self._dp_rank_world()
         out = torch.zeros(V, 4, 4, dtype=torch.float32, device=self.dev)

@@ -338,10 +338,10 @@ def test_evaluate_leaves_the_training_state_alone():
 
 
 @pytest.mark.gpu
-def test_evaluate_rebins_an_overflowing_view_under_sync_free():
-    """With config.sync_free the training step leaves its duplicate count unread; a test view that overflows the duplicate
-    buffers (here: the capacity is cut below any view's count) is re-binned inside evaluate, returns the right row, and
-    the next training step does not raise."""
+def test_evaluate_leaves_a_pending_sync_free_count_and_the_capacity_alone():
+    """With config.sync_free the training step leaves its duplicate count unread.  evaluate bins every view at its own
+    count: with the capacity cut below any view's count it returns the right rows, leaves the capacity and the pending
+    count as they were, and the next training steps (which grow the capacity from that count) do not raise."""
     from rodygs_b200 import engine
     step = _make_step(20_000, 176, 208)
     cams, vms, pms, bts = _views(step, 2)
@@ -359,7 +359,7 @@ def test_evaluate_rebins_an_overflowing_view_under_sync_free():
         pending = cap["pending"]
         cap["cap"] = 256
         table = step.evaluate(vms, pms, cams[0].tanfovx, cams[0].tanfovy, bts, gts)
-        assert cap["pending"] is pending and cap["cap"] > 256
+        assert cap["cap"] == 256 and cap["pending"] is pending
         assert torch.equal(table, ref)
         for _ in range(2):
             lp = step.forward_backward(vms[0], pms[0], cams[0].tanfovx, cams[0].tanfovy, bts[0], gt, None)

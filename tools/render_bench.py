@@ -65,11 +65,7 @@ def main():
     # the preprocess stage alone, into preallocated geometry buffers
     lib, stream, n = _lib.load(), _lib.stream_ptr(), step.ns + step.nd
     tiles = engine.tiles_of(H, W)
-    f32 = dict(dtype=torch.float32, device="cuda")
-    geoms = [{"radii": torch.empty(n, dtype=torch.int32, device="cuda"), "tiles_touched": torch.empty(n, dtype=torch.int32, device="cuda"),
-              "p0": torch.empty(n, 4, **f32), "p1": torch.empty(n, 4, **f32), "p2": torch.empty(n, 2, **f32),
-              "clamped": torch.empty(n, dtype=torch.uint8, device="cuda"),
-              "tile_count": torch.empty(tiles + 1, dtype=torch.int32, device="cuda")} for _ in range(V)]
+    geoms = [engine._alloc_geom(n, "cuda", tile_count=torch.empty(tiles + 1, dtype=torch.int32, device="cuda")) for _ in range(V)]
     gm = (_lib.RdgGeom * V)(*[engine._geom_struct(g) for g in geoms])
     vw = (_lib.RdgView * V)(*[engine._view_struct(p[1]) for p in pairs])
     sc_views = engine._scene_struct(step._scene_view(vms[0], pms[0], fx[0], fy[0], None)[0])
